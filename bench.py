@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # CPU reference arm (oracle port)
+    python bench.py ... --dump-outputs DIR                   # + the last timed step's outputs as DIR/*.npy
 
 Headline workload (BASELINE.json configs[1]): synthetic chr1-scale 30x fragment set - one
 249,250,621-bp contig, 80 M start-sorted fragments per GPU (SURVEY.md §8d seeds) - and one
@@ -54,6 +55,42 @@ def log(*a):
 def make_intervals():
     edges = np.arange(0, CONTIG_LEN + IVL, IVL, dtype=np.int64).clip(max=CONTIG_LEN)
     return edges[:-1].copy(), edges[1:].copy()
+
+
+DUMP_WPS_SAMPLE = 1 << 22       # WPS positions kept by --dump-outputs (a fixed, seeded sample of 249 M)
+DUMP_SEED = 20240
+
+
+def dump_outputs(out_dir, offsets, wps, cov, hist, job_hist=None):
+    """Write what one step hands its caller as ``out_dir/<name>.npy`` (float32 / float64, about 51 MB), so that
+    two builds can be compared output for output on the same seeded input:
+
+    - ``wps_sample``: WPS (float32, exact) at ``wps_sample_index`` (float64, positions into the concatenated
+      per-interval WPS: ``DUMP_WPS_SAMPLE`` seeded draws, duplicates dropped, sorted);
+    - ``wps_interval_sum``: the sum of the WPS over every interval (float64, exact): touches every position;
+    - ``coverage``: per-interval midpoint coverage; ``length_hist``: the fragment-length histogram;
+      ``job_length_hist``: the histogram all-reduced over the ranks (N > 1 only)."""
+    import torch
+    n_pos = wps.numel()
+    rng = np.random.default_rng(DUMP_SEED)
+    idx = np.unique(rng.integers(0, n_pos, size=min(DUMP_WPS_SAMPLE, n_pos), dtype=np.int64))
+    cs = torch.zeros(n_pos + 1, dtype=torch.int64, device=wps.device)
+    cs[1:] = torch.cumsum(wps, 0, dtype=torch.int64)
+    off = torch.from_numpy(np.asarray(offsets, dtype=np.int64)).to(wps.device)
+    arrays = {
+        "wps_sample": wps[torch.from_numpy(idx).to(wps.device)].cpu().numpy().astype(np.float32),
+        "wps_sample_index": idx.astype(np.float64),
+        "wps_interval_sum": (cs[off[1:]] - cs[off[:-1]]).cpu().numpy().astype(np.float64),
+        "coverage": cov.cpu().numpy().astype(np.float64),
+        "length_hist": hist.cpu().numpy().astype(np.float64),
+    }
+    del cs
+    if job_hist is not None:
+        arrays["job_length_hist"] = job_hist.cpu().numpy().astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    log(f"[bench] wrote {len(arrays)} arrays ({sum(a.nbytes for a in arrays.values()) / 1e6:.1f} MB) to {out_dir}")
 
 
 # --------------------------------------------------------------------- clocks
@@ -653,6 +690,8 @@ def run_ours(args):
     torch.cuda.current_stream().synchronize()
     clocks = sampler.finish()
     barrier()
+    if args.dump_outputs and rank == 0:     # before anything else runs on these buffers
+        dump_outputs(args.dump_outputs, plan.offsets, wps_out, cov_out, hist_out, job_hist if world > 1 else None)
     ms_total = e0.elapsed_time(e1)
     t_ms = torch.tensor([ms_total], dtype=torch.float64, device=dev)
     if world > 1:
@@ -823,7 +862,13 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline / parity leg")
     ap.add_argument("--no-extras", action="store_true", help="skip the secondary kernels' timings")
     ap.add_argument("--no-genome", action="store_true", help="skip the genome-scale (configs 3/4) block")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs (rank 0's shard) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -115,8 +115,22 @@ def agg_signal(rows, strand, trim_lo, out_len, device=None):
     return torch.from_numpy(out)
 
 
+def _import_whole_package():
+    """Import every module of the package now, while ``device`` still holds the real classes: a module first
+    imported under the patch (``pipeline`` is imported lazily) would keep a stand-in from its
+    ``from .device import ...`` after the monkeypatch is undone, and hand it to later tests."""
+    import importlib
+    import importlib.util
+    import pkgutil
+    import finaletoolkit_b200 as F
+    for m in pkgutil.walk_packages(F.__path__, F.__name__ + "."):
+        if not m.name.endswith(".__main__") and importlib.util.find_spec(m.name).origin.endswith(".py"):
+            importlib.import_module(m.name)     # (the walk also lists libftk_b200.so, a ctypes library)
+
+
 def install(monkeypatch, seqs: dict):
     """``seqs``: {contig: ASCII reference sequence (bytes)} for the motif / DELFI wrappers."""
+    _import_whole_package()
     import finaletoolkit_b200.device as D
     from finaletoolkit_b200.io.fragments import FragmentTable
     from finaletoolkit_b200.io.reference import ReferenceWrapper

@@ -39,10 +39,22 @@ def test_abi_library_exports_every_declared_symbol():
 
 
 def test_no_cpu_fallback():
-    """Without CUDA every feature fails loudly instead of computing on the host."""
+    """Without CUDA every feature fails loudly instead of computing on the host.  On a machine with a GPU
+    the checks run in a child process that sees no device."""
     import torch
-    if torch.cuda.is_available():
-        pytest.skip("CUDA present")
+    if not torch.cuda.is_available():
+        _check_no_cpu_fallback()
+        return
+    code = (f"import sys; sys.path[:0] = {[REPO, os.path.join(REPO, 'tests')]!r}\n"
+            "import test_host_logic as t; t._check_no_cpu_fallback(); print('no cpu fallback ok')")
+    env = dict(os.environ, CUDA_VISIBLE_DEVICES="")
+    r = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True, timeout=600)
+    assert r.returncode == 0 and "no cpu fallback ok" in r.stdout, r.stdout[-2000:] + r.stderr[-2000:]
+
+
+def _check_no_cpu_fallback():
+    import torch
+    assert not torch.cuda.is_available()
     import finaletoolkit_b200 as F
     from finaletoolkit_b200._lib import FtkLibraryError
     cols = {"c": (np.array([1, 5]), np.array([150, 170]), np.array([60, 60]), np.array([1, 0]))}
