@@ -115,8 +115,6 @@ def lib():
                 raise FtkLibraryError(f"{SO_PATH} does not export {name}; rebuild it") from e
             fn.restype = res
             fn.argtypes = args
-        if os.environ.get("FTK_WPS_IMPL"):   # debug: pick a WPS kernel variant (csrc/ftk_wps.cu, g_wps_impl)
-            h.ftk_debug_set_wps_impl(int(os.environ["FTK_WPS_IMPL"]))
         _lib = h
     return _lib
 

@@ -19,12 +19,7 @@
 
 namespace ftk {
 
-constexpr int kWpsThreads = 256;
-constexpr int kWpsWarps = kWpsThreads / 32;
 constexpr int kWpsCap = 5120;                    // smem slots per tile
-constexpr int kWpsIters = kWpsCap / (kWpsThreads * 4);  // int4 groups per lane
-constexpr int kWpsSpan = kWpsIters * 128;        // positions per warp
-static_assert(kWpsIters * kWpsThreads * 4 == kWpsCap, "tile must split evenly");
 static_assert(FTK_WPS_TILE < kWpsCap, "one guard slot for odd windows");
 
 // Per-tile fragment index range [lo, hi): a superset of the fragments with any
@@ -58,7 +53,7 @@ wps_tile_ranges_kernel(const int32_t *__restrict__ frag_start, int64_t n_frag,
 }
 
 // ---------------------------------------------------------------------------
-// Pieces shared by the two tile kernels
+// Tile parameters, the fragment scatter and the score stores
 // ---------------------------------------------------------------------------
 struct WpsParams {
     int window, a, b;       // window [c-a, c+b]
@@ -126,9 +121,6 @@ __device__ __forceinline__ void wps_scatter(int *__restrict__ D, const WpsParams
     }
 }
 
-// Block prefix scan of D and the store of the tile.  Lane owns int4 groups, warp owns a
-// contiguous span, one barrier for the warp totals.  `sync` = the CTA-wide (or
-// consumer-wide) barrier of the calling kernel.
 // Store four consecutive scores.  int32: one 128-bit streaming store.  int16 (halves the
 // device->host bytes of the end-to-end path): one 64-bit store + a range check that raises
 // *overflow so the caller can redo the launch in int32 (|WPS| <= local depth, so this needs a
@@ -164,137 +156,8 @@ __device__ __forceinline__ void store1(int16_t *p, int v, int *overflow) {
     *p = (int16_t)v;
 }
 
-template <bool ODD, typename OutT, typename Sync>
-__device__ __forceinline__ void wps_scan_store(int *__restrict__ D, int *__restrict__ warp_tot,
-                                               const WpsParams &P, const TileCtx &T,
-                                               OutT *__restrict__ dst, int *overflow, int tid, Sync sync) {
-    const int lane = tid & 31, warp = tid >> 5;
-    int4 v[kWpsIters];
-    int carry = 0;
-    const int span0 = warp * kWpsSpan;
-#pragma unroll
-    for (int j = 0; j < kWpsIters; ++j) {
-        const int base = span0 + j * 128 + lane * 4;
-        int4 d = *reinterpret_cast<const int4 *>(&D[base]);
-        d.y += d.x; d.z += d.y; d.w += d.z;
-        int t = d.w;
-#pragma unroll
-        for (int off = 1; off < 32; off <<= 1) {
-            int n = __shfl_up_sync(0xffffffffu, t, off);
-            if (lane >= off) t += n;
-        }
-        const int excl = t - d.w + carry;
-        v[j] = make_int4(d.x + excl, d.y + excl, d.z + excl, d.w + excl);
-        carry += __shfl_sync(0xffffffffu, t, 31);
-    }
-    if (lane == 0) warp_tot[warp] = carry;
-    sync();
-    int offset = 0;
-#pragma unroll
-    for (int w = 0; w < kWpsWarps; ++w) offset += (w < warp) ? warp_tot[w] : 0;
-
-    if (!ODD) {
-        const bool aligned = ((reinterpret_cast<uintptr_t>(dst) & (4 * sizeof(OutT) - 1)) == 0);
-#pragma unroll
-        for (int j = 0; j < kWpsIters; ++j) {
-            const int base = span0 + j * 128 + lane * 4;
-            const int4 r = make_int4(v[j].x + offset, v[j].y + offset, v[j].z + offset, v[j].w + offset);
-            if (aligned && base + 3 < T.len) {
-                store4(dst + base, r, overflow);
-            } else {
-                if (base + 0 < T.len) store1(dst + base + 0, r.x, overflow);
-                if (base + 1 < T.len) store1(dst + base + 1, r.y, overflow);
-                if (base + 2 < T.len) store1(dst + base + 2, r.z, overflow);
-                if (base + 3 < T.len) store1(dst + base + 3, r.w, overflow);
-            }
-        }
-    } else {
-        // odd W: out[c] = G[c - ((c - a) & 1)]; stage G in shared memory (own span only)
-#pragma unroll
-        for (int j = 0; j < kWpsIters; ++j) {
-            const int base = span0 + j * 128 + lane * 4;
-            *reinterpret_cast<int4 *>(&D[base]) =
-                make_int4(v[j].x + offset, v[j].y + offset, v[j].z + offset, v[j].w + offset);
-        }
-        sync();
-        for (int k = tid; k < T.len; k += kWpsThreads) {
-            const int c = T.p0 + k;
-            store1(dst + k, D[c - ((c - P.a) & 1) - T.g0], overflow);
-        }
-        sync();  // D is recycled by the caller
-    }
-}
-
 // ---------------------------------------------------------------------------
-// Kernel A ("direct"): one CTA per tile, fragments streamed with 128-bit loads.
-// Kept as the simple variant (ftk_debug_set_wps_impl(1)); the pipelined kernels below are faster.
-// ---------------------------------------------------------------------------
-template <bool ODD, typename OutT>
-__global__ void __launch_bounds__(kWpsThreads)
-wps_tile_kernel(const int32_t *__restrict__ frag_start, const int32_t *__restrict__ frag_stop,
-                const uint8_t *__restrict__ frag_mapq,
-                const int32_t *__restrict__ tile_p0, const int32_t *__restrict__ tile_len,
-                const int32_t *__restrict__ tile_mid_lo, const int32_t *__restrict__ tile_mid_hi,
-                const int64_t *__restrict__ tile_out_off, const int64_t *__restrict__ ranges,
-                WpsParams P, OutT *__restrict__ out, int *__restrict__ overflow) {
-    __shared__ __align__(16) int D[kWpsCap];
-    __shared__ int warp_tot[kWpsWarps];
-
-    const int tid = threadIdx.x;
-    const int64_t tile = blockIdx.x;
-    const TileCtx T = make_tile_ctx<ODD>(P, tile_p0[tile], tile_len[tile], tile_mid_lo[tile], tile_mid_hi[tile]);
-    const int64_t lo = ranges[2 * tile];
-    const int64_t hi = ranges[2 * tile + 1];
-
-    // The fragment slice [lo, hi) is widened to a 16-byte boundary on the left (extra
-    // fragments are harmless: the range is only a superset) so every lane streams 4
-    // fragments per 128-bit load: 3 loads per 4 fragments, 32-bit indexing.
-    const int64_t lo_al = lo & ~(int64_t)3;
-    const int cnt = (int)(hi - lo_al);
-    const int nvec = cnt >> 2;
-    const int4 *__restrict__ vs = reinterpret_cast<const int4 *>(frag_start + lo_al);
-    const int4 *__restrict__ ve = reinterpret_cast<const int4 *>(frag_stop + lo_al);
-    const uchar4 *__restrict__ vq = reinterpret_cast<const uchar4 *>(frag_mapq ? frag_mapq + lo_al : nullptr);
-
-    // first batch of loads is issued before the tile is zeroed so its latency hides behind that
-    int4 s0 = make_int4(0, 0, 0, 0), e0 = make_int4(-1, -1, -1, -1);
-    uchar4 q0 = make_uchar4(255, 255, 255, 255);
-    if (tid < nvec) {
-        s0 = __ldcs(vs + tid);
-        e0 = __ldcs(ve + tid);
-        if (vq) q0 = __ldcs(vq + tid);
-    }
-#pragma unroll
-    for (int j = 0; j < kWpsIters; ++j)
-        reinterpret_cast<int4 *>(D)[j * kWpsThreads + tid] = make_int4(0, 0, 0, 0);
-    __syncthreads();
-
-    for (int v = tid; v < nvec; v += kWpsThreads) {
-        const int4 s = s0, e = e0;
-        const uchar4 q = q0;
-        const int vn = v + kWpsThreads;
-        if (vn < nvec) {  // prefetch the next vector triple while this one turns into atomics
-            s0 = __ldcs(vs + vn);
-            e0 = __ldcs(ve + vn);
-            if (vq) q0 = __ldcs(vq + vn);
-        }
-        wps_scatter(D, P, T, s.x, e.x, q.x);
-        wps_scatter(D, P, T, s.y, e.y, q.y);
-        wps_scatter(D, P, T, s.z, e.z, q.z);
-        wps_scatter(D, P, T, s.w, e.w, q.w);
-    }
-    {   // tail: at most 3 fragments
-        const int i = nvec * 4 + tid;
-        if (i < cnt)
-            wps_scatter(D, P, T, __ldcs(frag_start + lo_al + i), __ldcs(frag_stop + lo_al + i),
-                        frag_mapq ? (int)__ldcs(frag_mapq + lo_al + i) : 255);
-    }
-    __syncthreads();
-    wps_scan_store<ODD>(D, warp_tot, P, T, out + tile_out_off[tile], overflow, tid, [] { __syncthreads(); });
-}
-
-// ---------------------------------------------------------------------------
-// Pieces shared by the persistent, warp-specialised, TMA-fed kernels below.
+// The WPS kernel: persistent, warp-specialised, TMA-fed.
 //
 // A producer lane runs ahead of the consumer warps: it reads the next tile's descriptor and
 // fragment range and issues 1-D bulk async copies (cp.async.bulk ... mbarrier::complete_tx::bytes,
@@ -302,8 +165,40 @@ wps_tile_kernel(const int32_t *__restrict__ frag_start, const int32_t *__restric
 // consumers wait on the buffer's "full" mbarrier, turn the staged fragments into shared atomics,
 // release the buffer through its "empty" mbarrier, then scan and store the tile - while the next
 // tile's bytes are already in flight.  HBM latency is therefore never exposed to the compute warps.
+//
+// The consumer warps form groups of four, each with its own difference array, its own staging
+// buffer and its own named barrier; producer warp p feeds groups 2p and 2p+1 alternately.  While
+// one group scans and stores its tile the other one is scattering the next, so the barrier / phase
+// latency of a tile is overlapped inside the CTA instead of across CTAs.  Both shapes keep six
+// tiles in flight per SM:
+//   * plain WPS: two groups and one producer warp per CTA, three CTAs per SM;
+//   * fused pass (FUSE): six groups and three producer warps, ONE CTA per SM.  The SM's shared
+//     memory is then one allocation: the 2 KB the two extra CTAs lose to the per-CTA reservation
+//     plus the slack at the end leave room for a CTA-wide 1024-bin length histogram, which is what
+//     lets the step make ONE pass over the fragments:
+//       - per-interval coverage (frag/_coverage.py:117-130, midpoint policy): a fragment's midpoint
+//         lies in exactly one tile of an interval, so the count of an interval is the sum of its
+//         tiles' counts - a register count per lane, one shuffle reduction and one 64-bit atomic
+//         per warp and tile;
+//       - pooled length histogram of the counted fragments (frag/_frag_length.py:147-153): shared
+//         atomics on the CTA's histogram, flushed once with 64-bit global atomics when the CTA
+//         ends (a CTA sees < 2^31 fragments: n_frag <= INT32_MAX).
+//     The coverage predicate has its own length window and mapq cut; the staged range is widened
+//     on the left so that every fragment whose midpoint can fall into the tile is staged.
 // ---------------------------------------------------------------------------
-constexpr int kStreamFrags = 1920;        // fragments per staging buffer (multiple of 16)
+constexpr int kStreamFrags = 1920;                   // fragments per staging buffer (multiple of 16)
+constexpr int kGroupWarps = 4;
+constexpr int kGroupThreads = kGroupWarps * 32;
+constexpr int kScanHalf = kWpsCap / 2;               // slots scanned per pass
+constexpr int kWpsSpan = kScanHalf / kGroupWarps;    // positions per warp and pass
+constexpr int kWpsIters = kWpsSpan / 128;            // int4 groups per lane and pass
+static_assert(2 * kWpsIters * kGroupThreads * 4 == kWpsCap, "tile must split evenly");
+constexpr int kPlainGroups = 2;
+constexpr int kFusedGroups = 6;
+constexpr int kFuseBins = 1024;                      // lengths below this are privatised in shared memory
+
+template <int GROUPS> constexpr int kStreamThreads = GROUPS * kGroupThreads + 32 * (GROUPS / 2);
+template <int GROUPS> constexpr int kStreamCtasPerSm = 6 / GROUPS;
 
 struct __align__(16) StreamDesc {
     int tile;        // -1: no more work
@@ -313,6 +208,19 @@ struct __align__(16) StreamDesc {
     int ivl;         // interval the tile belongs to (fused coverage counts); bit 31 = its first tile
     long long out_off;
     long long tail_lo, tail_hi;  // ragged end of the contig, read straight from global (rare)
+};
+
+template <int GROUPS, bool FUSE>
+struct __align__(128) StreamSmem {
+    int D[GROUPS][kWpsCap];
+    int start[GROUPS][kStreamFrags];
+    int stop[GROUPS][kStreamFrags];
+    unsigned char mapq[GROUPS][kStreamFrags];
+    StreamDesc desc[GROUPS];
+    unsigned long long full_bar[GROUPS];
+    unsigned long long empty_bar[GROUPS];
+    int warp_tot[GROUPS][kGroupWarps];
+    int hist[FUSE ? kFuseBins : 1];
 };
 
 __device__ __forceinline__ uint32_t smem_u32(const void *p) {
@@ -348,36 +256,13 @@ __device__ __forceinline__ void bulk_g2s(void *dst, const void *src, unsigned by
                  :: "r"(smem_u32(dst)), "l"(src), "r"(bytes), "r"(smem_u32(bar)) : "memory");
 }
 
-// ---------------------------------------------------------------------------
-// Kernel C ("dual", default for plain WPS): two tiles in flight per CTA.
-// The eight consumer warps are split into two groups of four, each with its own difference
-// array, its own staging buffer and its own named barrier; the producer warp feeds the groups
-// alternately.  While one group scans and stores its tile the other one is scattering the next,
-// so the barrier / phase latency of a tile is overlapped inside the CTA instead of across CTAs.
-// ---------------------------------------------------------------------------
-constexpr int kDualWarps = 4;
-constexpr int kDualGroupThreads = kDualWarps * 32;
-constexpr int kDualThreads = 2 * kDualGroupThreads + 32;
-constexpr int kDualCtasPerSm = 3;
-constexpr int kDualHalf = kWpsCap / 2;              // slots scanned per pass (4 warps x 640)
-
-struct __align__(128) DualSmem {
-    int D[2][kWpsCap];
-    int start[2][kStreamFrags];
-    int stop[2][kStreamFrags];
-    unsigned char mapq[2][kStreamFrags];
-    StreamDesc desc[2];
-    unsigned long long full_bar[2];
-    unsigned long long empty_bar[2];
-    int warp_tot[2][kDualWarps];
-};
-
 __device__ __forceinline__ void group_sync(int g) {
-    asm volatile("bar.sync %0, %1;" :: "r"(1 + g), "n"(kDualGroupThreads) : "memory");
+    asm volatile("bar.sync %0, %1;" :: "r"(1 + g), "n"(kGroupThreads) : "memory");
 }
 
-// Scan + store by one 4-warp group in two passes of kDualHalf slots (same lane layout as
-// wps_scan_store, so the stores stay coalesced and the register footprint stays at 5 int4).
+// Block prefix scan of D and the store of the tile by one 4-warp group, in two passes of kScanHalf
+// slots.  Lane owns int4 groups, warp owns a contiguous span, one barrier for the warp totals of a
+// pass; the stores stay coalesced and the register footprint stays at 5 int4.
 template <bool ODD, typename OutT>
 __device__ __forceinline__ void wps_scan_store_group(int *__restrict__ D, int *__restrict__ warp_tot,
                                                      const WpsParams &P, const TileCtx &T,
@@ -389,7 +274,7 @@ __device__ __forceinline__ void wps_scan_store_group(int *__restrict__ D, int *_
     for (int half = 0; half < 2; ++half) {
         int4 v[kWpsIters];
         int carry = 0;
-        const int span0 = half * kDualHalf + warp * kWpsSpan;
+        const int span0 = half * kScanHalf + warp * kWpsSpan;
 #pragma unroll
         for (int j = 0; j < kWpsIters; ++j) {
             const int base = span0 + j * 128 + lane * 4;
@@ -409,7 +294,7 @@ __device__ __forceinline__ void wps_scan_store_group(int *__restrict__ D, int *_
         group_sync(g);
         int offset = base_carry, total = 0;
 #pragma unroll
-        for (int w = 0; w < kDualWarps; ++w) {
+        for (int w = 0; w < kGroupWarps; ++w) {
             const int wt = warp_tot[w];
             offset += (w < warp) ? wt : 0;
             total += wt;
@@ -433,7 +318,8 @@ __device__ __forceinline__ void wps_scan_store_group(int *__restrict__ D, int *_
         group_sync(g);   // warp_tot is rewritten by the next pass / D by the next tile
     }
     if (ODD) {
-        for (int k = gt; k < T.len; k += kDualGroupThreads) {
+        // odd W: out[c] = G[c - ((c - a) & 1)]
+        for (int k = gt; k < T.len; k += kGroupThreads) {
             const int c = T.p0 + k;
             store1(dst + k, D[c - ((c - P.a) & 1) - T.g0], overflow);
         }
@@ -441,168 +327,12 @@ __device__ __forceinline__ void wps_scan_store_group(int *__restrict__ D, int *_
     }
 }
 
-template <bool ODD, typename OutT>
-__global__ void __launch_bounds__(kDualThreads, kDualCtasPerSm)
-wps_dual_kernel(const int32_t *__restrict__ frag_start, const int32_t *__restrict__ frag_stop,
-                const uint8_t *__restrict__ frag_mapq, int64_t n_frag,
-                const int32_t *__restrict__ tile_p0, const int32_t *__restrict__ tile_len,
-                const int32_t *__restrict__ tile_mid_lo, const int32_t *__restrict__ tile_mid_hi,
-                const int64_t *__restrict__ tile_out_off, const int64_t *__restrict__ ranges,
-                int n_tiles, WpsParams P, OutT *__restrict__ out, int *__restrict__ overflow) {
-    extern __shared__ __align__(128) unsigned char smem_raw[];
-    DualSmem &S = *reinterpret_cast<DualSmem *>(smem_raw);
-    const int tid = threadIdx.x;
-
-    if (tid == 0) {
-#pragma unroll
-        for (int g = 0; g < 2; ++g) {
-            mbar_init(&S.full_bar[g], 1);
-            mbar_init(&S.empty_bar[g], 1);
-        }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-
-    if (tid >= 2 * kDualGroupThreads) {
-        // ===================== producer warp (one elected lane) =====================
-        if (tid == 2 * kDualGroupThreads) {
-            unsigned ph[2] = {0u, 0u};
-            const int64_t n16 = n_frag & ~(int64_t)15;
-            int j = 0;
-            for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, ++j) {
-                const int g = j & 1;
-                const int64_t lo = ranges[2 * (int64_t)tile], hi = ranges[2 * (int64_t)tile + 1];
-                const int p0 = tile_p0[tile], len = tile_len[tile];
-                const int mlo = tile_mid_lo[tile], mhi = tile_mid_hi[tile];
-                const long long ooff = tile_out_off[tile];
-                const int64_t lo16 = lo & ~(int64_t)15;
-                int64_t hi16 = (hi + 15) & ~(int64_t)15;
-                if (hi16 > n16) hi16 = n16;
-                if (hi16 < lo16) hi16 = lo16;
-                const int64_t t_lo = (hi16 > lo16) ? hi16 : lo16;
-                const bool has_tail = hi > t_lo;
-                const int64_t span = hi16 - lo16;
-                const int n_chunks = span > 0 ? (int)((span + kStreamFrags - 1) / kStreamFrags) : 1;
-                for (int c = 0; c < n_chunks; ++c) {
-                    mbar_wait(&S.empty_bar[g], ph[g] ^ 1u);
-                    const int64_t c0 = lo16 + (int64_t)c * kStreamFrags;
-                    const int n = (int)min((int64_t)kStreamFrags, hi16 - c0);
-                    StreamDesc &d = S.desc[g];
-                    d.tile = tile; d.p0 = p0; d.len = len; d.mid_lo = mlo; d.mid_hi = mhi;
-                    d.n = n > 0 ? n : 0;
-                    d.first = (c == 0); d.last = (c == n_chunks - 1);
-                    d.out_off = ooff;
-                    d.tail_lo = (d.last && has_tail) ? t_lo : 0;
-                    d.tail_hi = (d.last && has_tail) ? hi : 0;
-                    if (n > 0) {
-                        const unsigned bytes = (unsigned)n * (frag_mapq ? 9u : 8u);
-                        mbar_arrive_expect_tx(&S.full_bar[g], bytes);
-                        bulk_g2s(S.start[g], frag_start + c0, (unsigned)n * 4u, &S.full_bar[g]);
-                        bulk_g2s(S.stop[g], frag_stop + c0, (unsigned)n * 4u, &S.full_bar[g]);
-                        if (frag_mapq) bulk_g2s(S.mapq[g], frag_mapq + c0, (unsigned)n, &S.full_bar[g]);
-                    } else {
-                        mbar_arrive(&S.full_bar[g]);
-                    }
-                    ph[g] ^= 1u;
-                }
-            }
-#pragma unroll 1
-            for (int g = 0; g < 2; ++g) {
-                mbar_wait(&S.empty_bar[g], ph[g] ^ 1u);
-                S.desc[g].tile = -1;
-                mbar_arrive(&S.full_bar[g]);
-            }
-        }
-        return;
-    }
-
-    // ========================= consumer groups =========================
-    const int g = tid / kDualGroupThreads;
-    const int gt = tid - g * kDualGroupThreads;
-    int *__restrict__ D = S.D[g];
-    unsigned phase = 0;
-    TileCtx T = make_tile_ctx<ODD>(P, 0, 0, 0, 0);
-    for (;;) {
-        mbar_wait(&S.full_bar[g], phase);
-        const StreamDesc d = S.desc[g];
-        if (d.tile < 0) break;
-        if (d.first) {
-            T = make_tile_ctx<ODD>(P, d.p0, d.len, d.mid_lo, d.mid_hi);
-#pragma unroll
-            for (int j = 0; j < kWpsCap / (4 * kDualGroupThreads); ++j)
-                reinterpret_cast<int4 *>(D)[j * kDualGroupThreads + gt] = make_int4(0, 0, 0, 0);
-            group_sync(g);
-        }
-        const int nvec = d.n >> 2;
-        const int4 *__restrict__ vs = reinterpret_cast<const int4 *>(S.start[g]);
-        const int4 *__restrict__ ve = reinterpret_cast<const int4 *>(S.stop[g]);
-        const uchar4 *__restrict__ vq = reinterpret_cast<const uchar4 *>(S.mapq[g]);
-        for (int v = gt; v < nvec; v += kDualGroupThreads) {
-            const int4 s = vs[v], e = ve[v];
-            const uchar4 q = frag_mapq ? vq[v] : make_uchar4(255, 255, 255, 255);
-            wps_scatter(D, P, T, s.x, e.x, q.x);
-            wps_scatter(D, P, T, s.y, e.y, q.y);
-            wps_scatter(D, P, T, s.z, e.z, q.z);
-            wps_scatter(D, P, T, s.w, e.w, q.w);
-        }
-        if (d.tail_hi > d.tail_lo) {
-            const int64_t i = d.tail_lo + gt;
-            if (i < d.tail_hi)
-                wps_scatter(D, P, T, __ldcs(frag_start + i), __ldcs(frag_stop + i),
-                            frag_mapq ? (int)__ldcs(frag_mapq + i) : 255);
-        }
-        group_sync(g);                                   // scatter done; the staging buffer is free
-        if (gt == 0) mbar_arrive(&S.empty_bar[g]);
-        if (d.last)
-            wps_scan_store_group<ODD>(D, S.warp_tot[g], P, T, out + d.out_off, overflow, gt, g);
-        phase ^= 1u;
-    }
-}
-
-
-// ---------------------------------------------------------------------------
-// Kernel D ("hex"; the one with the fused coverage / length-histogram pass):
-// ONE persistent CTA per SM with SIX consumer groups of four warps and THREE producer warps
-// (producer p feeds groups 2p and 2p+1 exactly like the producer of the dual kernel feeds its
-// two).  Six tiles are in flight per SM as with three dual CTAs, but the SM's shared memory is
-// one allocation: the 2 KB the two extra CTAs lost to the per-CTA reservation plus the slack at
-// the end leave room for a CTA-wide 1024-bin length histogram, which is what lets the step make
-// ONE pass over the fragments (FUSE):
-//   * per-interval coverage (frag/_coverage.py:117-130, midpoint policy): a fragment's midpoint
-//     lies in exactly one tile of an interval, so the count of an interval is the sum of its
-//     tiles' counts - a register count per lane, one shuffle reduction and one 64-bit atomic per
-//     warp and tile;
-//   * pooled length histogram of the counted fragments (frag/_frag_length.py:147-153): shared
-//     atomics on the CTA's histogram, flushed once with 64-bit global atomics when the CTA ends
-//     (a CTA sees < 2^31 fragments: n_frag <= INT32_MAX).
-// The coverage predicate has its own length window and mapq cut; the staged range is widened
-// on the left so that every fragment whose midpoint can fall into the tile is staged.
-// ---------------------------------------------------------------------------
-constexpr int kHexGroups = 6;
-constexpr int kHexProducers = kHexGroups / 2;
-constexpr int kHexConsumerThreads = kHexGroups * kDualGroupThreads;
-constexpr int kHexThreads = kHexConsumerThreads + 32 * kHexProducers;
-constexpr int kFuseBins = 1024;           // lengths below this are privatised in shared memory
-
 struct CovParams {
     int len_lo;
     unsigned len_span;
     int min_mapq;
     int n_bins;             // 0: no histogram
 };
-
-struct __align__(128) HexSmem {
-    int D[kHexGroups][kWpsCap];
-    int start[kHexGroups][kStreamFrags];
-    int stop[kHexGroups][kStreamFrags];
-    unsigned char mapq[kHexGroups][kStreamFrags];
-    StreamDesc desc[kHexGroups];
-    unsigned long long full_bar[kHexGroups];
-    unsigned long long empty_bar[kHexGroups];
-    int warp_tot[kHexGroups][kDualWarps];
-    int hist[kFuseBins];
-};
-static_assert(sizeof(HexSmem) <= 227 * 1024, "HexSmem must fit the 227 KB a CTA may own on sm_100a");
 
 // Coverage / histogram side of one staged fragment: the stream of region [p0, p0+len) under the
 // midpoint policy (io/alignment.py:270-302 overlap rows: stop > S; utils/_frag_generator.py:117-123).
@@ -628,171 +358,173 @@ struct TileRec {
     int tile, p0, len, mlo, mhi, ivl;
 };
 
-template <bool ODD, typename OutT, bool FUSE>
-__global__ void __launch_bounds__(kHexThreads, 1)
-wps_hex_kernel(const int32_t *__restrict__ frag_start, const int32_t *__restrict__ frag_stop,
-               const uint8_t *__restrict__ frag_mapq, int64_t n_frag,
-               const int32_t *__restrict__ tile_p0, const int32_t *__restrict__ tile_len,
-               const int32_t *__restrict__ tile_mid_lo, const int32_t *__restrict__ tile_mid_hi,
-               const int64_t *__restrict__ tile_out_off, const int32_t *__restrict__ tile_ivl,
-               const int64_t *__restrict__ ranges, int n_tiles, WpsParams P, CovParams C,
-               OutT *__restrict__ out, int *__restrict__ overflow,
-               unsigned long long *__restrict__ counts, unsigned long long *__restrict__ ghist) {
+template <bool ODD, typename OutT, int GROUPS, bool FUSE>
+__global__ void __launch_bounds__(kStreamThreads<GROUPS>, kStreamCtasPerSm<GROUPS>)
+wps_stream_kernel(const int32_t *__restrict__ frag_start, const int32_t *__restrict__ frag_stop,
+                  const uint8_t *__restrict__ frag_mapq, int64_t n_frag,
+                  const int32_t *__restrict__ tile_p0, const int32_t *__restrict__ tile_len,
+                  const int32_t *__restrict__ tile_mid_lo, const int32_t *__restrict__ tile_mid_hi,
+                  const int64_t *__restrict__ tile_out_off, const int32_t *__restrict__ tile_ivl,
+                  const int64_t *__restrict__ ranges, int n_tiles, WpsParams P, CovParams C,
+                  OutT *__restrict__ out, int *__restrict__ overflow,
+                  unsigned long long *__restrict__ counts, unsigned long long *__restrict__ ghist) {
+    constexpr int kConsumerThreads = GROUPS * kGroupThreads;
     extern __shared__ __align__(128) unsigned char smem_raw[];
-    HexSmem &S = *reinterpret_cast<HexSmem *>(smem_raw);
+    StreamSmem<GROUPS, FUSE> &S = *reinterpret_cast<StreamSmem<GROUPS, FUSE> *>(smem_raw);
     const int tid = threadIdx.x;
 
     if (tid == 0) {
 #pragma unroll
-        for (int g = 0; g < kHexGroups; ++g) {
+        for (int g = 0; g < GROUPS; ++g) {
             mbar_init(&S.full_bar[g], 1);
             mbar_init(&S.empty_bar[g], 1);
         }
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     if (FUSE) {
-        for (int b = tid; b < kFuseBins; b += kHexThreads) S.hist[b] = 0;
+        for (int b = tid; b < kFuseBins; b += kStreamThreads<GROUPS>) S.hist[b] = 0;
     }
     __syncthreads();
 
-    if (tid >= kHexConsumerThreads) {
-        // ============ producer warps (one elected lane each, two groups per producer) ============
-        const int pt = tid - kHexConsumerThreads;
-        if ((pt & 31) == 0) {
-            const int p = pt >> 5;
-            unsigned ph[2] = {0u, 0u};
-            const int64_t n16 = n_frag & ~(int64_t)15;
-            // the CTA's k-th tile is blockIdx.x + k * gridDim.x and goes to group k % 6; this
-            // producer's j-th tile is k = 6 * (j / 2) + 2p + (j & 1)
-            auto fetch = [&](int j, TileRec &r) -> bool {
-                const int64_t k = 6 * (int64_t)(j >> 1) + 2 * p + (j & 1);
-                const int64_t tile = blockIdx.x + k * (int64_t)gridDim.x;
-                if (tile >= n_tiles) return false;
-                r.tile = (int)tile;
-                r.lo = ranges[2 * tile]; r.hi = ranges[2 * tile + 1];
-                r.p0 = tile_p0[tile]; r.len = tile_len[tile];
-                r.mlo = tile_mid_lo[tile]; r.mhi = tile_mid_hi[tile];
-                r.ooff = tile_out_off[tile];
-                r.ivl = FUSE ? tile_ivl[tile] : 0;
-                return true;
-            };
-            TileRec r, rn;
-            bool have = fetch(0, r);
-            for (int j = 0; have; ++j) {
-                // the next tile's descriptor loads are in flight while this tile waits for its buffer
-                const bool have_next = fetch(j + 1, rn);
-                const int sub = j & 1;
-                const int g = 2 * p + sub;
-                const int64_t lo16 = r.lo & ~(int64_t)15;
-                int64_t hi16 = (r.hi + 15) & ~(int64_t)15;
-                if (hi16 > n16) hi16 = n16;
-                if (hi16 < lo16) hi16 = lo16;
-                const int64_t t_lo = (hi16 > lo16) ? hi16 : lo16;
-                const bool has_tail = r.hi > t_lo;
-                const int64_t span = hi16 - lo16;
-                const int n_chunks = span > 0 ? (int)((span + kStreamFrags - 1) / kStreamFrags) : 1;
-                for (int c = 0; c < n_chunks; ++c) {
-                    mbar_wait(&S.empty_bar[g], ph[sub] ^ 1u);
-                    const int64_t c0 = lo16 + (int64_t)c * kStreamFrags;
-                    const int n = (int)min((int64_t)kStreamFrags, hi16 - c0);
-                    StreamDesc &d = S.desc[g];
-                    d.tile = r.tile; d.p0 = r.p0; d.len = r.len; d.mid_lo = r.mlo; d.mid_hi = r.mhi;
-                    d.n = n > 0 ? n : 0;
-                    d.first = (c == 0); d.last = (c == n_chunks - 1);
-                    d.ivl = r.ivl;
-                    d.out_off = r.ooff;
-                    d.tail_lo = (d.last && has_tail) ? t_lo : 0;
-                    d.tail_hi = (d.last && has_tail) ? r.hi : 0;
-                    if (n > 0) {
-                        const unsigned bytes = (unsigned)n * (frag_mapq ? 9u : 8u);
-                        mbar_arrive_expect_tx(&S.full_bar[g], bytes);
-                        bulk_g2s(S.start[g], frag_start + c0, (unsigned)n * 4u, &S.full_bar[g]);
-                        bulk_g2s(S.stop[g], frag_stop + c0, (unsigned)n * 4u, &S.full_bar[g]);
-                        if (frag_mapq) bulk_g2s(S.mapq[g], frag_mapq + c0, (unsigned)n, &S.full_bar[g]);
-                    } else {
-                        mbar_arrive(&S.full_bar[g]);
-                    }
-                    ph[sub] ^= 1u;
-                }
-                r = rn;
-                have = have_next;
+    if (tid < kConsumerThreads) {
+        // ========================= consumer groups =========================
+        const int g = tid / kGroupThreads;
+        const int gt = tid - g * kGroupThreads;
+        int *__restrict__ D = S.D[g];
+        unsigned phase = 0;
+        int cnt = 0;
+        TileCtx T = make_tile_ctx<ODD>(P, 0, 0, 0, 0);
+        for (;;) {
+            mbar_wait(&S.full_bar[g], phase);
+            const StreamDesc d = S.desc[g];
+            if (d.tile < 0) break;
+            if (d.first) {
+                T = make_tile_ctx<ODD>(P, d.p0, d.len, d.mid_lo, d.mid_hi);
+                if (FUSE && d.ivl < 0) T.zl_excl = d.p0;
+                cnt = 0;
+#pragma unroll
+                for (int j = 0; j < kWpsCap / (4 * kGroupThreads); ++j)
+                    reinterpret_cast<int4 *>(D)[j * kGroupThreads + gt] = make_int4(0, 0, 0, 0);
+                group_sync(g);
             }
-#pragma unroll 1
-            for (int sub = 0; sub < 2; ++sub) {
-                const int g = 2 * p + sub;
-                mbar_wait(&S.empty_bar[g], ph[sub] ^ 1u);
-                S.desc[g].tile = -1;
-                mbar_arrive(&S.full_bar[g]);
+            const int nvec = d.n >> 2;
+            const int4 *__restrict__ vs = reinterpret_cast<const int4 *>(S.start[g]);
+            const int4 *__restrict__ ve = reinterpret_cast<const int4 *>(S.stop[g]);
+            const uchar4 *__restrict__ vq = reinterpret_cast<const uchar4 *>(S.mapq[g]);
+            for (int v = gt; v < nvec; v += kGroupThreads) {
+                const int4 s = vs[v], e = ve[v];
+                const uchar4 q = frag_mapq ? vq[v] : make_uchar4(255, 255, 255, 255);
+                wps_scatter(D, P, T, s.x, e.x, q.x);
+                wps_scatter(D, P, T, s.y, e.y, q.y);
+                wps_scatter(D, P, T, s.z, e.z, q.z);
+                wps_scatter(D, P, T, s.w, e.w, q.w);
+                if (FUSE) {
+                    cov_visit(S.hist, ghist, C, T, s.x, e.x, q.x, cnt);
+                    cov_visit(S.hist, ghist, C, T, s.y, e.y, q.y, cnt);
+                    cov_visit(S.hist, ghist, C, T, s.z, e.z, q.z, cnt);
+                    cov_visit(S.hist, ghist, C, T, s.w, e.w, q.w, cnt);
+                }
+            }
+            if (d.tail_hi > d.tail_lo) {
+                const int64_t i = d.tail_lo + gt;
+                if (i < d.tail_hi) {
+                    const int fs = __ldcs(frag_start + i), fe = __ldcs(frag_stop + i);
+                    const int q = frag_mapq ? (int)__ldcs(frag_mapq + i) : 255;
+                    wps_scatter(D, P, T, fs, fe, q);
+                    if (FUSE) cov_visit(S.hist, ghist, C, T, fs, fe, q, cnt);
+                }
+            }
+            group_sync(g);                                   // scatter done; the staging buffer is free
+            if (gt == 0) mbar_arrive(&S.empty_bar[g]);
+            if (d.last) {
+                if (FUSE) {
+                    const int c = __reduce_add_sync(0xffffffffu, cnt);
+                    if ((gt & 31) == 0 && c) atomicAdd(&counts[d.ivl & 0x7fffffff], (unsigned long long)c);
+                }
+                wps_scan_store_group<ODD>(D, S.warp_tot[g], P, T, out + d.out_off, overflow, gt, g);
+            }
+            phase ^= 1u;
+        }
+        if (FUSE && C.n_bins > 0) {
+            // all consumer groups are done: flush the CTA's histogram (the producers have exited)
+            asm volatile("bar.sync %0, %1;" :: "n"(GROUPS + 1), "n"(kConsumerThreads) : "memory");
+            const int nb = min(C.n_bins, kFuseBins);
+            for (int b = tid; b < nb; b += kConsumerThreads) {
+                const int v = S.hist[b];
+                if (v) atomicAdd(&ghist[b], (unsigned long long)v);
             }
         }
         return;
     }
 
-    // ========================= consumer groups =========================
-    const int g = tid / kDualGroupThreads;
-    const int gt = tid - g * kDualGroupThreads;
-    int *__restrict__ D = S.D[g];
-    unsigned phase = 0;
-    int cnt = 0;
-    TileCtx T = make_tile_ctx<ODD>(P, 0, 0, 0, 0);
-    for (;;) {
-        mbar_wait(&S.full_bar[g], phase);
-        const StreamDesc d = S.desc[g];
-        if (d.tile < 0) break;
-        if (d.first) {
-            T = make_tile_ctx<ODD>(P, d.p0, d.len, d.mid_lo, d.mid_hi);
-            if (FUSE && d.ivl < 0) T.zl_excl = d.p0;
-            cnt = 0;
-#pragma unroll
-            for (int j = 0; j < kWpsCap / (4 * kDualGroupThreads); ++j)
-                reinterpret_cast<int4 *>(D)[j * kDualGroupThreads + gt] = make_int4(0, 0, 0, 0);
-            group_sync(g);
-        }
-        const int nvec = d.n >> 2;
-        const int4 *__restrict__ vs = reinterpret_cast<const int4 *>(S.start[g]);
-        const int4 *__restrict__ ve = reinterpret_cast<const int4 *>(S.stop[g]);
-        const uchar4 *__restrict__ vq = reinterpret_cast<const uchar4 *>(S.mapq[g]);
-        for (int v = gt; v < nvec; v += kDualGroupThreads) {
-            const int4 s = vs[v], e = ve[v];
-            const uchar4 q = frag_mapq ? vq[v] : make_uchar4(255, 255, 255, 255);
-            wps_scatter(D, P, T, s.x, e.x, q.x);
-            wps_scatter(D, P, T, s.y, e.y, q.y);
-            wps_scatter(D, P, T, s.z, e.z, q.z);
-            wps_scatter(D, P, T, s.w, e.w, q.w);
-            if (FUSE) {
-                cov_visit(S.hist, ghist, C, T, s.x, e.x, q.x, cnt);
-                cov_visit(S.hist, ghist, C, T, s.y, e.y, q.y, cnt);
-                cov_visit(S.hist, ghist, C, T, s.z, e.z, q.z, cnt);
-                cov_visit(S.hist, ghist, C, T, s.w, e.w, q.w, cnt);
+    // ============ producer warps (one elected lane each, two groups per producer) ============
+    const int pt = tid - kConsumerThreads;
+    if ((pt & 31) == 0) {
+        const int p = pt >> 5;
+        // bit sub: phase of group 2p + sub (a runtime-indexed array would live in local memory)
+        unsigned ph = 0u;
+        const int64_t n16 = n_frag & ~(int64_t)15;
+        // the CTA's k-th tile is blockIdx.x + k * gridDim.x and goes to group k % GROUPS; this
+        // producer's j-th tile is k = GROUPS * (j / 2) + 2p + (j & 1)
+        auto fetch = [&](int j, TileRec &r) -> bool {
+            const int64_t k = GROUPS * (int64_t)(j >> 1) + 2 * p + (j & 1);
+            const int64_t tile = blockIdx.x + k * (int64_t)gridDim.x;
+            if (tile >= n_tiles) return false;
+            r.tile = (int)tile;
+            r.lo = ranges[2 * tile]; r.hi = ranges[2 * tile + 1];
+            r.p0 = tile_p0[tile]; r.len = tile_len[tile];
+            r.mlo = tile_mid_lo[tile]; r.mhi = tile_mid_hi[tile];
+            r.ooff = tile_out_off[tile];
+            r.ivl = FUSE ? tile_ivl[tile] : 0;
+            return true;
+        };
+        TileRec r, rn;
+        bool have = fetch(0, r);
+        for (int j = 0; have; ++j) {
+            // the next tile's descriptor loads are in flight while this tile waits for its buffer
+            const bool have_next = fetch(j + 1, rn);
+            const int sub = j & 1;
+            const int g = 2 * p + sub;
+            const int64_t lo16 = r.lo & ~(int64_t)15;
+            int64_t hi16 = (r.hi + 15) & ~(int64_t)15;
+            if (hi16 > n16) hi16 = n16;
+            if (hi16 < lo16) hi16 = lo16;
+            const int64_t t_lo = (hi16 > lo16) ? hi16 : lo16;
+            const bool has_tail = r.hi > t_lo;
+            const int64_t span = hi16 - lo16;
+            const int n_chunks = span > 0 ? (int)((span + kStreamFrags - 1) / kStreamFrags) : 1;
+            for (int c = 0; c < n_chunks; ++c) {
+                mbar_wait(&S.empty_bar[g], ((ph >> sub) & 1u) ^ 1u);
+                const int64_t c0 = lo16 + (int64_t)c * kStreamFrags;
+                const int n = (int)min((int64_t)kStreamFrags, hi16 - c0);
+                StreamDesc &d = S.desc[g];
+                d.tile = r.tile; d.p0 = r.p0; d.len = r.len; d.mid_lo = r.mlo; d.mid_hi = r.mhi;
+                d.n = n > 0 ? n : 0;
+                d.first = (c == 0); d.last = (c == n_chunks - 1);
+                d.ivl = r.ivl;
+                d.out_off = r.ooff;
+                d.tail_lo = (d.last && has_tail) ? t_lo : 0;
+                d.tail_hi = (d.last && has_tail) ? r.hi : 0;
+                if (n > 0) {
+                    const unsigned bytes = (unsigned)n * (frag_mapq ? 9u : 8u);
+                    mbar_arrive_expect_tx(&S.full_bar[g], bytes);
+                    bulk_g2s(S.start[g], frag_start + c0, (unsigned)n * 4u, &S.full_bar[g]);
+                    bulk_g2s(S.stop[g], frag_stop + c0, (unsigned)n * 4u, &S.full_bar[g]);
+                    if (frag_mapq) bulk_g2s(S.mapq[g], frag_mapq + c0, (unsigned)n, &S.full_bar[g]);
+                } else {
+                    mbar_arrive(&S.full_bar[g]);
+                }
+                ph ^= 1u << sub;
             }
+            r = rn;
+            have = have_next;
         }
-        if (d.tail_hi > d.tail_lo) {
-            const int64_t i = d.tail_lo + gt;
-            if (i < d.tail_hi) {
-                const int fs = __ldcs(frag_start + i), fe = __ldcs(frag_stop + i);
-                const int q = frag_mapq ? (int)__ldcs(frag_mapq + i) : 255;
-                wps_scatter(D, P, T, fs, fe, q);
-                if (FUSE) cov_visit(S.hist, ghist, C, T, fs, fe, q, cnt);
-            }
-        }
-        group_sync(g);                                   // scatter done; the staging buffer is free
-        if (gt == 0) mbar_arrive(&S.empty_bar[g]);
-        if (d.last) {
-            if (FUSE) {
-                const int c = __reduce_add_sync(0xffffffffu, cnt);
-                if ((gt & 31) == 0 && c) atomicAdd(&counts[d.ivl & 0x7fffffff], (unsigned long long)c);
-            }
-            wps_scan_store_group<ODD>(D, S.warp_tot[g], P, T, out + d.out_off, overflow, gt, g);
-        }
-        phase ^= 1u;
-    }
-    if (FUSE && C.n_bins > 0) {
-        // all consumer groups are done: flush the CTA's histogram (the producers have exited)
-        asm volatile("bar.sync %0, %1;" :: "n"(kHexGroups + 1), "n"(kHexConsumerThreads) : "memory");
-        const int nb = min(C.n_bins, kFuseBins);
-        for (int b = tid; b < nb; b += kHexConsumerThreads) {
-            const int v = S.hist[b];
-            if (v) atomicAdd(&ghist[b], (unsigned long long)v);
+#pragma unroll 1
+        for (int sub = 0; sub < 2; ++sub) {
+            const int g = 2 * p + sub;
+            mbar_wait(&S.empty_bar[g], ((ph >> sub) & 1u) ^ 1u);
+            S.desc[g].tile = -1;
+            mbar_arrive(&S.full_bar[g]);
         }
     }
 }
@@ -883,11 +615,6 @@ extern "C" int ftk_wps_tile_ranges(const int32_t *frag_start, int64_t n_frag,
                               wps_left_reach(window_size, max_len), scratch, static_cast<cudaStream_t>(stream_));
 }
 
-// plain WPS: 0 = dual (three CTAs per SM, two tiles in flight each; default: 0.350 ms at chr1 scale),
-// 1 = direct (one CTA per tile, 0.458 ms), 2 = hex without the fused pass (0.362 ms)
-static int g_wps_impl = 0;
-extern "C" void ftk_debug_set_wps_impl(int impl) { g_wps_impl = impl; }
-
 static int device_sm_count(int *sm) {
     static thread_local int sm_count[64] = {0};
     int dev = 0;
@@ -908,56 +635,33 @@ struct WpsLaunch {
     cudaStream_t stream;
 };
 
-template <bool ODD, typename OutT, bool FUSE>
-static int launch_hex(const WpsLaunch &a, OutT *out) {
+template <bool ODD, typename OutT, int GROUPS, bool FUSE>
+static int launch_stream(const WpsLaunch &a, OutT *out) {
     using namespace ftk;
+    using Smem = StreamSmem<GROUPS, FUSE>;
+    constexpr int ctas_per_sm = kStreamCtasPerSm<GROUPS>;
+    static_assert(sizeof(Smem) <= 227 * 1024, "a CTA may own at most 227 KB of shared memory on sm_100a");
+    static_assert(ctas_per_sm * (sizeof(Smem) + 1024) <= 228 * 1024,
+                  "the resident CTAs, with the 1 KB reserved for each, must fit the SM's 228 KB");
     int sm = 0;
     int rc = device_sm_count(&sm);
     if (rc != FTK_OK) return rc;
     static thread_local bool attr_set = false;
-    const int smem = (int)sizeof(HexSmem);
+    const int smem = (int)sizeof(Smem);
     if (!attr_set) {
-        FTK_CUDA_TRY(cudaFuncSetAttribute(wps_hex_kernel<ODD, OutT, FUSE>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+        FTK_CUDA_TRY(cudaFuncSetAttribute(wps_stream_kernel<ODD, OutT, GROUPS, FUSE>,
+                                          cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
         attr_set = true;
     }
-    int64_t grid = sm;                      // one persistent CTA per SM
-    if (grid > a.n_tiles) grid = a.n_tiles;
-    wps_hex_kernel<ODD, OutT, FUSE><<<(unsigned)grid, kHexThreads, smem, a.stream>>>(
+    // persistent CTAs; a plain-WPS CTA is launched only when there are two tiles for its two groups
+    int64_t grid = (int64_t)sm * ctas_per_sm;
+    const int64_t max_grid = GROUPS == kPlainGroups ? (a.n_tiles + 1) / 2 : a.n_tiles;
+    if (grid > max_grid) grid = max_grid;
+    wps_stream_kernel<ODD, OutT, GROUPS, FUSE><<<(unsigned)grid, kStreamThreads<GROUPS>, smem, a.stream>>>(
         a.frag_start, a.frag_stop, a.frag_mapq, a.n_frag, a.tile_p0, a.tile_len, a.tile_mid_lo, a.tile_mid_hi,
         a.tile_out_off, a.tile_ivl, a.ranges, (int)a.n_tiles, a.P, a.C, out, a.overflow, a.counts, a.hist);
-    FTK_CHECK_LAUNCH("wps_hex_kernel");
+    FTK_CHECK_LAUNCH("wps_stream_kernel");
     return FTK_OK;
-}
-
-template <bool ODD, typename OutT>
-static int launch_wps(const WpsLaunch &a, OutT *out) {
-    using namespace ftk;
-    if (g_wps_impl == 1) {
-        wps_tile_kernel<ODD, OutT><<<(unsigned)a.n_tiles, kWpsThreads, 0, a.stream>>>(
-            a.frag_start, a.frag_stop, a.frag_mapq, a.tile_p0, a.tile_len, a.tile_mid_lo, a.tile_mid_hi,
-            a.tile_out_off, a.ranges, a.P, out, a.overflow);
-        FTK_CHECK_LAUNCH("wps_tile_kernel");
-        return FTK_OK;
-    }
-    if (g_wps_impl != 2) {
-        int sm = 0;
-        int rc = device_sm_count(&sm);
-        if (rc != FTK_OK) return rc;
-        static thread_local bool dual_attr_set = false;
-        const int dsmem = (int)sizeof(DualSmem);
-        if (!dual_attr_set) {
-            FTK_CUDA_TRY(cudaFuncSetAttribute(wps_dual_kernel<ODD, OutT>, cudaFuncAttributeMaxDynamicSharedMemorySize, dsmem));
-            dual_attr_set = true;
-        }
-        int64_t dgrid = (int64_t)sm * kDualCtasPerSm;
-        if (dgrid > (a.n_tiles + 1) / 2) dgrid = (a.n_tiles + 1) / 2;
-        wps_dual_kernel<ODD, OutT><<<(unsigned)dgrid, kDualThreads, dsmem, a.stream>>>(
-            a.frag_start, a.frag_stop, a.frag_mapq, a.n_frag, a.tile_p0, a.tile_len, a.tile_mid_lo, a.tile_mid_hi,
-            a.tile_out_off, a.ranges, (int)a.n_tiles, a.P, out, a.overflow);
-        FTK_CHECK_LAUNCH("wps_dual_kernel");
-        return FTK_OK;
-    }
-    return launch_hex<ODD, OutT, false>(a, out);
 }
 
 static void wps_fill_params(ftk::WpsParams &P, int32_t window_size, int32_t min_len, int32_t max_len,
@@ -1003,7 +707,8 @@ static int wps_tiles_impl(const int32_t *frag_start, const int32_t *frag_stop,
     a.stream = static_cast<cudaStream_t>(stream_);
     wps_fill_params(a.P, window_size, min_len, max_len, min_mapq);
     a.C = CovParams{0, 0u, 0, 0};
-    return (window_size & 1) ? launch_wps<true, OutT>(a, out) : launch_wps<false, OutT>(a, out);
+    return (window_size & 1) ? launch_stream<true, OutT, kPlainGroups, false>(a, out)
+                             : launch_stream<false, OutT, kPlainGroups, false>(a, out);
 }
 
 extern "C" int ftk_wps_tiles_i32(const int32_t *frag_start, const int32_t *frag_stop,
@@ -1047,7 +752,7 @@ extern "C" int ftk_wps_tiles_i8(const int32_t *frag_start, const int32_t *frag_s
                                   ranges_ready, scratch, out, overflow_flag, stream_);
 }
 
-// ---- fused pass: WPS + per-interval coverage + pooled length histogram (wps_hex_kernel<.., FUSE>)
+// ---- fused pass: WPS + per-interval coverage + pooled length histogram (wps_stream_kernel<.., FUSE>)
 // a fragment whose midpoint fs + (L >> 1) is >= p0 starts at fs >= p0 - (Lmax >> 1)
 static int64_t fused_left_reach(int32_t window_size, int32_t max_len, int32_t cov_max_len, int32_t max_frag_len) {
     const int64_t cov_hi = (cov_max_len == FTK_NONE) ? INT32_MAX : cov_max_len;
@@ -1115,8 +820,9 @@ extern "C" int ftk_wps_cov_tiles(const int32_t *frag_start, const int32_t *frag_
     a.hist = reinterpret_cast<unsigned long long *>(hist);
     a.stream = stream;
     const bool odd = (window_size & 1) != 0;
-#define FTK_FUSED(T)                                                                        \
-    (odd ? launch_hex<true, T, true>(a, static_cast<T *>(out)) : launch_hex<false, T, true>(a, static_cast<T *>(out)))
+#define FTK_FUSED(T)                                                            \
+    (odd ? launch_stream<true, T, kFusedGroups, true>(a, static_cast<T *>(out)) \
+         : launch_stream<false, T, kFusedGroups, true>(a, static_cast<T *>(out)))
     if (out_kind == 0) return FTK_FUSED(int32_t);
     if (out_kind == 1) return FTK_FUSED(int16_t);
     return FTK_FUSED(int8_t);

@@ -237,9 +237,6 @@ class WpsPlan:
             "ftk_wps_tiles_i32")
         return out
 
-
-    _KIND = {"int32": 0, "int16": 1, "int8": 2}
-
     def ranges_fused(self, frags: ContigFragments, window_size=120, cov_max_length=None, zero_counts=None,
                      zero_hist=None):
         """Only the fragment-range prepass of ``run_fused`` (lets a caller time the main kernel alone).

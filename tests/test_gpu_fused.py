@@ -1,6 +1,6 @@
 """Fused pass (WPS + per-interval coverage + pooled length histogram in one sweep over the fragments,
-``ftk_wps_cov_tiles``) vs the CPU oracle and vs the three separate kernels; every WPS kernel variant
-(hex / dual / direct) must give identical scores."""
+``ftk_wps_cov_tiles``) vs the CPU oracle and vs the separate kernels; the fused (six-group) and the plain
+(two-group) shape of the WPS kernel must give identical scores."""
 import numpy as np
 import pytest
 
@@ -75,11 +75,10 @@ def test_fused_random_vs_oracle(seed, dev):
             assert np.array_equal(hist.cpu().numpy(), _oracle_hist(ofr, live, c_lo, c_hi, cq, n_bins)), (seed, n_bins)
 
 
-def test_fused_equals_separate_kernels_and_all_variants_agree(dev):
-    """3 M fragments: fused pass == WpsPlan.run + interval_hist(pooled='hist'); hex == dual == direct."""
+def test_fused_equals_plain_and_separate_kernels(dev):
+    """3 M fragments: fused pass (six groups) == WpsPlan.run (plain, two groups) + interval_hist(pooled='hist')."""
     import torch
     from finaletoolkit_b200 import device as D
-    from finaletoolkit_b200._lib import lib
     from finaletoolkit_b200.synth import synth_fragments
     clen, n = 10_000_000, 3_200_000
     st, sp, mq, sd = synth_fragments(clen, n, 7)
@@ -92,15 +91,9 @@ def test_fused_equals_separate_kernels_and_all_variants_agree(dev):
     c2 = torch.zeros(ivl.n, dtype=torch.int64, device=dev); h2 = torch.zeros((1, n_bins), dtype=torch.int64, device=dev)
     D.interval_hist(fr, intersect_policy="midpoint", quality_threshold=30, n_bins=n_bins, pooled="hist", ivl_set=ivl,
                     out=(c2, h2, None))
-    try:
-        outs = {}
-        for impl in (0, 2, 1):
-            lib().ftk_debug_set_wps_impl(impl)
-            outs[impl] = plan.run(fr, 120, 120, 180, 30).clone()
-    finally:
-        lib().ftk_debug_set_wps_impl(0)
+    plain = plan.run(fr, 120, 120, 180, 30)
     torch.cuda.synchronize()
-    assert torch.equal(outs[0], outs[2]) and torch.equal(outs[0], outs[1]) and torch.equal(wps, outs[0])
+    assert torch.equal(wps, plain)
     assert torch.equal(cnt, c2) and torch.equal(hist, h2[0])
     # odd window + int8 output through the fused entry
     flag = torch.zeros(1, dtype=torch.int32, device=dev)

@@ -222,6 +222,16 @@ def test_streamed_pipeline_matches_resident(dev):
     w8, c8, h8, t8 = pipe8.run()
     assert w8.dtype == torch.int8 and np.array_equal(w8.numpy()[: pipe8.n_positions].astype(np.int32), ref)
     assert np.array_equal(c8.numpy(), cov.cpu().numpy()) and pipe8.d2h_bytes < pipe.d2h_bytes
+    # WPS alone (no coverage, no histogram) runs the plain kernel with narrow outputs: even and odd window
+    ref121 = D.WpsPlan(edges[:-1], edges[1:], clen, 180, dev).run(fr, 121).cpu().numpy()
+    assert np.abs(ref121).max() <= 127
+    for W, exp in ((120, ref), (121, ref121)):
+        for dtype in ("int16", "int8"):
+            plain = StreamedContig(torch.from_numpy(st).pin_memory(), torch.from_numpy(sp).pin_memory(),
+                                   torch.from_numpy(mq).pin_memory(), edges[:-1], edges[1:], clen, window_size=W,
+                                   n_chunks=3, device=dev, coverage=False, length_hist=False, wps_dtype=dtype)
+            wp, _, _, _ = plain.run()
+            assert np.array_equal(wp.numpy()[: plain.n_positions].astype(np.int32), exp), (W, dtype)
     deep_s = np.sort(np.random.default_rng(2).integers(1000, 1400, 30_000)).astype(np.int32)
     deep = StreamedContig(torch.from_numpy(deep_s).pin_memory(), torch.from_numpy(deep_s + 150).pin_memory(),
                           torch.full((30_000,), 60, dtype=torch.uint8).pin_memory(), [0], [5000], 10_000, device=dev,

@@ -1,7 +1,7 @@
 """Profiling target (run under ncu on a GPU box): one fused WPS+coverage+histogram step and one fused
 adjust (rank median + Savitzky-Golay) call at chr1 scale.
     EXTRAS=1 ncu --set full --clock-control none --import-source on \
-        -k regex:"adjust_rank_kernel|wps_hex_kernel|end_motif_kernel|cleavage_tile_kernel|delfi_count_kernel" -c 5 \
+        -k regex:"adjust_rank_kernel|wps_stream_kernel|end_motif_kernel|cleavage_tile_kernel|delfi_count_kernel" -c 5 \
         -o gpurun_out/r2b_top python tools/prof_kernels.py
 """
 import os

@@ -3,8 +3,6 @@ import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import sys, time
 import numpy as np, torch, os, ctypes
-from finaletoolkit_b200._lib import lib
-lib().ftk_debug_set_wps_impl(int(os.environ.get('FTK_WPS_IMPL','0')))
 from finaletoolkit_b200.device import ContigFragments, WpsPlan
 from finaletoolkit_b200.synth import synth_fragments
 clen = 249_250_621; n = int(sys.argv[1]) if len(sys.argv) > 1 else 80_000_000

@@ -1,4 +1,4 @@
-"""A/B timings of the WPS kernel variants, the fused pass, the unpack kernel and the e2e pipelines
+"""Timings of the plain WPS kernel, the fused pass, the unpack kernel and the e2e pipelines
 at chr1 scale (CUDA events, min/mean of several launches).  Run on a GPU box:
     python tools/wps_variants.py [n_frag]
 """
@@ -12,7 +12,6 @@ import torch
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from finaletoolkit_b200 import device as D
-from finaletoolkit_b200._lib import lib
 from finaletoolkit_b200.packed import PackedFragments
 from finaletoolkit_b200.pipeline import StreamedContig
 from finaletoolkit_b200.synth import synth_fragments
@@ -43,10 +42,7 @@ def main():
     res = {"n_frag": N}
     plan.ranges(fr)
     res["ranges"] = timed(lambda: plan.ranges(fr))
-    for name, impl in (("hex", 2), ("dual", 0), ("direct", 1)):
-        lib().ftk_debug_set_wps_impl(impl)
-        res["wps_" + name] = timed(lambda: plan.run(fr, out=out, ranges_ready=True))
-    lib().ftk_debug_set_wps_impl(0)
+    res["wps"] = timed(lambda: plan.run(fr, out=out, ranges_ready=True))
     cnt = torch.zeros(plan.n_intervals, dtype=torch.int64, device=dev)
     hist = torch.zeros(601, dtype=torch.int64, device=dev)
     res["fused_wps_cov_hist(incl ranges)"] = timed(lambda: plan.run_fused(fr, n_bins=601, out=out, counts=cnt, hist=hist))
