@@ -5,7 +5,7 @@ Table-driven Click group.  For every in-scope subcommand the flag spellings, par
 (cli/commands/__init__.py:87-640); dispatch filters the parameters by the target's signature like
 cli/_dispatch.py:96-118 and expands ``--strand`` into both_strands / negative_strand
 (cli/_dispatch.py:25-36).  Out-of-scope subcommands (delfi, breakpoint motifs, filter-file, agg-bw,
-gap-bed) are not registered.
+gap-bed) are not registered.  ``EXTRA_COMMANDS`` holds the subcommands this package adds (coverage-profile).
 """
 from __future__ import annotations
 
@@ -157,6 +157,24 @@ COMMANDS = {
                       help="Apply the Miller-Madow bias correction.")]),
 }
 
+# subcommands with no reference counterpart, kept apart from the reference's command table
+EXTRA_COMMANDS = {
+    "coverage-profile": ("finaletoolkit_b200.frag", "multi_coverage_profile",
+                         "Per-base fragment depth (or fragment-midpoint count) over BED intervals.", [
+        _INPUT, _arg("interval_file", metavar="REGIONS"), _arg("chrom_sizes", metavar="CHROM_SIZES"), _REF,
+        _out("bigWig or gzipped bedGraph of per-base depth."), _minlen(None), _maxlen(None), _mapq(30),
+        _opt("--pad-left", "left", metavar="BP", default=0, show_default=True, type=int,
+             help="Base pairs to subtract from each start coordinate."),
+        _opt("--pad-right", "right", metavar="BP", default=0, show_default=True, type=int,
+             help="Base pairs to add to each stop coordinate."),
+        _opt("--midpoint", "midpoint", is_flag=True, help="Count fragment midpoints instead of spanned bases."),
+        _opt("--scale-factor", "scale_factor", metavar="X", default=1.0, show_default=True, type=float,
+             help="Scale factor for depth values."),
+        _opt("-n", "--normalize", "normalize", is_flag=True,
+             help="Divide the scale factor by the number of passing fragments in the file."),
+        _THREADS, _VERBOSE]),
+}
+
 
 def run(module: str, func: str, params: dict):
     """Import the target lazily, translate --strand, keep only the kwargs it accepts, call it."""
@@ -185,7 +203,7 @@ def main_cli():
     """finaletoolkit_b200: the B200-native hot path of FinaleToolkit."""
 
 
-for _name, (_module, _func, _help, _spec) in COMMANDS.items():
+for _name, (_module, _func, _help, _spec) in {**COMMANDS, **EXTRA_COMMANDS}.items():
     main_cli.add_command(_make(_name, _module, _func, _help, _spec))
 
 

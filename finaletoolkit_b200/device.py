@@ -818,3 +818,24 @@ def cleavage_intervals(frags: ContigFragments, ivl_start, ivl_stop, chrom_size, 
             none_to_ftk(min_length), none_to_ftk(max_length), int(quality_threshold),
             plan.scratch.data_ptr(), out.data_ptr(), _stream_ptr(frags.device)), "ftk_cleavage_tiles_f64")
     return out[: plan.n_positions], plan.offsets
+
+
+def depth_intervals(frags: ContigFragments, ivl_start, ivl_stop, chrom_size, min_length=None, max_length=None,
+                    quality_threshold=30, midpoint=False):
+    """Per-base fragment depth (int32) of every interval back to back + host offsets.
+
+    Span depth (the coverage of _coverage_and_ends, frag/_cleavage_profile.py:33-90) counts the passing
+    fragments with start <= p < stop; ``midpoint=True`` counts those with (start + stop) // 2 == p.
+    ``ivl_start/ivl_stop`` are already padded/clamped bounds; one launch for all of them.
+    """
+    t = torch()
+    plan = WpsPlan(ivl_start, ivl_stop, int(chrom_size), 0, frags.device)   # the tile table of cleavage_intervals
+    out = t.empty(max(plan.n_positions, 1), dtype=t.int32, device=frags.device)
+    if plan.n_tiles:
+        fs, fe, mq = frags.ptrs()
+        check(lib().ftk_depth_tiles_i32(
+            fs, fe, mq, frags.n, frags.max_len, plan.tile_p0.data_ptr(), plan.tile_len.data_ptr(),
+            plan.tile_mid_lo.data_ptr(), plan.tile_mid_hi.data_ptr(), plan.tile_out_off.data_ptr(), plan.n_tiles,
+            none_to_ftk(min_length), none_to_ftk(max_length), int(quality_threshold), int(bool(midpoint)),
+            plan.scratch.data_ptr(), out.data_ptr(), _stream_ptr(frags.device)), "ftk_depth_tiles_i32")
+    return out[: plan.n_positions], plan.offsets

@@ -81,21 +81,8 @@ def _read_intervals(interval_file, left, right, chrom_dict):
     return contigs[1:], starts[1:], stops[1:]
 
 
-def multi_cleavage_profile(input_file, interval_file, chrom_sizes, left=0, right=0, min_length=None,
-                           max_length=None, quality_threshold=30, output_file="-", workers=1, verbose=0,
-                           fraction_low=None, fraction_high=None, reference_file=None) -> str:
-    """Cleavage profiles over the intervals of a (sorted) BED; ``.bw`` / ``.bed.gz`` / ``bedgraph.gz``."""
-    from ..device import cleavage_intervals
-    if verbose:
-        start_time = time.time()
-    min_length, max_length = resolve_length_aliases(min_length, max_length, fraction_low, fraction_high)
-    if input_file == "-" and interval_file == "-":
-        raise ValueError("input_file and site_bed cannot both read from stdin")
-    if chrom_sizes is None:
-        raise ValueError("chrom_sizes must be specified.")
-    header = chrom_sizes_to_list(chrom_sizes)
-    chrom_dict = chrom_sizes_to_dict(chrom_sizes)
-    contigs, starts, stops = _read_intervals(interval_file, left, right, chrom_dict)
+def _check_output_file(output_file, input_file):
+    """``output_file`` must be None or a ``.bw`` / ``.bed.gz`` / ``bedgraph.gz`` path or '-'."""
     if isinstance(output_file, str):
         if not (output_file.endswith(".bw") or output_file.endswith(".bed.gz") or output_file.endswith("bedgraph.gz")
                 or output_file == "-"):
@@ -103,24 +90,10 @@ def multi_cleavage_profile(input_file, interval_file, chrom_sizes, left=0, right
     elif output_file is not None:
         raise TypeError(f'output_file is unsupported type "{type(input_file)}". output_file should be a string '
                         "specifying the path of the file to output scores to.")
-    table = as_table(input_file, reference_file)
-    size_dict = dict(header)
-    results: list = [None] * len(contigs)
-    for contig, idx in group_by_contig(contigs).items():
-        # cleavage_profile() re-clamps each interval (left = right = 0 here, frag/_cleavage_profile.py:352-353)
-        s = [max(starts[i], 0) for i in idx]
-        e = [min(stops[i], size_dict[contig]) for i in idx]
 
-        def run(tab, sel, contig=contig, s=s, e=e):
-            if tab.n_fragments(contig) == 0:
-                return [np.zeros(max(e[k] - s[k], 0)) for k in sel]
-            out, off = cleavage_intervals(tab.device(contig), [s[k] for k in sel], [e[k] for k in sel],
-                                          size_dict[contig], min_length, max_length, quality_threshold)
-            host = out.cpu().numpy()
-            return [host[off[j]: off[j + 1]] for j in range(len(sel))]
 
-        for i, scores in zip(idx, per_fetch(table, contig, s, e, run)):
-            results[i] = scores
+def _write_tracks(output_file, header, contigs, starts, results):
+    """Per-base values of every interval (float64 arrays) as bigWig entries (``.bw``) or gzipped bedGraph lines."""
     if isinstance(output_file, str):
         if output_file.endswith(".bw"):
             with pbw.open(output_file, "w") as bigwig:
@@ -141,6 +114,43 @@ def multi_cleavage_profile(input_file, interval_file, chrom_sizes, left=0, right
                     pos = max(start, 0)
                     bedgraph.write("".join(f"{contig}\t{p}\t{p + 1}\t{v}\n"
                                            for p, v in zip(range(pos, pos + len(scores)), scores.tolist())))
+
+
+def multi_cleavage_profile(input_file, interval_file, chrom_sizes, left=0, right=0, min_length=None,
+                           max_length=None, quality_threshold=30, output_file="-", workers=1, verbose=0,
+                           fraction_low=None, fraction_high=None, reference_file=None) -> str:
+    """Cleavage profiles over the intervals of a (sorted) BED; ``.bw`` / ``.bed.gz`` / ``bedgraph.gz``."""
+    from ..device import cleavage_intervals
+    if verbose:
+        start_time = time.time()
+    min_length, max_length = resolve_length_aliases(min_length, max_length, fraction_low, fraction_high)
+    if input_file == "-" and interval_file == "-":
+        raise ValueError("input_file and site_bed cannot both read from stdin")
+    if chrom_sizes is None:
+        raise ValueError("chrom_sizes must be specified.")
+    header = chrom_sizes_to_list(chrom_sizes)
+    chrom_dict = chrom_sizes_to_dict(chrom_sizes)
+    contigs, starts, stops = _read_intervals(interval_file, left, right, chrom_dict)
+    _check_output_file(output_file, input_file)
+    table = as_table(input_file, reference_file)
+    size_dict = dict(header)
+    results: list = [None] * len(contigs)
+    for contig, idx in group_by_contig(contigs).items():
+        # cleavage_profile() re-clamps each interval (left = right = 0 here, frag/_cleavage_profile.py:352-353)
+        s = [max(starts[i], 0) for i in idx]
+        e = [min(stops[i], size_dict[contig]) for i in idx]
+
+        def run(tab, sel, contig=contig, s=s, e=e):
+            if tab.n_fragments(contig) == 0:
+                return [np.zeros(max(e[k] - s[k], 0)) for k in sel]
+            out, off = cleavage_intervals(tab.device(contig), [s[k] for k in sel], [e[k] for k in sel],
+                                          size_dict[contig], min_length, max_length, quality_threshold)
+            host = out.cpu().numpy()
+            return [host[off[j]: off[j + 1]] for j in range(len(sel))]
+
+        for i, scores in zip(idx, per_fetch(table, contig, s, e, run)):
+            results[i] = scores
+    _write_tracks(output_file, header, contigs, starts, results)
     if verbose:
         stderr.write(f"cleavage profile took {time.time() - start_time} s to complete\n")
     return output_file

@@ -389,6 +389,27 @@ int ftk_cleavage_tiles_f64(const int32_t *frag_start_dev, const int32_t *frag_st
                            int32_t min_len, int32_t max_len, int32_t min_mapq,
                            int64_t *scratch_dev, double *out_dev, ftk_stream_t stream);
 
+/* ------------------------------------------------------ per-base fragment depth
+ * The depth track of coverage_profile: the coverage array of _coverage_and_ends
+ * (frag/_cleavage_profile.py:33-90) as its own output, or the fragment-midpoint count.  Same tile
+ * table and fragment filter as ftk_cleavage_tiles_f64 (mapq >= min_mapq, min_len <= L <= max_len,
+ * FTK_NONE = unbounded); no strand column is read.
+ * midpoint == 0: out[tile_out_off + (p - p0)] = #{passing fragments with start <= p < stop}
+ * midpoint != 0: out[tile_out_off + (p - p0)] = #{passing fragments with (start + stop) / 2 == p}
+ * (int32).  A fragment of length >= 1 that covers, or is centred on, a position overlaps that
+ * position's interval, so tile_ivl_lo/hi are validated but never read.  The one exception is a
+ * zero-length fragment (start == stop, passing only with min_len <= 0): midpoint mode counts it at
+ * start by the definition above, also at an interval's first position, where the "any" overlap
+ * test (stop > ivl_lo) of ftk_cleavage_tiles_f64 would drop it.  Span mode never counts it.
+ * scratch_dev: int64[2 * n_tiles]. */
+int ftk_depth_tiles_i32(const int32_t *frag_start_dev, const int32_t *frag_stop_dev,
+                        const uint8_t *frag_mapq_dev, int64_t n_frag, int32_t max_frag_len,
+                        const int32_t *tile_p0_dev, const int32_t *tile_len_dev,
+                        const int32_t *tile_ivl_lo_dev, const int32_t *tile_ivl_hi_dev,
+                        const int64_t *tile_out_off_dev, int64_t n_tiles,
+                        int32_t min_len, int32_t max_len, int32_t min_mapq, int32_t midpoint,
+                        int64_t *scratch_dev, int32_t *out_dev, ftk_stream_t stream);
+
 /* ------------------------------------------------- fragment file decode (host)
  * Multi-threaded decode of a BGZF / gzip fragment file into per-contig columns; replaces the
  * per-interval pysam.TabixFile.fetch text stream of io/alignment.py:270-302 (5-column FinaleDB

@@ -1,5 +1,6 @@
-"""Kernel timing helper (python tools/quick_kernels.py [motif] [bp] [adjust] [delfi] [cleavage]): CUDA-event time of
-the secondary kernels at chr1 scale (80 M fragments drawn on the GPU), median of 7 calls after 3 warm-ups."""
+"""Kernel timing helper (python tools/quick_kernels.py [motif] [bp] [adjust] [delfi] [cleavage] [depth] [depth-mid]): CUDA-event time of
+the secondary kernels at chr1 scale (80 M fragments drawn on the GPU), median of 7 calls after 3 warm-ups (the call:
+planning and uploads included); cleavage / depth also print each kernel's own device time (torch.profiler)."""
 import os
 import sys
 
@@ -33,6 +34,18 @@ def timed(name, fn, nbytes):
     return out
 
 
+def kernels(fn, reps=5):
+    """Device time per call of each ftk:: kernel fn launches (CUPTI through torch.profiler, a separate run)."""
+    from torch.profiler import ProfilerActivity, profile
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        for _ in range(reps):
+            fn()
+        torch.cuda.synchronize()
+    for ev in prof.key_averages():
+        if "ftk::" in ev.key:
+            print(f"  kernel {ev.key.split('(')[0]}: {ev.device_time_total / reps / 1e3:.3f} ms", flush=True)
+
+
 if what & {"motif", "bp", "delfi"}:
     codes, nm = synth_twobit(CLEN, 0)
     ref = D.PackedContig.from_codes(codes, nm, device=dev)
@@ -49,7 +62,17 @@ if "delfi" in what:
     timed("delfi 100-kb bins", lambda: D.delfi_windows(fr, ref, bs, be, quality_threshold=30), 9 * N + CLEN * 3 // 8)
 if "cleavage" in what:
     edges = np.arange(0, CLEN + 5000, 5000, dtype=np.int64).clip(max=CLEN)
-    timed("cleavage", lambda: D.cleavage_intervals(fr, edges[:-1], edges[1:], CLEN, None, None, 30), 10 * N + 8 * CLEN)
+    run = lambda: D.cleavage_intervals(fr, edges[:-1], edges[1:], CLEN, None, None, 30)   # noqa: E731
+    timed("cleavage", run, 10 * N + 8 * CLEN)
+    kernels(run)
+if what & {"depth", "depth-mid"}:
+    edges = np.arange(0, CLEN + 5000, 5000, dtype=np.int64).clip(max=CLEN)
+    for name in ("depth", "depth-mid"):
+        if name in what:
+            run = lambda: D.depth_intervals(fr, edges[:-1], edges[1:], CLEN, None, None, 30, name == "depth-mid")  # noqa: E731
+            o = timed(name, run, 9 * N + 4 * CLEN)
+            print("  checksum", int(o[0].sum(dtype=torch.int64)))
+            kernels(run)
 if "hist" in what:
     edges = np.arange(0, CLEN + 5000, 5000, dtype=np.int64).clip(max=CLEN)
     timed("coverage counts (5-kb intervals)", lambda: D.interval_hist(fr, edges[:-1], edges[1:], "midpoint", None, None, 30), 9 * N)
