@@ -31,19 +31,6 @@ constexpr int kClvThreads = 256;
 constexpr int kClvCap = 5120;
 constexpr int kClvPer = kClvCap / kClvThreads;   // 20 contiguous positions per thread
 
-__global__ void clv_tile_ranges_kernel(const int32_t *__restrict__ frag_start, int64_t n_frag,
-                                       const int32_t *__restrict__ tile_p0, const int32_t *__restrict__ tile_len,
-                                       int64_t n_tiles, int halo, int64_t *__restrict__ ranges) {
-    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= 2 * n_tiles) return;
-    const int64_t tile = t >> 1;
-    const int64_t p0 = tile_p0[tile];
-    // a covering fragment has stop > p0 (=> start > p0 - max_frag_len) and start < p0 + len; so has a
-    // fragment whose midpoint lies in the tile (start <= midpoint < stop)
-    const int64_t key = (t & 1) ? p0 + tile_len[tile] : p0 - halo;
-    ranges[t] = lower_bound(frag_start, n_frag, key);
-}
-
 enum class ClvMode { kCleavage, kDepthSpan, kDepthMid };
 
 // Store len int32 positions of the shared tile to dst (4-byte aligned) with coalesced 16-byte streaming stores:
@@ -94,7 +81,7 @@ __device__ __forceinline__ void clv_tile_body(
     }
     __syncthreads();
     const uint32_t d_addr = smem_addr_once(D), e_addr = kEnds ? smem_addr_once(E) : 0u;
-    auto visit = [&](int fs, int fe, int q, int sd) {
+    auto visit = [&](int fs, int fe, int q, int sd, int) {
         const int L = fe - fs;
         if constexpr (kEnds) {
             // frag_array(..., "any") of the INTERVAL: tabix overlap + mapq + inclusive length window
@@ -115,46 +102,7 @@ __device__ __forceinline__ void clv_tile_body(
             if (end_idx >= 0 && end_idx < len) red_shared_inc(e_addr + 4u * (unsigned)end_idx);
         }
     };
-    // the candidate slice is widened to a 16-byte boundary on the left (extra fragments are harmless:
-    // the range is only a superset) so every lane streams 4 fragments per 128-bit load
-    constexpr int kU = 2;   // independent vector loads in flight per thread (8 fragments)
-    const int64_t lo_al = lo & ~(int64_t)3;
-    const int cnt = (hi > lo_al) ? (int)(hi - lo_al) : 0;
-    const int nvec = cnt >> 2;
-    const int4 *__restrict__ vs = reinterpret_cast<const int4 *>(frag_start + lo_al);
-    const int4 *__restrict__ ve = reinterpret_cast<const int4 *>(frag_stop + lo_al);
-    const uchar4 *__restrict__ vq = reinterpret_cast<const uchar4 *>(frag_mapq ? frag_mapq + lo_al : nullptr);
-    const uchar4 *__restrict__ vd = reinterpret_cast<const uchar4 *>(frag_strand ? frag_strand + lo_al : nullptr);
-    for (int v0 = tid; v0 < nvec; v0 += kU * kClvThreads) {
-        int4 s4[kU], e4[kU];
-        uchar4 q4[kU], d4[kU];
-#pragma unroll
-        for (int u = 0; u < kU; ++u) {
-            const int v = v0 + u * kClvThreads;
-            if (v < nvec) {
-                s4[u] = __ldcs(vs + v); e4[u] = __ldcs(ve + v);
-                q4[u] = vq ? __ldcs(vq + v) : make_uchar4(255, 255, 255, 255);
-                d4[u] = vd ? __ldcs(vd + v) : make_uchar4(1, 1, 1, 1);
-            } else {
-                s4[u] = make_int4(0, 0, 0, 0); e4[u] = make_int4(-1, -1, -1, -1);   // L < 0: skipped
-                q4[u] = make_uchar4(0, 0, 0, 0); d4[u] = make_uchar4(1, 1, 1, 1);
-            }
-        }
-#pragma unroll
-        for (int u = 0; u < kU; ++u) {
-            visit(s4[u].x, e4[u].x, q4[u].x, d4[u].x);
-            visit(s4[u].y, e4[u].y, q4[u].y, d4[u].y);
-            visit(s4[u].z, e4[u].z, q4[u].z, d4[u].z);
-            visit(s4[u].w, e4[u].w, q4[u].w, d4[u].w);
-        }
-    }
-    {   // tail: at most 3 fragments
-        const int i = nvec * 4 + tid;
-        if (i < cnt)
-            visit(__ldcs(frag_start + lo_al + i), __ldcs(frag_stop + lo_al + i),
-                  frag_mapq ? (int)__ldcs(frag_mapq + lo_al + i) : 255,
-                  frag_strand ? (int)__ldcs(frag_strand + lo_al + i) : 1);
-    }
+    stream_fragments<kClvThreads, 2>(FragCols{frag_start, frag_stop, frag_mapq, frag_strand}, lo, hi, tid, visit);
     __syncthreads();
     if constexpr (MODE == ClvMode::kDepthMid) {
         clv_store_i32(D, out + tile_out_off[tile], len, tid);
@@ -247,6 +195,21 @@ depth_tile_kernel(const int32_t *__restrict__ frag_start, const int32_t *__restr
 
 using namespace ftk;
 
+// Argument checks of the cleavage and depth entry points, then the tile-range prepass: a fragment covering a tile
+// position has stop > p0 (=> start > p0 - max_frag_len) and start < p0 + len; so has a fragment whose midpoint
+// lies in the tile.
+static int clv_tile_ranges(const int32_t *frag_start, const int32_t *frag_stop, int64_t n_frag, int32_t max_frag_len,
+                           const int32_t *tile_p0, const int32_t *tile_len, const int32_t *tile_ivl_lo,
+                           const int32_t *tile_ivl_hi, const int64_t *tile_out_off, int64_t n_tiles,
+                           int64_t *scratch, const void *out, cudaStream_t stream) {
+    if (n_frag < 0 || n_tiles < 0) return FTK_E_INVALID;
+    if (!tile_p0 || !tile_len || !tile_ivl_lo || !tile_ivl_hi || !tile_out_off || !scratch || !out) return FTK_E_INVALID;
+    if (n_frag > 0 && (!frag_start || !frag_stop)) return FTK_E_INVALID;
+    if (n_tiles > INT32_MAX / 2) return FTK_E_RANGE;
+    return launch_candidate_ranges(frag_start, n_frag, tile_p0, tile_len, true, n_tiles, max_frag_len < 0 ? 0 : max_frag_len,
+                                   0, scratch, stream);
+}
+
 extern "C" int ftk_cleavage_tiles_f64(const int32_t *frag_start, const int32_t *frag_stop,
                                       const uint8_t *frag_mapq, const uint8_t *frag_strand,
                                       int64_t n_frag, int32_t max_frag_len,
@@ -256,15 +219,10 @@ extern "C" int ftk_cleavage_tiles_f64(const int32_t *frag_start, const int32_t *
                                       int32_t min_len, int32_t max_len, int32_t min_mapq,
                                       int64_t *scratch, double *out, ftk_stream_t stream_) {
     if (n_tiles == 0) return FTK_OK;
-    if (n_frag < 0 || n_tiles < 0) return FTK_E_INVALID;
-    if (!tile_p0 || !tile_len || !tile_ivl_lo || !tile_ivl_hi || !tile_out_off || !scratch || !out) return FTK_E_INVALID;
-    if (n_frag > 0 && (!frag_start || !frag_stop)) return FTK_E_INVALID;
-    if (n_tiles > INT32_MAX / 2) return FTK_E_RANGE;
     cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-    const int64_t n = 2 * n_tiles;
-    clv_tile_ranges_kernel<<<(unsigned)((n + 127) / 128), 128, 0, stream>>>(
-        frag_start, n_frag, tile_p0, tile_len, n_tiles, max_frag_len < 0 ? 0 : max_frag_len, scratch);
-    FTK_CHECK_LAUNCH("clv_tile_ranges_kernel");
+    const int rc = clv_tile_ranges(frag_start, frag_stop, n_frag, max_frag_len, tile_p0, tile_len, tile_ivl_lo,
+                                   tile_ivl_hi, tile_out_off, n_tiles, scratch, out, stream);
+    if (rc != FTK_OK) return rc;
     cleavage_tile_kernel<<<(unsigned)n_tiles, kClvThreads, 0, stream>>>(
         frag_start, frag_stop, frag_mapq, frag_strand, tile_p0, tile_len, tile_ivl_lo, tile_ivl_hi, tile_out_off,
         scratch, min_len, max_len, min_mapq, out);
@@ -280,15 +238,10 @@ extern "C" int ftk_depth_tiles_i32(const int32_t *frag_start, const int32_t *fra
                                    int32_t min_len, int32_t max_len, int32_t min_mapq, int32_t midpoint,
                                    int64_t *scratch, int32_t *out, ftk_stream_t stream_) {
     if (n_tiles == 0) return FTK_OK;
-    if (n_frag < 0 || n_tiles < 0) return FTK_E_INVALID;
-    if (!tile_p0 || !tile_len || !tile_ivl_lo || !tile_ivl_hi || !tile_out_off || !scratch || !out) return FTK_E_INVALID;
-    if (n_frag > 0 && (!frag_start || !frag_stop)) return FTK_E_INVALID;
-    if (n_tiles > INT32_MAX / 2) return FTK_E_RANGE;
     cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-    const int64_t n = 2 * n_tiles;
-    clv_tile_ranges_kernel<<<(unsigned)((n + 127) / 128), 128, 0, stream>>>(
-        frag_start, n_frag, tile_p0, tile_len, n_tiles, max_frag_len < 0 ? 0 : max_frag_len, scratch);
-    FTK_CHECK_LAUNCH("clv_tile_ranges_kernel");
+    const int rc = clv_tile_ranges(frag_start, frag_stop, n_frag, max_frag_len, tile_p0, tile_len, tile_ivl_lo,
+                                   tile_ivl_hi, tile_out_off, n_tiles, scratch, out, stream);
+    if (rc != FTK_OK) return rc;
     if (midpoint)
         depth_tile_kernel<true><<<(unsigned)n_tiles, kClvThreads, 0, stream>>>(
             frag_start, frag_stop, frag_mapq, tile_p0, tile_len, tile_out_off, scratch, min_len, max_len, min_mapq, out);

@@ -20,17 +20,6 @@ namespace ftk {
 
 constexpr int kDelfiThreads = 256;
 
-__global__ void delfi_ranges_kernel(const int32_t *__restrict__ frag_start, int64_t n_frag,
-                                    const int32_t *__restrict__ win_start,
-                                    const int32_t *__restrict__ win_stop, int64_t n_win,
-                                    int halo, int64_t *__restrict__ ranges) {
-    int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= 2 * n_win) return;
-    const int64_t k = t >> 1;
-    const int64_t key = (t & 1) ? (int64_t)win_stop[k] : (int64_t)win_start[k] - halo;
-    ranges[t] = lower_bound(frag_start, n_frag, key);
-}
-
 struct DelfiGaps { int use, c0, c1, has_telo, t0_max, t1_min; };
 
 __global__ void __launch_bounds__(kDelfiThreads)
@@ -46,18 +35,15 @@ delfi_count_kernel(const int32_t *__restrict__ frag_start, const int32_t *__rest
     const int split = blockIdx.x % splits;
     const int S = win_start[win], E = win_stop[win];
     const int b_lo = bl_off ? bl_off[win] : 0, b_hi = bl_off ? bl_off[win + 1] : 0;
-    const int64_t lo_all = ranges[2 * win], hi_all = ranges[2 * win + 1];
-    int64_t chunk = (hi_all - lo_all + splits - 1) / splits;
-    chunk = (chunk + 3) & ~(int64_t)3;
-    const int64_t lo = lo_all + (int64_t)split * chunk;
-    const int64_t hi = min(hi_all, lo + chunk);
+    int64_t lo, hi;
+    slice_of(ranges, win, split, splits, lo, hi);
 
     int n_short = 0, n_long = 0;
     // One fragment, branch-free: every test of frag/_delfi.py:437-470 is a predicate (the tabix overlap
     // `stop > S and start < E` is implied by 100 <= length and the midpoint lying in [S, E)).  Only the
     // blacklist walk (a bin's own CSR list, nearly always empty) branches.
     const unsigned span = E > S ? (unsigned)(E - S) : 0u;
-    auto visit = [&](int fs, int fe, int q) {
+    auto visit = [&](int fs, int fe, int q, int, int) {
         const int len = fe - fs;
         const int mid = (int)(((int64_t)fs + fe) >> 1);   // floor, like Python's //
         bool pass = (q >= min_mapq) & ((unsigned)(len - 100) <= 120u) & ((unsigned)(mid - S) < span);
@@ -76,50 +62,7 @@ delfi_count_kernel(const int32_t *__restrict__ frag_start, const int32_t *__rest
         n_long += pass & is_long;
         n_short += pass & !is_long;
     };
-    // 128-bit streaming loads, two vectors (eight fragments) in flight per thread; the slice is widened
-    // to a 16-byte boundary on the left, the fragments before `lo` get mapq -1 (never counted)
-    const int64_t lo_al = lo & ~(int64_t)3;
-    const int skip = (int)(lo - lo_al);
-    const int cnt = (hi > lo) ? (int)(hi - lo_al) : 0;
-    const int nvec = cnt >> 2;
-    const int4 *__restrict__ vs = reinterpret_cast<const int4 *>(frag_start + lo_al);
-    const int4 *__restrict__ ve = reinterpret_cast<const int4 *>(frag_stop + lo_al);
-    const uchar4 *__restrict__ vq = reinterpret_cast<const uchar4 *>(frag_mapq ? frag_mapq + lo_al : nullptr);
-    constexpr int kU = 2;
-    for (int v0 = tid; v0 < nvec; v0 += kU * kDelfiThreads) {
-        int4 s4[kU], e4[kU];
-        int q0[kU], q1[kU], q2[kU], q3[kU];
-#pragma unroll
-        for (int u = 0; u < kU; ++u) {
-            const int v = v0 + u * kDelfiThreads;
-            if (v < nvec) {
-                s4[u] = __ldcs(vs + v); e4[u] = __ldcs(ve + v);
-                const uchar4 q = vq ? __ldcs(vq + v) : make_uchar4(255, 255, 255, 255);
-                q0[u] = q.x; q1[u] = q.y; q2[u] = q.z; q3[u] = q.w;
-            } else {
-                s4[u] = make_int4(0, 0, 0, 0); e4[u] = make_int4(0, 0, 0, 0);
-                q0[u] = q1[u] = q2[u] = q3[u] = -1;
-            }
-        }
-        if (v0 == 0 && skip) {       // thread 0, first vector only
-            q0[0] = -1;
-            if (skip > 1) q1[0] = -1;
-            if (skip > 2) q2[0] = -1;
-        }
-#pragma unroll
-        for (int u = 0; u < kU; ++u) {
-            visit(s4[u].x, e4[u].x, q0[u]);
-            visit(s4[u].y, e4[u].y, q1[u]);
-            visit(s4[u].z, e4[u].z, q2[u]);
-            visit(s4[u].w, e4[u].w, q3[u]);
-        }
-    }
-    {   // tail: at most 3 fragments
-        const int i = nvec * 4 + tid;
-        if (i < cnt && i >= skip)
-            visit(__ldcs(frag_start + lo_al + i), __ldcs(frag_stop + lo_al + i),
-                  frag_mapq ? (int)__ldcs(frag_mapq + lo_al + i) : 255);
-    }
+    stream_fragments<kDelfiThreads, 2>(FragCols{frag_start, frag_stop, frag_mapq, nullptr}, lo, hi, tid, visit);
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) {
         n_short += __shfl_down_sync(0xffffffffu, n_short, o);
@@ -204,14 +147,10 @@ extern "C" int ftk_delfi_windows_u64(const int32_t *frag_start, const int32_t *f
     if (gaps5) {   // host array: centromere start, stop, n_telomeres, max telomere start, min telomere stop
         g.use = 1; g.c0 = gaps5[0]; g.c1 = gaps5[1]; g.has_telo = gaps5[2] > 0; g.t0_max = gaps5[3]; g.t1_min = gaps5[4];
     }
-    {
-        const int64_t n = 2 * n_win;
-        delfi_ranges_kernel<<<(unsigned)((n + 127) / 128), 128, 0, stream>>>(
-            frag_start, n_frag, win_start, win_stop, n_win, max_frag_len < 0 ? 0 : max_frag_len, scratch);
-        FTK_CHECK_LAUNCH("delfi_ranges_kernel");
-    }
+    const int rc = launch_candidate_ranges(frag_start, n_frag, win_start, win_stop, false, n_win,
+                                           max_frag_len < 0 ? 0 : max_frag_len, 0, scratch, stream);
+    if (rc != FTK_OK) return rc;
     auto *c = reinterpret_cast<unsigned long long *>(counts);
-    if (min_mapq < 0) min_mapq = 0;      // mapq is a uint8 column; the kernel masks rows with mapq -1
     delfi_count_kernel<<<(unsigned)(n_win * splits), kDelfiThreads, 0, stream>>>(
         frag_start, frag_stop, frag_mapq, win_start, win_stop, scratch, bl_off, bl_start, bl_stop, g,
         min_mapq, splits, c);

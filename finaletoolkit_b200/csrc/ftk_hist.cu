@@ -59,23 +59,6 @@ __device__ __forceinline__ bool frag_in_stream(int fs, int fe, int q, int S, int
     return Stream(S, E, p)(fs, fe, q);
 }
 
-// Candidate index range of each interval: a superset of its stream.
-__global__ void interval_ranges_kernel(const int32_t *__restrict__ frag_start, int64_t n_frag,
-                                       const int32_t *__restrict__ ivl_start,
-                                       const int32_t *__restrict__ ivl_stop, int64_t n_ivl,
-                                       int halo, int64_t *__restrict__ ranges) {
-    int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= 2 * n_ivl) return;
-    const int64_t k = t >> 1;
-    if ((t & 1) == 0) {
-        const int S = ivl_start[k];
-        ranges[t] = (S == FTK_NONE) ? 0 : lower_bound(frag_start, n_frag, (int64_t)S - halo);
-    } else {
-        const int E = ivl_stop[k];
-        ranges[t] = (E == FTK_NONE) ? n_frag : lower_bound(frag_start, n_frag, (int64_t)E);
-    }
-}
-
 template <bool HIST>
 __global__ void __launch_bounds__(kHistThreads)
 interval_hist_kernel(const int32_t *__restrict__ frag_start, const int32_t *__restrict__ frag_stop,
@@ -93,12 +76,8 @@ interval_hist_kernel(const int32_t *__restrict__ frag_start, const int32_t *__re
     const int split = blockIdx.x % splits;
     const int64_t row = pooled ? 0 : ivl;
     const int S = ivl_start[ivl], E = ivl_stop[ivl];
-    const int64_t lo_all = ranges[2 * ivl], hi_all = ranges[2 * ivl + 1];
-    // contiguous slice of the candidate range for this split (multiple of 4 fragments)
-    int64_t chunk = (hi_all - lo_all + splits - 1) / splits;
-    chunk = (chunk + 3) & ~(int64_t)3;
-    const int64_t lo = lo_all + (int64_t)split * chunk;
-    const int64_t hi = min(hi_all, lo + chunk);
+    int64_t lo, hi;
+    slice_of(ranges, ivl, split, splits, lo, hi);
     const bool want_first = HIST && (first_seen != nullptr);
 
     if (HIST) {
@@ -109,7 +88,7 @@ interval_hist_kernel(const int32_t *__restrict__ frag_start, const int32_t *__re
     const Stream in_stream(S, E, pred);
     unsigned my_count32 = 0;  // a CTA slice never holds 2^32 fragments (n_frag <= INT32_MAX)
     const uint32_t cnt_addr = HIST ? smem_addr_once(s_cnt) : 0u, first_addr = HIST ? smem_addr_once(s_first) : 0u;
-    auto visit = [&](int fs, int fe, int q, int idx) {
+    auto visit = [&](int fs, int fe, int q, int, int idx) {
         if (!in_stream(fs, fe, q)) return;
         ++my_count32;
         if (HIST) {
@@ -123,55 +102,7 @@ interval_hist_kernel(const int32_t *__restrict__ frag_start, const int32_t *__re
             }
         }
     };
-    // 128-bit streaming loads: the slice is widened to 16-byte boundaries on the left (fragments
-    // outside [lo, hi) are masked by index), 4 fragments per lane per load, kHistUnroll loads in flight.
-    const int64_t lo_al = lo & ~(int64_t)3;
-    const int skip = (int)(lo - lo_al);
-    const int cnt = (hi > lo) ? (int)(hi - lo_al) : 0;
-    const int nvec = cnt >> 2;
-    const int4 *__restrict__ vs = reinterpret_cast<const int4 *>(frag_start + lo_al);
-    const int4 *__restrict__ ve = reinterpret_cast<const int4 *>(frag_stop + lo_al);
-    const uchar4 *__restrict__ vq = reinterpret_cast<const uchar4 *>(frag_mapq ? frag_mapq + lo_al : nullptr);
-    const int base_idx = (int)lo_al;
-    for (int v0 = tid; v0 < nvec; v0 += kHistUnroll * kHistThreads) {
-        int4 s4[kHistUnroll], e4[kHistUnroll];
-        uchar4 q4[kHistUnroll];
-#pragma unroll
-        for (int u = 0; u < kHistUnroll; ++u) {
-            const int v = v0 + u * kHistThreads;
-            if (v < nvec) {
-                s4[u] = __ldcs(vs + v);
-                e4[u] = __ldcs(ve + v);
-                q4[u] = vq ? __ldcs(vq + v) : make_uchar4(255, 255, 255, 255);
-            } else {
-                s4[u] = make_int4(0, 0, 0, 0);
-                e4[u] = make_int4(-1, -1, -1, -1);  // L < 0: never in a stream
-                q4[u] = make_uchar4(0, 0, 0, 0);
-            }
-        }
-#pragma unroll
-        for (int u = 0; u < kHistUnroll; ++u) {
-            const int v = v0 + u * kHistThreads;
-            const int i = v * 4;
-            if (v == 0 && skip) {  // the widened head: mask fragments left of lo
-                if (skip <= 0) visit(s4[u].x, e4[u].x, q4[u].x, base_idx + i);
-                if (skip <= 1) visit(s4[u].y, e4[u].y, q4[u].y, base_idx + i + 1);
-                if (skip <= 2) visit(s4[u].z, e4[u].z, q4[u].z, base_idx + i + 2);
-                visit(s4[u].w, e4[u].w, q4[u].w, base_idx + i + 3);
-            } else {
-                visit(s4[u].x, e4[u].x, q4[u].x, base_idx + i);
-                visit(s4[u].y, e4[u].y, q4[u].y, base_idx + i + 1);
-                visit(s4[u].z, e4[u].z, q4[u].z, base_idx + i + 2);
-                visit(s4[u].w, e4[u].w, q4[u].w, base_idx + i + 3);
-            }
-        }
-    }
-    {   // tail: at most 3 fragments (and the head mask when the whole slice is shorter than a vector)
-        const int i = nvec * 4 + tid;
-        if (i < cnt && i >= skip)
-            visit(__ldcs(frag_start + lo_al + i), __ldcs(frag_stop + lo_al + i),
-                  frag_mapq ? (int)__ldcs(frag_mapq + lo_al + i) : 255, base_idx + i);
-    }
+    stream_fragments<kHistThreads, kHistUnroll>(FragCols{frag_start, frag_stop, frag_mapq, nullptr}, lo, hi, tid, visit);
     unsigned long long my_count = my_count32;
 
     // block reduction of the count -> one 64-bit atomic per CTA
@@ -226,13 +157,12 @@ interval_count_warp_kernel(const int32_t *__restrict__ frag_start, const int32_t
         const int64_t ivl = unit / splits;
         const int split = (int)(unit % splits);
         const int S = __ldg(ivl_start + ivl), E = __ldg(ivl_stop + ivl);
-        const int64_t lo_all = __ldg(ranges + 2 * ivl), hi_all = __ldg(ranges + 2 * ivl + 1);
-        int64_t chunk = (hi_all - lo_all + splits - 1) / splits;
-        chunk = (chunk + 3) & ~(int64_t)3;
-        const int64_t lo = lo_all + (int64_t)split * chunk;
-        const int64_t hi = min(hi_all, lo + chunk);
+        int64_t lo, hi;
+        slice_of(ranges, ivl, split, splits, lo, hi);
         const Stream in_stream(S, E, pred);
 
+        // Its own copy of the stream_fragments loop, with the head lanes masked by a flag instead of the
+        // sentinel: at the 64-register cap every formulation of the shared loop tried (nvcc 12.9) spilled more.
         const int64_t lo_al = lo & ~(int64_t)3;
         const int skip = (int)(lo - lo_al);
         const int cnt = (hi > lo) ? (int)(hi - lo_al) : 0;
@@ -445,12 +375,8 @@ extern "C" int ftk_interval_hist_u64(const int32_t *frag_start, const int32_t *f
     if (n_ivl * (int64_t)splits > INT32_MAX) return FTK_E_RANGE;
     cudaStream_t stream = static_cast<cudaStream_t>(stream_);
     const int halo = effective_halo(policy, max_frag_len, max_len);
-    {
-        const int64_t n = 2 * n_ivl;
-        interval_ranges_kernel<<<(unsigned)((n + 127) / 128), 128, 0, stream>>>(
-            frag_start, n_frag, ivl_start, ivl_stop, n_ivl, halo, scratch);
-        FTK_CHECK_LAUNCH("interval_ranges_kernel");
-    }
+    const int rc = launch_candidate_ranges(frag_start, n_frag, ivl_start, ivl_stop, false, n_ivl, halo, 0, scratch, stream);
+    if (rc != FTK_OK) return rc;
     Pred pred{policy, min_len, max_len, min_mapq};
     const unsigned grid = (unsigned)(n_ivl * splits);
     auto *c = reinterpret_cast<unsigned long long *>(counts);

@@ -48,18 +48,6 @@ __device__ __forceinline__ uint32_t digit_reverse(uint32_t x, int k) {
     return x >> (32 - 2 * k);
 }
 
-__global__ void motif_ranges_kernel(const int32_t *__restrict__ frag_start, int64_t n_frag,
-                                    const int32_t *__restrict__ ivl_start,
-                                    const int32_t *__restrict__ ivl_stop, int64_t n_ivl,
-                                    int halo, int64_t *__restrict__ ranges) {
-    int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= 2 * n_ivl) return;
-    const int64_t k = t >> 1;
-    // overlap: fe > S (=> fs > S - maxL) and fs < E
-    const int64_t key = (t & 1) ? (int64_t)ivl_stop[k] : (int64_t)ivl_start[k] - halo;
-    ranges[t] = lower_bound(frag_start, n_frag, key);
-}
-
 // Fragments are fetched four per lane with 128-bit loads (two vectors = eight fragments in flight per
 // thread); the k-mer windows are read from the L2-resident packed contig.  (A variant that staged the
 // contig span of every 4096-fragment sub-chunk in shared memory was measured in round 2 and lost:
@@ -115,11 +103,8 @@ end_motif_kernel(const int32_t *__restrict__ frag_start, const int32_t *__restri
     const int64_t ivl = blockIdx.x / splits;
     const int split = blockIdx.x % splits;
     unsigned long long *__restrict__ row = counts + (pooled ? 0 : ivl * (int64_t)n_bins);
-    const int64_t lo_all = ranges[2 * ivl], hi_all = ranges[2 * ivl + 1];
-    int64_t chunk = (hi_all - lo_all + splits - 1) / splits;
-    chunk = (chunk + 3) & ~(int64_t)3;
-    const int64_t lo = lo_all + (int64_t)split * chunk;
-    const int64_t hi = min(hi_all, lo + chunk);
+    int64_t lo, hi;
+    slice_of(ranges, ivl, split, splits, lo, hi);
     if (hi <= lo) return;
 
     const int S = ivl_start[ivl], E = ivl_stop[ivl];
@@ -282,15 +267,12 @@ static int motif_hist_launch(const int32_t *frag_start, const int32_t *frag_stop
     if (n_frag > 0 && (!frag_start || !frag_stop)) return FTK_E_INVALID;
     if (n_ivl * (int64_t)splits > INT32_MAX) return FTK_E_RANGE;
     cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-    {
-        const int64_t n = 2 * n_ivl;
-        motif_ranges_kernel<<<(unsigned)((n + 127) / 128), 128, 0, stream>>>(
-            frag_start, n_frag, ivl_start, ivl_stop, n_ivl, max_frag_len < 0 ? 0 : max_frag_len, scratch);
-        FTK_CHECK_LAUNCH("motif_ranges_kernel");
-    }
+    // overlap: fe > S (=> fs > S - max_frag_len) and fs < E
+    const int mfl = max_frag_len < 0 ? 0 : max_frag_len;
+    const int rc = launch_candidate_ranges(frag_start, n_frag, ivl_start, ivl_stop, false, n_ivl, mfl, 0, scratch, stream);
+    if (rc != FTK_OK) return rc;
     const unsigned grid = (unsigned)(n_ivl * splits);
     auto *c = reinterpret_cast<unsigned long long *>(counts);
-    const int mfl = max_frag_len < 0 ? 0 : max_frag_len;
 #define FTK_MOTIF(K, MODE, SMEM)                                                                             \
     end_motif_kernel<K, MODE, SMEM, BREAKPOINT><<<grid, kMotifThreads, 0, stream>>>(                         \
         frag_start, frag_stop, frag_mapq, frag_strand, seq_words, nmask_words, contig_len, ivl_start,        \

@@ -22,36 +22,6 @@ namespace ftk {
 constexpr int kWpsCap = 5120;                    // smem slots per tile
 static_assert(FTK_WPS_TILE < kWpsCap, "one guard slot for odd windows");
 
-// Per-tile fragment index range [lo, hi): a superset of the fragments with any
-// event inside the tile.  One thread per bound; the upper levels of the search tree stay in L2, so
-// this costs ~30 us per chr1-scale launch.  (A warp-cooperative 32-ary search - 6 dependent rounds
-// instead of 27 - was measured in round 2 and lost, 64 us: every round touches 32 sectors per warp.)
-// The prepass also zeroes the accumulators of the fused pass, so a step is two launches.
-__global__ void __launch_bounds__(128)
-wps_tile_ranges_kernel(const int32_t *__restrict__ frag_start, int64_t n_frag,
-                       const int32_t *__restrict__ tile_p0, const int32_t *__restrict__ tile_len,
-                       int64_t n_tiles, int left_reach, int b, int64_t *__restrict__ ranges,
-                       unsigned long long *__restrict__ zero_a, int64_t n_zero_a,
-                       unsigned long long *__restrict__ zero_b, int64_t n_zero_b) {
-    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    const int64_t gthreads = (int64_t)gridDim.x * blockDim.x;
-    for (int64_t i = t; i < n_zero_a; i += gthreads) zero_a[i] = 0ull;
-    for (int64_t i = t; i < n_zero_b; i += gthreads) zero_b[i] = 0ull;
-    if (t >= 2 * n_tiles) return;
-    const int64_t tile = t >> 1;
-    const int64_t p0 = tile_p0[tile];
-    int64_t key;
-    if ((t & 1) == 0) {
-        // a fragment starting more than left_reach before p0 - 1 cannot matter to the tile
-        // (WPS: its last event sits at fe+a+1 <= fs+max_len+a+1 and must be > g0 >= p0-1)
-        key = p0 - 1 - (int64_t)left_reach;
-    } else {
-        // first event sits at fs-b; it must be < p0+len
-        key = p0 + (int64_t)tile_len[tile] + (int64_t)b;
-    }
-    ranges[t] = lower_bound(frag_start, n_frag, key);
-}
-
 // ---------------------------------------------------------------------------
 // Tile parameters, the fragment scatter and the score stores
 // ---------------------------------------------------------------------------
@@ -578,24 +548,20 @@ static int wps_check_args(const int32_t *frag_start, const int32_t *frag_stop, i
     return FTK_OK;
 }
 
-// left_reach: how far left of p0 - 1 a fragment may start and still matter to the tile
+// Per-tile fragment index range [lo, hi): a superset of the fragments with any event inside the tile.
+// left_reach: how far left of p0 - 1 a fragment may start and still matter to the tile; a fragment's first
+// event sits at fs - b and must be < p0 + len.
 static int launch_tile_ranges(const int32_t *frag_start, int64_t n_frag, const int32_t *tile_p0,
                               const int32_t *tile_len, int64_t n_tiles, int32_t window_size,
                               int64_t left_reach, int64_t *scratch, cudaStream_t stream,
                               unsigned long long *zero_a = nullptr, int64_t n_zero_a = 0,
                               unsigned long long *zero_b = nullptr, int64_t n_zero_b = 0) {
-    using namespace ftk;
     const bool odd = (window_size & 1) != 0;
     const int a = odd ? (window_size - 1) / 2 : window_size / 2;
     const int b = odd ? a : a - 1;
     if (left_reach > INT32_MAX / 2) left_reach = INT32_MAX / 2;
-    const int64_t n = 2 * n_tiles;
-    const int threads = 128;
-    wps_tile_ranges_kernel<<<(unsigned)((n + threads - 1) / threads), threads, 0, stream>>>(
-        frag_start, n_frag, tile_p0, tile_len, n_tiles, (int)left_reach, b, scratch, zero_a, n_zero_a, zero_b,
-        n_zero_b);
-    FTK_CHECK_LAUNCH("wps_tile_ranges_kernel");
-    return FTK_OK;
+    return ftk::launch_candidate_ranges(frag_start, n_frag, tile_p0, tile_len, true, n_tiles, 1 + left_reach, b,
+                                        scratch, stream, zero_a, n_zero_a, zero_b, n_zero_b);
 }
 
 static int64_t wps_left_reach(int32_t window_size, int32_t max_len) {

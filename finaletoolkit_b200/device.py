@@ -315,8 +315,7 @@ def _splits_for(n_ivl: int, n_frag: int, unit_frags: int | None = None) -> int:
     waves of units; estimated from the contig-wide mean fragments per interval."""
     if n_ivl <= 0:
         return 1
-    import os
-    unit = int(os.environ.get("FTK_UNIT_FRAGS", _UNIT_FRAGS)) if unit_frags is None else int(unit_frags)
+    unit = _UNIT_FRAGS if unit_frags is None else int(unit_frags)
     by_size = -(-(n_frag // max(n_ivl, 1)) // unit)
     by_grid = -(-4 * _TARGET_CTAS // n_ivl)
     return int(max(1, min(max(by_size, by_grid), 65536)))
@@ -433,28 +432,24 @@ def end_motif_hist(frags: ContigFragments, ref: PackedContig, ivl_start, ivl_sto
         counts = t.zeros((max(rows, 1), 4 ** k), dtype=t.int64, device=dev)
     if n_ivl == 0:
         return counts[:rows]
-    s_dev, e_dev = _ivl_to_device(ivl_start, ivl_stop, dev)
-    scratch = t.empty(2 * n_ivl, dtype=t.int64, device=dev)
+    ivl = IntervalSet(ivl_start, ivl_stop, dev)
     err = t.zeros(1, dtype=t.int32, device=dev)
     fs, fe, mq = frags.ptrs()
     sd = 0 if frags.strand is None else frags.strand.data_ptr()
-    # a CTA zeroes and flushes a 4^k-bin histogram: give it enough fragments to amortise that
     # a CTA's fixed latency chain (ranges -> slice bounds -> N pre-scan -> first fragments -> windows) is
     # paid once per slice: 16 K fragments amortise it (and the zero + flush of a 4^k-bin histogram)
-    import os
-    unit = int(os.environ.get("FTK_MOTIF_UNIT", 16384))
-    splits = _splits_for(n_ivl, frags.n, unit_frags=max(unit, 16 * 4 ** min(int(k), 6)))
+    splits = _splits_for(n_ivl, frags.n, unit_frags=max(16384, 16 * 4 ** min(int(k), 6)))
     if breakpoint:
         check(lib().ftk_breakpoint_motif_hist_u64(
             fs, fe, mq, sd, frags.n, frags.max_len, ref.seq.data_ptr(), ref.nmask.data_ptr(), ref.length,
-            s_dev.data_ptr(), e_dev.data_ptr(), n_ivl, int(k), int(strand_mode), int(quality_threshold),
-            int(bool(pooled)), splits, scratch.data_ptr(), counts.data_ptr(),
+            ivl.start.data_ptr(), ivl.stop.data_ptr(), n_ivl, int(k), int(strand_mode), int(quality_threshold),
+            int(bool(pooled)), splits, ivl.scratch.data_ptr(), counts.data_ptr(),
             _stream_ptr(dev)), "ftk_breakpoint_motif_hist_u64")
         return counts[:rows]
     check(lib().ftk_end_motif_hist_u64(
         fs, fe, mq, sd, frags.n, frags.max_len, ref.seq.data_ptr(), ref.nmask.data_ptr(), ref.length,
-        s_dev.data_ptr(), e_dev.data_ptr(), n_ivl, int(k), int(strand_mode), int(quality_threshold),
-        int(bool(pooled)), splits, scratch.data_ptr(), counts.data_ptr(),
+        ivl.start.data_ptr(), ivl.stop.data_ptr(), n_ivl, int(k), int(strand_mode), int(quality_threshold),
+        int(bool(pooled)), splits, ivl.scratch.data_ptr(), counts.data_ptr(),
         err.data_ptr(), _stream_ptr(dev)), "ftk_end_motif_hist_u64")
     if int(err.item()):
         raise RuntimeError(
@@ -497,8 +492,7 @@ def delfi_windows(frags: ContigFragments, ref: PackedContig | None, win_start, w
     counts = t.zeros((max(n_win, 1), 4), dtype=t.int64, device=dev)
     if n_win == 0:
         return counts[:0]
-    s_dev, e_dev = _ivl_to_device(win_start, win_stop, dev)
-    scratch = t.empty(2 * n_win, dtype=t.int64, device=dev)
+    win = IntervalSet(win_start, win_stop, dev)
     fs, fe, mq = frags.ptrs()
     bl = (0, 0, 0)
     keep = []
@@ -516,8 +510,8 @@ def delfi_windows(frags: ContigFragments, ref: PackedContig | None, win_start, w
     check(lib().ftk_delfi_windows_u64(
         fs, fe, mq, frags.n, frags.max_len, 0 if ref is None else ref.seq.data_ptr(),
         0 if ref is None else ref.nmask.data_ptr(), 0 if ref is None else ref.length,
-        s_dev.data_ptr(), e_dev.data_ptr(), n_win, *bl, None if g5 is None else _np_ptr(g5, c_int32),
-        int(quality_threshold), _splits_for(n_win, frags.n), scratch.data_ptr(), counts.data_ptr(),
+        win.start.data_ptr(), win.stop.data_ptr(), n_win, *bl, None if g5 is None else _np_ptr(g5, c_int32),
+        int(quality_threshold), _splits_for(n_win, frags.n), win.scratch.data_ptr(), counts.data_ptr(),
         _stream_ptr(dev)), "ftk_delfi_windows_u64")
     return counts
 

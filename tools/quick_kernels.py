@@ -1,6 +1,7 @@
-"""Kernel timing helper (python tools/quick_kernels.py [motif] [bp] [adjust] [delfi] [cleavage] [depth] [depth-mid]): CUDA-event time of
-the secondary kernels at chr1 scale (80 M fragments drawn on the GPU), median of 7 calls after 3 warm-ups (the call:
-planning and uploads included); cleavage / depth also print each kernel's own device time (torch.profiler)."""
+"""Kernel timing helper (python tools/quick_kernels.py [motif] [bp] [adjust] [delfi] [hist] [cleavage] [depth] [depth-mid]):
+CUDA-event time of the secondary kernels at chr1 scale (80 M fragments drawn on the GPU), median of 7 calls after 3
+warm-ups (the call: planning and uploads included).  Every op except adjust also prints an order-sensitive checksum
+of its output (compare two builds with it) and each kernel's own device time (torch.profiler, a separate run)."""
 import os
 import sys
 
@@ -46,41 +47,51 @@ def kernels(fn, reps=5):
             print(f"  kernel {ev.key.split('(')[0]}: {ev.device_time_total / reps / 1e3:.3f} ms", flush=True)
 
 
+def checksum(o):
+    """Order-sensitive checksum of an output tensor's bits (int64 arithmetic wraps)."""
+    x = o.contiguous().flatten()
+    if x.is_floating_point():
+        x = x.view({8: torch.int64, 4: torch.int32}[x.element_size()])
+    x = x.to(torch.int64)
+    return int((x * torch.arange(1, x.numel() + 1, dtype=torch.int64, device=x.device)).sum())
+
+
+def op(name, fn, nbytes, result=lambda o: o):
+    o = timed(name, fn, nbytes)
+    print("  checksum", checksum(result(o)), flush=True)
+    kernels(fn)
+
+
 if what & {"motif", "bp", "delfi"}:
     codes, nm = synth_twobit(CLEN, 0)
     ref = D.PackedContig.from_codes(codes, nm, device=dev)
     ws = np.arange(0, CLEN, 1_000_000, dtype=np.int64); we = np.minimum(ws + 1_000_000, CLEN)
+tiles = np.arange(0, CLEN + 5000, 5000, dtype=np.int64).clip(max=CLEN)
 if "motif" in what:
-    o = timed("end_motifs k=4", lambda: D.end_motif_hist(fr, ref, ws, we, k=4, strand_mode=0, quality_threshold=30, pooled=True), 10 * N)
-    print("  checksum", int(o.sum()))
-    timed("end_motifs k=3 (runtime-K variant)", lambda: D.end_motif_hist(fr, ref, ws, we, k=3, strand_mode=0, quality_threshold=30, pooled=True), 10 * N)
+    op("end_motifs k=4", lambda: D.end_motif_hist(fr, ref, ws, we, k=4, strand_mode=0, quality_threshold=30, pooled=True), 10 * N)
+    op("end_motifs k=3 (runtime-K variant)", lambda: D.end_motif_hist(fr, ref, ws, we, k=3, strand_mode=0, quality_threshold=30, pooled=True), 10 * N)
 if "bp" in what:
-    o = timed("breakpoint_motifs k=6", lambda: D.end_motif_hist(fr, ref, ws, we, k=6, strand_mode=0, quality_threshold=30, pooled=True, breakpoint=True), 10 * N)
-    print("  checksum", int(o.sum()))
+    op("breakpoint_motifs k=6", lambda: D.end_motif_hist(fr, ref, ws, we, k=6, strand_mode=0, quality_threshold=30, pooled=True, breakpoint=True), 10 * N)
 if "delfi" in what:
     bs = np.arange(0, CLEN, 100_000, dtype=np.int64); be = np.minimum(bs + 100_000, CLEN)
-    timed("delfi 100-kb bins", lambda: D.delfi_windows(fr, ref, bs, be, quality_threshold=30), 9 * N + CLEN * 3 // 8)
+    op("delfi 100-kb bins", lambda: D.delfi_windows(fr, ref, bs, be, quality_threshold=30), 9 * N + CLEN * 3 // 8)
 if "cleavage" in what:
-    edges = np.arange(0, CLEN + 5000, 5000, dtype=np.int64).clip(max=CLEN)
-    run = lambda: D.cleavage_intervals(fr, edges[:-1], edges[1:], CLEN, None, None, 30)   # noqa: E731
-    timed("cleavage", run, 10 * N + 8 * CLEN)
-    kernels(run)
-if what & {"depth", "depth-mid"}:
-    edges = np.arange(0, CLEN + 5000, 5000, dtype=np.int64).clip(max=CLEN)
-    for name in ("depth", "depth-mid"):
-        if name in what:
-            run = lambda: D.depth_intervals(fr, edges[:-1], edges[1:], CLEN, None, None, 30, name == "depth-mid")  # noqa: E731
-            o = timed(name, run, 9 * N + 4 * CLEN)
-            print("  checksum", int(o[0].sum(dtype=torch.int64)))
-            kernels(run)
+    op("cleavage", lambda: D.cleavage_intervals(fr, tiles[:-1], tiles[1:], CLEN, None, None, 30), 10 * N + 8 * CLEN, lambda o: o[0])
+for name in ("depth", "depth-mid"):
+    if name in what:
+        op(name, lambda: D.depth_intervals(fr, tiles[:-1], tiles[1:], CLEN, None, None, 30, name == "depth-mid"), 9 * N + 4 * CLEN,
+           lambda o: o[0])
 if "hist" in what:
-    edges = np.arange(0, CLEN + 5000, 5000, dtype=np.int64).clip(max=CLEN)
-    timed("coverage counts (5-kb intervals)", lambda: D.interval_hist(fr, edges[:-1], edges[1:], "midpoint", None, None, 30), 9 * N)
-    timed("coverage counts + pooled length histogram", lambda: D.interval_hist(fr, edges[:-1], edges[1:], "midpoint", None, None, 30, n_bins=601, pooled="hist"), 9 * N)
-    timed("per-interval length histograms (frag_length_intervals)", lambda: D.interval_hist(fr, edges[:-1], edges[1:], "midpoint", None, None, 30, n_bins=601, first_seen=True), 9 * N)
+    op("coverage counts (5-kb intervals)", lambda: D.interval_hist(fr, tiles[:-1], tiles[1:], "midpoint", None, None, 30), 9 * N,
+       lambda o: o[0])
+    op("coverage counts + pooled length histogram",
+       lambda: D.interval_hist(fr, tiles[:-1], tiles[1:], "midpoint", None, None, 30, n_bins=601, pooled="hist"), 9 * N,
+       lambda o: torch.cat([o[0], o[1].flatten()]))
+    op("per-interval length histograms (frag_length_intervals)",
+       lambda: D.interval_hist(fr, tiles[:-1], tiles[1:], "midpoint", None, None, 30, n_bins=601, first_seen=True), 9 * N,
+       lambda o: torch.cat([o[0], o[1].flatten(), o[2].flatten().to(torch.int64)]))
 if "adjust" in what:
-    edges = np.arange(0, CLEN + 5000, 5000, dtype=np.int64).clip(max=CLEN)
-    plan = D.WpsPlan(edges[:-1], edges[1:], CLEN, 180, dev)
+    plan = D.WpsPlan(tiles[:-1], tiles[1:], CLEN, 180, dev)
     wps = plan.run(fr)
     ap = D.AdjustPlan(np.diff(plan.offsets), 1000, True, 21, 2, dev, skip_short=True)
     out = torch.empty(ap.n_total, dtype=torch.float64, device=dev)
