@@ -5,7 +5,8 @@ Table-driven Click group.  For every in-scope subcommand the flag spellings, par
 (cli/commands/__init__.py:87-640); dispatch filters the parameters by the target's signature like
 cli/_dispatch.py:96-118 and expands ``--strand`` into both_strands / negative_strand
 (cli/_dispatch.py:25-36).  Out-of-scope subcommands (delfi, breakpoint motifs, filter-file, agg-bw,
-gap-bed) are not registered.  ``EXTRA_COMMANDS`` holds the subcommands this package adds (coverage-profile).
+gap-bed) are not registered.  ``EXTRA_COMMANDS`` and ``SITE_COMMANDS`` hold the subcommands this package adds (coverage-profile,
+vplot).
 """
 from __future__ import annotations
 
@@ -175,6 +176,20 @@ EXTRA_COMMANDS = {
         _THREADS, _VERBOSE]),
 }
 
+# site-aggregate subcommands added here, in their own table so COMMANDS / EXTRA_COMMANDS keep their exact sets
+SITE_COMMANDS = {
+    "vplot": ("finaletoolkit_b200.frag", "vplot",
+              "Fragment-length x midpoint-offset counts (V-plot) summed over BED sites.", [
+        _INPUT, _arg("site_bed", metavar="SITES"), _REF, _out("TSV (or .tsv.gz) of the V-plot matrix."),
+        _opt("--flank", "flank", metavar="BP", default=1000, show_default=True, type=int,
+             help="Largest midpoint offset from a site centre."),
+        _opt("--min-length", "min_length", metavar="BP", default=0, show_default=True, type=int,
+             help="Minimum fragment length (first row)."),
+        _opt("--max-length", "max_length", metavar="BP", default=500, show_default=True, type=int,
+             help="Maximum fragment length (last row)."),
+        _mapq(30), _THREADS, _VERBOSE]),
+}
+
 
 def run(module: str, func: str, params: dict):
     """Import the target lazily, translate --strand, keep only the kwargs it accepts, call it."""
@@ -203,7 +218,7 @@ def main_cli():
     """finaletoolkit_b200: the B200-native hot path of FinaleToolkit."""
 
 
-for _name, (_module, _func, _help, _spec) in {**COMMANDS, **EXTRA_COMMANDS}.items():
+for _name, (_module, _func, _help, _spec) in {**COMMANDS, **EXTRA_COMMANDS, **SITE_COMMANDS}.items():
     main_cli.add_command(_make(_name, _module, _func, _help, _spec))
 
 

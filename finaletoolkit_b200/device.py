@@ -13,7 +13,8 @@ import numpy as np
 from ._lib import FTK_NONE, FtkLibraryError, check, lib
 
 __all__ = ["ContigFragments", "WpsPlan", "AdjustPlan", "IntervalSet", "PackedContig", "interval_hist", "frag_lengths",
-           "end_motif_hist", "delfi_windows", "blacklist_in_windows", "agg_signal", "require_cuda", "none_to_ftk", "policy_code"]
+           "end_motif_hist", "delfi_windows", "blacklist_in_windows", "agg_signal", "require_cuda", "none_to_ftk", "policy_code",
+           "vplot_sites"]
 
 _torch = None
 
@@ -382,6 +383,59 @@ def interval_hist(frags: ContigFragments, ivl_start=None, ivl_stop=None, interse
         ivl_set.scratch.data_ptr(), counts.data_ptr(), 0 if hist is None else hist.data_ptr(),
         0 if first is None else first.data_ptr(), _stream_ptr(dev)), "ftk_interval_hist_u64")
     return counts[:rows], hist, first
+
+
+VPLOT_MAX_FLANK = 1 << 20
+VPLOT_MAX_CELLS = 1 << 27
+
+
+def vplot_check(flank, min_length, max_length):
+    """ValueError unless ``0 <= min_length <= max_length`` (integers), ``0 <= flank <= 2**20`` and the matrix has at
+    most 2**27 cells; returns its shape ``(max_length - min_length + 1, 2 * flank + 1)``."""
+    if min_length is None or max_length is None:
+        raise ValueError("min_length and max_length must both be given (the rows of the V-plot matrix)")
+    flank, min_length, max_length = int(flank), int(min_length), int(max_length)
+    if min_length < 0 or max_length < min_length:
+        raise ValueError(f"need 0 <= min_length <= max_length, got {min_length} and {max_length}")
+    if flank < 0 or flank > VPLOT_MAX_FLANK:
+        raise ValueError(f"flank must lie in [0, {VPLOT_MAX_FLANK}], got {flank}")
+    shape = (max_length - min_length + 1, 2 * flank + 1)
+    if shape[0] * shape[1] > VPLOT_MAX_CELLS:
+        raise ValueError(f"a {shape[0]} x {shape[1]} V-plot exceeds {VPLOT_MAX_CELLS} cells")
+    return shape
+
+
+def vplot_sites(frags: ContigFragments, site_center, site_flip, flank, min_length, max_length, quality_threshold=30,
+                out=None):
+    """Fragment-length x midpoint-offset counts summed over the sites of one contig (``ftk_vplot_u64``).
+
+    Site k is centred on ``site_center[k]`` and mirrored when ``site_flip[k]`` is true; a passing fragment (mapq >=
+    ``quality_threshold``, ``min_length <= L <= max_length``) whose midpoint ``(start + stop) // 2`` lies within
+    ``flank`` of the centre adds 1 at ``[L - min_length, offset + flank]``.  Returns the device int64 matrix of
+    shape ``(max_length - min_length + 1, 2 * flank + 1)``; ``out`` (such a matrix) is accumulated into."""
+    t = torch()
+    shape = vplot_check(flank, min_length, max_length)
+    dev = frags.device
+    if out is None:
+        out = t.zeros(shape, dtype=t.int64, device=dev)
+    elif out.dtype != t.int64 or tuple(out.shape) != shape or not out.is_contiguous():
+        raise ValueError(f"out must be a contiguous int64 tensor of shape {shape}")
+    c = np.asarray(site_center, dtype=np.int64).reshape(-1)
+    n = c.size
+    if n == 0:
+        return out
+    flank = int(flank)
+    lim = 2 ** 31 - 1
+    if int(c.min()) - flank < -lim or int(c.max()) > lim:
+        raise ValueError("site centres must lie within the int32 coordinate range")
+    sites = IntervalSet(c - flank, c + flank + 1, dev)   # centre = window start + flank
+    flip = _to_device(np.asarray(site_flip, dtype=bool).reshape(-1).astype(np.uint8), dev, np.uint8)
+    fs, fe, mq = frags.ptrs()
+    check(lib().ftk_vplot_u64(
+        fs, fe, mq, frags.n, frags.max_len, sites.start.data_ptr(), sites.stop.data_ptr(), flip.data_ptr(), n,
+        flank, int(min_length), int(max_length), int(quality_threshold), _splits_for(n, frags.n),
+        sites.scratch.data_ptr(), out.data_ptr(), _stream_ptr(dev)), "ftk_vplot_u64")
+    return out
 
 
 def frag_lengths(frags: ContigFragments, start=None, stop=None, intersect_policy="midpoint",

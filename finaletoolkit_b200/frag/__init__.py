@@ -6,6 +6,7 @@ from ._multi_wps import multi_wps
 from ._adjust_wps import adjust_wps
 from ._cleavage_profile import cleavage_profile, multi_cleavage_profile
 from ._coverage_profile import coverage_profile, multi_coverage_profile
+from ._vplot import vplot
 from ._end_motifs import (EndMotifFreqs, EndMotifsIntervals, region_end_motifs, end_motifs,
                           interval_end_motifs)
 from ._delfi import delfi, delfi_gc_correct, delfi_merge_bins, trim_coverage
@@ -14,7 +15,7 @@ from ._breakpoint_motifs import (BreakpointMotifFreqs, BreakpointMotifsIntervals
 
 __all__ = ["frag_length", "frag_length_bins", "frag_length_intervals", "FragLengthStats", "coverage",
            "single_coverage", "CoverageResult", "wps", "multi_wps", "adjust_wps", "cleavage_profile",
-           "multi_cleavage_profile", "coverage_profile", "multi_coverage_profile", "EndMotifFreqs",
+           "multi_cleavage_profile", "coverage_profile", "multi_coverage_profile", "vplot", "EndMotifFreqs",
            "EndMotifsIntervals", "region_end_motifs", "end_motifs", "interval_end_motifs", "BreakpointMotifFreqs",
            "BreakpointMotifsIntervals", "region_breakpoint_motifs", "breakpoint_motifs",
            "interval_breakpoint_motifs", "delfi", "delfi_gc_correct", "delfi_merge_bins", "trim_coverage"]

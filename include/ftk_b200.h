@@ -410,6 +410,26 @@ int ftk_depth_tiles_i32(const int32_t *frag_start_dev, const int32_t *frag_stop_
                         int32_t min_len, int32_t max_len, int32_t min_mapq, int32_t midpoint,
                         int64_t *scratch_dev, int32_t *out_dev, ftk_stream_t stream);
 
+/* ---------------------------------------------------------------- V-plot
+ * Site-centred fragment V-plot: a fragment-length x midpoint-offset count matrix summed over sites.
+ * Site k has the window [win_lo[k], win_hi[k]) = [c - flank, c + flank + 1) around its centre c (the
+ * kernel reads c = win_lo[k] + flank; win_hi only bounds the candidate search) and is flipped when
+ * site_flip[k] != 0 ('-' strand).  A fragment passes when mapq >= min_mapq and min_len <= L <= max_len,
+ * L = stop - start; its midpoint is m = (start + stop) / 2 and its offset d = m - c (flipped: c - m).
+ * For every site and every passing fragment with |d| <= flank:
+ *   out[(L - min_len) * (2 * flank + 1) + d + flank] += 1
+ * so a fragment counts once per site whose window holds its midpoint (duplicate sites count again).
+ * out_dev: uint64[(max_len - min_len + 1) * (2 * flank + 1)], ACCUMULATED (the caller zeroes it).
+ * Each site's candidate range is split into `splits` slices, one warp each.  scratch_dev: int64[2*n_sites].
+ * max_frag_len = max(stop - start) over the contig.  0 <= min_len <= max_len, 0 <= flank <= FTK_VPLOT_MAX_FLANK,
+ * at most FTK_VPLOT_MAX_CELLS cells; n_sites == 0 or n_frag == 0 returns 0 without a launch. */
+#define FTK_VPLOT_MAX_FLANK (1 << 20)
+#define FTK_VPLOT_MAX_CELLS (1 << 27)
+int ftk_vplot_u64(const int32_t *frag_start_dev, const int32_t *frag_stop_dev, const uint8_t *frag_mapq_dev,
+                  int64_t n_frag, int32_t max_frag_len, const int32_t *win_lo_dev, const int32_t *win_hi_dev,
+                  const uint8_t *site_flip_dev, int64_t n_sites, int32_t flank, int32_t min_len, int32_t max_len,
+                  int32_t min_mapq, int32_t splits, int64_t *scratch_dev, uint64_t *out_dev, ftk_stream_t stream);
+
 /* ------------------------------------------------- fragment file decode (host)
  * Multi-threaded decode of a BGZF / gzip fragment file into per-contig columns; replaces the
  * per-interval pysam.TabixFile.fetch text stream of io/alignment.py:270-302 (5-column FinaleDB

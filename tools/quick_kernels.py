@@ -1,4 +1,5 @@
-"""Kernel timing helper (python tools/quick_kernels.py [motif] [bp] [adjust] [delfi] [hist] [cleavage] [depth] [depth-mid]):
+"""Kernel timing helper (python tools/quick_kernels.py [motif] [bp] [adjust] [delfi] [hist] [cleavage] [depth] [depth-mid]
+[vplot] [vplot-dense]):
 CUDA-event time of the secondary kernels at chr1 scale (80 M fragments drawn on the GPU), median of 7 calls after 3
 warm-ups (the call: planning and uploads included).  Every op except adjust also prints an order-sensitive checksum
 of its output (compare two builds with it) and each kernel's own device time (torch.profiler, a separate run)."""
@@ -30,7 +31,7 @@ def timed(name, fn, nbytes):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record(); out = fn(); e1.record(); torch.cuda.synchronize()
         ts.append(e0.elapsed_time(e1))
-    ms = float(np.median(ts))
+    ms = timed.ms = float(np.median(ts))
     print(f"{name}: {ms:.3f} ms (min {min(ts):.3f})  {nbytes / ms / 1e6:.0f} GB/s = {nbytes / ms / 1e6 / 6541.1:.1%} of measured HBM peak", flush=True)
     return out
 
@@ -90,6 +91,21 @@ if "hist" in what:
     op("per-interval length histograms (frag_length_intervals)",
        lambda: D.interval_hist(fr, tiles[:-1], tiles[1:], "midpoint", None, None, 30, n_bins=601, first_seen=True), 9 * N,
        lambda o: torch.cat([o[0], o[1].flatten(), o[2].flatten().to(torch.int64)]))
+for name, step in (("vplot", 5000), ("vplot-dense", 500)):
+    if name in what:
+        # sites every `step` bp (49 850 at 5 kb), strands alternating, flank 1000, lengths 0..600
+        vc = np.arange(step // 2, CLEN, step, dtype=np.int64)
+        vf = np.arange(vc.size) % 2 == 1
+        made = []
+        interval_set = D.IntervalSet
+        D.IntervalSet = lambda *a, **k: made.append(interval_set(*a, **k)) or made[-1]   # keep the range scratch
+        m = D.vplot_sites(fr, vc, vf, 1000, 0, 600, 30)
+        D.IntervalSet = interval_set
+        rng = made[-1].scratch[: 2 * vc.size].view(-1, 2)
+        cand, events = int((rng[:, 1] - rng[:, 0]).sum()), int(m.sum())
+        print(f"{name}: {vc.size} sites, {cand} candidates, {events} events", flush=True)
+        op(name, lambda: D.vplot_sites(fr, vc, vf, 1000, 0, 600, 30), 9 * cand)
+        print(f"  {events / timed.ms / 1e6:.2f} G events/s over the call", flush=True)
 if "adjust" in what:
     plan = D.WpsPlan(tiles[:-1], tiles[1:], CLEN, 180, dev)
     wps = plan.run(fr)
