@@ -29,9 +29,10 @@ struct Pred {
 // None handling and the length window folded into per-CTA constants:
 //   tabix fetch(contig, S, E): rec.stop > start (None -> 0) and rec.start < stop
 //   length filter inclusive; midpoint policy mid in [S, E); "any" = the overlap test itself
+// The upper bound is kept inclusive (e_last = E - 1) so that E = None admits a start or midpoint of 2^31 - 1.
 struct Stream {
     int len_lo; unsigned len_span; bool len_any;
-    int min_mapq; int s_over; int e_eff; int s_mid; bool midpoint;
+    int min_mapq; int s_over; int e_last; int s_mid; bool midpoint;
     __device__ __forceinline__ Stream(int S, int E, const Pred &p) {
         len_lo = (p.min_len == FTK_NONE || p.min_len < 0) ? 0 : p.min_len;
         const int hi = (p.max_len == FTK_NONE) ? INT32_MAX : p.max_len;
@@ -40,7 +41,7 @@ struct Stream {
         min_mapq = p.min_mapq;
         s_over = (S == FTK_NONE) ? 0 : S;
         s_mid = (S == FTK_NONE) ? INT32_MIN : S;
-        e_eff = (E == FTK_NONE) ? INT32_MAX : E;
+        e_last = (E == FTK_NONE) ? INT32_MAX : E - 1;   // E > FTK_NONE here: no wrap
         midpoint = p.policy == FTK_POLICY_MIDPOINT;
     }
     // Branch-free: every test is evaluated and AND-ed (predicate logic, no short-circuit branches).
@@ -49,8 +50,8 @@ struct Stream {
         const int mid = fs + (L >> 1);
         const unsigned ok_len = (unsigned)((unsigned)(L - len_lo) <= len_span);
         const unsigned ok_q = (unsigned)(q >= min_mapq);
-        const unsigned ok_over = (unsigned)(fe > s_over) & (unsigned)(fs < e_eff);
-        const unsigned ok_mid = midpoint ? ((unsigned)(mid >= s_mid) & (unsigned)(mid < e_eff)) : 1u;
+        const unsigned ok_over = (unsigned)(fe > s_over) & (unsigned)(fs <= e_last);
+        const unsigned ok_mid = midpoint ? ((unsigned)(mid >= s_mid) & (unsigned)(mid <= e_last)) : 1u;
         return (ok_len & ok_q & ok_over & ok_mid & (unsigned)len_any) != 0u;
     }
 };

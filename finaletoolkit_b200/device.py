@@ -428,7 +428,10 @@ def vplot_sites(frags: ContigFragments, site_center, site_flip, flank, min_lengt
     lim = 2 ** 31 - 1
     if int(c.min()) - flank < -lim or int(c.max()) > lim:
         raise ValueError("site centres must lie within the int32 coordinate range")
-    sites = IntervalSet(c - flank, c + flank + 1, dev)   # centre = window start + flank
+    # centre = window start + flank; a window that ends past 2**31 - 1 has no upper bound (None), since a stop
+    # clipped to 2**31 - 1 would drop a fragment starting there
+    hi = c + flank + 1
+    sites = IntervalSet(c - flank, hi if int(hi.max()) <= lim else [None if v > lim else v for v in hi.tolist()], dev)
     flip = _to_device(np.asarray(site_flip, dtype=bool).reshape(-1).astype(np.uint8), dev, np.uint8)
     fs, fe, mq = frags.ptrs()
     check(lib().ftk_vplot_u64(
