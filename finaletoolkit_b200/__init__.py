@@ -19,7 +19,7 @@ _EXPORTS = {
     "wps": ("frag", "wps"), "multi_wps": ("frag", "multi_wps"), "adjust_wps": ("frag", "adjust_wps"),
     "cleavage_profile": ("frag", "cleavage_profile"), "multi_cleavage_profile": ("frag", "multi_cleavage_profile"),
     "coverage_profile": ("frag", "coverage_profile"), "multi_coverage_profile": ("frag", "multi_coverage_profile"),
-    "vplot": ("frag", "vplot"),
+    "vplot": ("frag", "vplot"), "gc_bias": ("frag", "gc_bias"), "GCBias": ("frag", "GCBias"),
     "end_motifs": ("frag", "end_motifs"), "region_end_motifs": ("frag", "region_end_motifs"),
     "interval_end_motifs": ("frag", "interval_end_motifs"),
     "EndMotifFreqs": ("frag", "EndMotifFreqs"), "EndMotifsIntervals": ("frag", "EndMotifsIntervals"),

@@ -75,6 +75,9 @@ SYMBOLS = {
                                     c_int32, c_int32, c_int32, c_int32, _P, _P, _P]),
     "ftk_vplot_u64": (c_int, [_P, _P, _P, c_int64, c_int32, _P, _P, _P, c_int64, c_int32, c_int32, c_int32,
                               c_int32, c_int32, _P, _P, _P]),
+    "ftk_gc_observed_u64": (c_int, [_P, _P, _P, c_int64, c_int32, _P, _P, c_int64, _P, _P, c_int64, c_int32, c_int32,
+                                    c_int32, c_int32, _P, _P, _P]),
+    "ftk_gc_expected_u64": (c_int, [_P, _P, c_int64, _P, _P, c_int64, c_int32, c_int32, c_int32, _P, _P]),
     "ftk_fragfile_open": (c_void_p, [c_char_p, c_int32, _i32p]),
     "ftk_fragfile_open_slice": (c_void_p, [c_char_p, c_int64, c_int32, c_int64, c_int32, c_int32, c_int32, _i32p]),
     "ftk_bamfile_open": (c_void_p, [c_char_p, c_int32, _i32p]),

@@ -5,8 +5,8 @@ Table-driven Click group.  For every in-scope subcommand the flag spellings, par
 (cli/commands/__init__.py:87-640); dispatch filters the parameters by the target's signature like
 cli/_dispatch.py:96-118 and expands ``--strand`` into both_strands / negative_strand
 (cli/_dispatch.py:25-36).  Out-of-scope subcommands (delfi, breakpoint motifs, filter-file, agg-bw,
-gap-bed) are not registered.  ``EXTRA_COMMANDS`` and ``SITE_COMMANDS`` hold the subcommands this package adds (coverage-profile,
-vplot).
+gap-bed) are not registered.  ``EXTRA_COMMANDS``, ``SITE_COMMANDS`` and ``BIAS_COMMANDS`` hold the subcommands this package adds
+(coverage-profile, vplot, gc-bias).
 """
 from __future__ import annotations
 
@@ -190,6 +190,21 @@ SITE_COMMANDS = {
         _mapq(30), _THREADS, _VERBOSE]),
 }
 
+# bias-measurement subcommands added here, in their own table for the same reason
+BIAS_COMMANDS = {
+    "gc-bias": ("finaletoolkit_b200.frag", "gc_bias",
+                "Observed and expected fragment counts by length and G+C content, and their ratio.", [
+        _INPUT, _arg("refseq_file", metavar="REFERENCE"),
+        _opt("--regions", "interval_file", metavar="BED", default=None,
+             help="BED of regions to count in (default: every contig the input and the reference share)."),
+        _REF, _out("TSV (or .tsv.gz) of counts and ratios by length and G+C bases."),
+        _opt("--min-length", "min_length", metavar="BP", default=50, show_default=True, type=int,
+             help="Minimum fragment length (first row)."),
+        _opt("--max-length", "max_length", metavar="BP", default=500, show_default=True, type=int,
+             help="Maximum fragment length (last row, at most 1024)."),
+        _mapq(30), _THREADS, _VERBOSE]),
+}
+
 
 def run(module: str, func: str, params: dict):
     """Import the target lazily, translate --strand, keep only the kwargs it accepts, call it."""
@@ -218,7 +233,7 @@ def main_cli():
     """finaletoolkit_b200: the B200-native hot path of FinaleToolkit."""
 
 
-for _name, (_module, _func, _help, _spec) in {**COMMANDS, **EXTRA_COMMANDS, **SITE_COMMANDS}.items():
+for _name, (_module, _func, _help, _spec) in {**COMMANDS, **EXTRA_COMMANDS, **SITE_COMMANDS, **BIAS_COMMANDS}.items():
     main_cli.add_command(_make(_name, _module, _func, _help, _spec))
 
 

@@ -14,7 +14,7 @@ from ._lib import FTK_NONE, FtkLibraryError, check, lib
 
 __all__ = ["ContigFragments", "WpsPlan", "AdjustPlan", "IntervalSet", "PackedContig", "interval_hist", "frag_lengths",
            "end_motif_hist", "delfi_windows", "blacklist_in_windows", "agg_signal", "require_cuda", "none_to_ftk", "policy_code",
-           "vplot_sites"]
+           "vplot_sites", "gc_observed", "gc_expected"]
 
 _torch = None
 
@@ -438,6 +438,102 @@ def vplot_sites(frags: ContigFragments, site_center, site_flip, flank, min_lengt
         fs, fe, mq, frags.n, frags.max_len, sites.start.data_ptr(), sites.stop.data_ptr(), flip.data_ptr(), n,
         flank, int(min_length), int(max_length), int(quality_threshold), _splits_for(n, frags.n),
         sites.scratch.data_ptr(), out.data_ptr(), _stream_ptr(dev)), "ftk_vplot_u64")
+    return out
+
+
+GC_MAX_LENGTH = 1024   # FTK_GC_MAX_LENGTH
+GC_MAX_TILE = 16384    # FTK_GC_MAX_TILE
+
+
+def gc_check(min_length, max_length):
+    """ValueError unless ``1 <= min_length <= max_length <= 1024`` (integers); returns the shape of the GC-bias
+    matrices ``(max_length - min_length + 1, max_length + 1)``."""
+    if min_length is None or max_length is None or isinstance(min_length, bool) or isinstance(max_length, bool) \
+            or int(min_length) != min_length or int(max_length) != max_length:
+        raise ValueError(f"min_length and max_length must be integers, got {min_length!r} and {max_length!r}")
+    min_length, max_length = int(min_length), int(max_length)
+    if not 1 <= min_length <= max_length <= GC_MAX_LENGTH:
+        raise ValueError(f"need 1 <= min_length <= max_length <= {GC_MAX_LENGTH}, got {min_length} and {max_length}")
+    return (max_length - min_length + 1, max_length + 1)
+
+
+def _gc_out(shape, out, dev):
+    t = torch()
+    if out is None:
+        return t.zeros(shape, dtype=t.int64, device=dev)
+    if out.dtype != t.int64 or tuple(out.shape) != shape or not out.is_contiguous():
+        raise ValueError(f"out must be a contiguous int64 tensor of shape {shape}")
+    return out
+
+
+def _gc_regions(reg_start, reg_stop):
+    s = np.asarray(reg_start, dtype=np.int64).reshape(-1)
+    e = np.asarray(reg_stop, dtype=np.int64).reshape(-1)
+    if s.shape != e.shape:
+        raise ValueError("reg_start and reg_stop must have the same length")
+    return s, e
+
+
+def gc_observed(frags: ContigFragments, ref: PackedContig, reg_start, reg_stop, min_length, max_length,
+                quality_threshold=30, out=None):
+    """Fragment counts by (length, G+C bases) of one contig (``ftk_gc_observed_u64``).
+
+    A fragment ``[s, e)`` with ``mapq >= quality_threshold`` and ``min_length <= L <= max_length`` adds 1 at
+    ``[L - min_length, g]`` (g = C/G bases of ``[s, e)``) when its midpoint ``(s + e) // 2`` lies in one of the regions
+    (sorted, disjoint, clipped to ``[0, ref.length]``), ``0 <= s``, ``e <= ref.length`` and no base of it is N.
+    Returns the device int64 matrix of shape ``(max_length - min_length + 1, max_length + 1)``; ``out`` (such a
+    matrix) is accumulated into."""
+    shape = gc_check(min_length, max_length)
+    out = _gc_out(shape, out, frags.device)
+    s, e = _gc_regions(reg_start, reg_stop)
+    n = s.size
+    if n == 0:
+        return out
+    regs = IntervalSet(s, e, frags.device)
+    fs, fe, mq = frags.ptrs()
+    check(lib().ftk_gc_observed_u64(
+        fs, fe, mq, frags.n, frags.max_len, ref.seq.data_ptr(), ref.nmask.data_ptr(), ref.length,
+        regs.start.data_ptr(), regs.stop.data_ptr(), n, int(min_length), int(max_length), int(quality_threshold),
+        _splits_for(n, frags.n), regs.scratch.data_ptr(), out.data_ptr(), _stream_ptr(frags.device)),
+        "ftk_gc_observed_u64")
+    return out
+
+
+def _gc_tile_for(max_length: int) -> int:
+    """Midpoints per ``gc_expected_kernel`` CTA: long enough that the flush of its ``32 x (max_length + 1)`` bins is
+    small next to its ``32 x tile`` placements, short enough that two CTAs of lengths <= 500 share an SM."""
+    return 8192
+
+
+def gc_tiles(reg_start, reg_stop, tile: int):
+    """The regions cut into consecutive midpoint tiles of at most ``tile`` positions: ``(lo, hi)`` int64 arrays."""
+    s, e = _gc_regions(reg_start, reg_stop)
+    n = np.maximum(-(-(e - s) // tile), 0)
+    first = np.repeat(s, n)
+    k = np.arange(int(n.sum()), dtype=np.int64) - np.repeat(np.cumsum(n) - n, n)
+    lo = first + k * tile
+    return lo, np.minimum(lo + tile, np.repeat(e, n))
+
+
+def gc_expected(ref: PackedContig, reg_start, reg_stop, min_length, max_length, out=None):
+    """Counts by (length, G+C bases) of every placement of one contig (``ftk_gc_expected_u64``).
+
+    Every ``[p, p + L)`` with ``min_length <= L <= max_length``, ``p >= 0``, ``p + L <= ref.length``, its midpoint
+    ``p + L // 2`` in one of the regions (sorted, disjoint, clipped) and no N base adds 1 at ``[L - min_length, g]``.
+    Returns the device int64 matrix of shape ``(max_length - min_length + 1, max_length + 1)``; ``out`` is
+    accumulated into."""
+    shape = gc_check(min_length, max_length)
+    out = _gc_out(shape, out, ref.device)
+    tile = int(_gc_tile_for(int(max_length)))
+    if not 1 <= tile <= GC_MAX_TILE:
+        raise ValueError(f"the midpoint tile must lie in [1, {GC_MAX_TILE}], got {tile}")
+    lo, hi = gc_tiles(reg_start, reg_stop, tile)
+    if lo.size == 0:
+        return out
+    d_lo, d_hi = _to_device(lo, ref.device, np.int32), _to_device(hi, ref.device, np.int32)
+    check(lib().ftk_gc_expected_u64(
+        ref.seq.data_ptr(), ref.nmask.data_ptr(), ref.length, d_lo.data_ptr(), d_hi.data_ptr(), lo.size, tile,
+        int(min_length), int(max_length), out.data_ptr(), _stream_ptr(ref.device)), "ftk_gc_expected_u64")
     return out
 
 

@@ -107,3 +107,27 @@ def bedgraph_lines(contig: str, start: int, scores: np.ndarray) -> str:
     a = np.char.add(np.char.add(a, "\t"), (pos + 1).astype(str))
     a = np.char.add(np.char.add(a, "\t"), scores.astype(np.int64).astype(str))
     return "\n".join(a.tolist()) + "\n"
+
+
+def check_tsv_output(output_file, what: str) -> None:
+    """``output_file`` must be None, a ``.tsv`` / ``.tsv.gz`` path or '-'; ``what`` names the table in the error."""
+    if isinstance(output_file, str):
+        if not (output_file.endswith(".tsv") or output_file.endswith(".tsv.gz") or output_file == "-"):
+            raise ValueError("output_file can only have suffix .tsv or .tsv.gz, or be '-'.")
+    elif output_file is not None:
+        raise TypeError(f'output_file is unsupported type "{type(output_file)}". output_file should be a string '
+                        f"specifying the path of the file to output {what} to.")
+
+
+def write_text(output_file: str, text: str) -> None:
+    """``text`` to stdout ('-'), a gzip file (``.gz``) or a plain file."""
+    import sys
+    if output_file == "-":
+        sys.stdout.write(text)
+    elif output_file.endswith(".gz"):
+        from ..io.textout import GzipTextWriter
+        with GzipTextWriter(output_file) as out:
+            out.write(text)
+    else:
+        with open(output_file, "w") as out:
+            out.write(text)

@@ -9,15 +9,13 @@ midpoint ``m = (start + stop) // 2`` lies within ``flank`` of ``c``, ``M[L - min
 """
 from __future__ import annotations
 
-import sys
 import time
 from sys import stderr, stdin
 
 import numpy as np
 
 from ..io.fragments import as_table
-from ..io.textout import GzipTextWriter
-from ._common import dist_context, group_by_contig, is_writer, per_fetch
+from ._common import check_tsv_output, dist_context, group_by_contig, is_writer, per_fetch, write_text
 
 __all__ = ["vplot"]
 
@@ -46,33 +44,12 @@ def _read_sites(site_bed):
     return contigs, centers, flips
 
 
-def _check_output_file(output_file):
-    """``output_file`` must be None, a ``.tsv`` / ``.tsv.gz`` path or '-'."""
-    if isinstance(output_file, str):
-        if not (output_file.endswith(".tsv") or output_file.endswith(".tsv.gz") or output_file == "-"):
-            raise ValueError("output_file can only have suffix .tsv or .tsv.gz, or be '-'.")
-    elif output_file is not None:
-        raise TypeError(f'output_file is unsupported type "{type(output_file)}". output_file should be a string '
-                        "specifying the path of the file to output the V-plot to.")
-
-
 def vplot_text(matrix: np.ndarray, flank: int, min_length: int) -> str:
     """Header ``length\\t-flank\\t...\\tflank``, then ``L\\tcount\\t...`` for every length."""
     lines = ["\t".join(["length"] + [str(d) for d in range(-flank, flank + 1)])]
     for j, row in enumerate(matrix.tolist()):
         lines.append("\t".join([str(min_length + j)] + [str(v) for v in row]))
     return "\n".join(lines) + "\n"
-
-
-def _write(output_file, text: str) -> None:
-    if output_file == "-":
-        sys.stdout.write(text)
-    elif output_file.endswith(".tsv.gz"):
-        with GzipTextWriter(output_file) as out:
-            out.write(text)
-    else:
-        with open(output_file, "w") as out:
-            out.write(text)
 
 
 def vplot(input_file, site_bed, output_file=None, flank=1000, min_length=0, max_length=500, quality_threshold=30,
@@ -91,7 +68,7 @@ def vplot(input_file, site_bed, output_file=None, flank=1000, min_length=0, max_
         raise ValueError("input_file and site_bed cannot both read from stdin")
     shape = vplot_check(flank, min_length, max_length)
     flank, min_length, max_length = int(flank), int(min_length), int(max_length)
-    _check_output_file(output_file)
+    check_tsv_output(output_file, "the V-plot")
     contigs, centers, flips = _read_sites(site_bed)
     table = as_table(input_file, reference_file)
     ctx = dist_context()   # torch.distributed initialised: contigs sharded over the ranks, one all-reduce
@@ -124,7 +101,7 @@ def vplot(input_file, site_bed, output_file=None, flank=1000, min_length=0, max_
             output_file = None
     result = np.zeros(shape, np.int64) if acc is None else acc.cpu().numpy().astype(np.int64, copy=False)
     if output_file is not None:
-        _write(output_file, vplot_text(result, flank, min_length))
+        write_text(output_file, vplot_text(result, flank, min_length))
     if verbose:
         stderr.write(f"vplot took {time.time() - start_time} s to complete\n")
     return result

@@ -430,6 +430,38 @@ int ftk_vplot_u64(const int32_t *frag_start_dev, const int32_t *frag_stop_dev, c
                   const uint8_t *site_flip_dev, int64_t n_sites, int32_t flank, int32_t min_len, int32_t max_len,
                   int32_t min_mapq, int32_t splits, int64_t *scratch_dev, uint64_t *out_dev, ftk_stream_t stream);
 
+/* ---------------------------------------------------------------- GC bias
+ * Fragment-level GC model (Benjamini & Speed 2012): fragment counts by (length, G+C bases), observed over the
+ * sample's fragments and expected over every placement a fragment of that length could take.
+ * A placement [p, p + L) of one contig counts when p >= 0, p + L <= contig_len, its midpoint p + L / 2 lies in
+ * a region [reg_start[k], reg_stop[k]) and none of its bases is N; its G/C count g is the number of C or G
+ * bases in it.  Each counting placement adds
+ *   out[(L - min_len) * (max_len + 1) + g] += 1
+ *   ftk_gc_observed_u64: one placement per fragment with mapq >= min_mapq and min_len <= L <= max_len,
+ *                        L = stop - start (the midpoint is (start + stop) / 2);
+ *   ftk_gc_expected_u64: one placement per (p, L) with min_len <= L <= max_len.
+ * seq_words_dev / nmask_words_dev: the contig packed as synth.pack_twobit does (2 bits per base, A0 C1 G2 T3,
+ * N bit mask, two spare words of padding; seq_words_dev 8-byte aligned).  1 <= min_len <= max_len <=
+ * FTK_GC_MAX_LENGTH, contig_len <= INT32_MAX.  out_dev: uint64[(max_len - min_len + 1) * (max_len + 1)],
+ * ACCUMULATED (the caller zeroes it).
+ * Observed: regions sorted, disjoint and clipped to [0, contig_len]; each region's candidate range is split
+ * into `splits` slices, one warp each; scratch_dev: int64[2 * n_reg]; max_frag_len = max(stop - start) over
+ * the contig.  n_reg == 0 or n_frag == 0 returns 0 without a launch.
+ * Expected: a table of midpoint tiles [tile_lo[t], tile_hi[t]), each inside one region, disjoint, at most
+ * tile_cap <= FTK_GC_MAX_TILE midpoints long; one CTA per (tile, 32 consecutive lengths).  n_tiles == 0
+ * returns 0 without a launch. */
+#define FTK_GC_MAX_LENGTH 1024
+#define FTK_GC_MAX_TILE 16384
+int ftk_gc_observed_u64(const int32_t *frag_start_dev, const int32_t *frag_stop_dev, const uint8_t *frag_mapq_dev,
+                        int64_t n_frag, int32_t max_frag_len, const uint32_t *seq_words_dev,
+                        const uint32_t *nmask_words_dev, int64_t contig_len, const int32_t *reg_start_dev,
+                        const int32_t *reg_stop_dev, int64_t n_reg, int32_t min_len, int32_t max_len,
+                        int32_t min_mapq, int32_t splits, int64_t *scratch_dev, uint64_t *out_dev,
+                        ftk_stream_t stream);
+int ftk_gc_expected_u64(const uint32_t *seq_words_dev, const uint32_t *nmask_words_dev, int64_t contig_len,
+                        const int32_t *tile_lo_dev, const int32_t *tile_hi_dev, int64_t n_tiles, int32_t tile_cap,
+                        int32_t min_len, int32_t max_len, uint64_t *out_dev, ftk_stream_t stream);
+
 /* ------------------------------------------------- fragment file decode (host)
  * Multi-threaded decode of a BGZF / gzip fragment file into per-contig columns; replaces the
  * per-interval pysam.TabixFile.fetch text stream of io/alignment.py:270-302 (5-column FinaleDB

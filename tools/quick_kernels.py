@@ -1,5 +1,6 @@
 """Kernel timing helper (python tools/quick_kernels.py [motif] [bp] [adjust] [delfi] [hist] [cleavage] [depth] [depth-mid]
-[vplot] [vplot-dense]):
+[vplot] [vplot-dense]
+[gc-obs] [gc-exp]):
 CUDA-event time of the secondary kernels at chr1 scale (80 M fragments drawn on the GPU), median of 7 calls after 3
 warm-ups (the call: planning and uploads included).  Every op except adjust also prints an order-sensitive checksum
 of its output (compare two builds with it) and each kernel's own device time (torch.profiler, a separate run)."""
@@ -63,7 +64,7 @@ def op(name, fn, nbytes, result=lambda o: o):
     kernels(fn)
 
 
-if what & {"motif", "bp", "delfi"}:
+if what & {"motif", "bp", "delfi", "gc-obs", "gc-exp"}:
     codes, nm = synth_twobit(CLEN, 0)
     ref = D.PackedContig.from_codes(codes, nm, device=dev)
     ws = np.arange(0, CLEN, 1_000_000, dtype=np.int64); we = np.minimum(ws + 1_000_000, CLEN)
@@ -106,6 +107,19 @@ for name, step in (("vplot", 5000), ("vplot-dense", 500)):
         print(f"{name}: {vc.size} sites, {cand} candidates, {events} events", flush=True)
         op(name, lambda: D.vplot_sites(fr, vc, vf, 1000, 0, 600, 30), 9 * cand)
         print(f"  {events / timed.ms / 1e6:.2f} G events/s over the call", flush=True)
+# GC bias: one whole-contig region, lengths 50..500, q 30
+if "gc-obs" in what:
+    o = D.gc_observed(fr, ref, [0], [CLEN], 50, 500, 30)
+    reach = min(fr.max_len, 500) >> 1
+    cand = int(torch.searchsorted(st, torch.tensor([CLEN], dtype=torch.int32, device=dev)).item()) - \
+        int(torch.searchsorted(st, torch.tensor([-reach], dtype=torch.int32, device=dev)).item())
+    print(f"gc-obs: {cand} candidates, {int(o.sum())} counted", flush=True)
+    op("gc-obs", lambda: D.gc_observed(fr, ref, [0], [CLEN], 50, 500, 30), 9 * cand)
+    print(f"  {cand / timed.ms / 1e6:.2f} G candidates/s over the call", flush=True)
+if "gc-exp" in what:
+    pairs = sum(max(CLEN - L + 1, 0) for L in range(50, 501))   # (m, L) pairs the kernel walks
+    op("gc-exp", lambda: D.gc_expected(ref, [0], [CLEN], 50, 500), 0)
+    print(f"  {pairs} (m, L) pairs, {pairs / timed.ms / 1e9:.3f} T pairs/s over the call", flush=True)
 if "adjust" in what:
     plan = D.WpsPlan(tiles[:-1], tiles[1:], CLEN, 180, dev)
     wps = plan.run(fr)
