@@ -20,6 +20,9 @@ _EXPORTS = {
     "cleavage_profile": ("frag", "cleavage_profile"), "multi_cleavage_profile": ("frag", "multi_cleavage_profile"),
     "coverage_profile": ("frag", "coverage_profile"), "multi_coverage_profile": ("frag", "multi_coverage_profile"),
     "vplot": ("frag", "vplot"), "gc_bias": ("frag", "gc_bias"), "GCBias": ("frag", "GCBias"),
+    "read_gc_bias": ("frag", "read_gc_bias"), "gc_corrected_coverage": ("frag", "gc_corrected_coverage"),
+    "gc_corrected_profile": ("frag", "gc_corrected_profile"), "GCCoverageResult": ("frag", "GCCoverageResult"),
+    "GCSiteProfile": ("frag", "GCSiteProfile"),
     "end_motifs": ("frag", "end_motifs"), "region_end_motifs": ("frag", "region_end_motifs"),
     "interval_end_motifs": ("frag", "interval_end_motifs"),
     "EndMotifFreqs": ("frag", "EndMotifFreqs"), "EndMotifsIntervals": ("frag", "EndMotifsIntervals"),

@@ -5,8 +5,8 @@ Table-driven Click group.  For every in-scope subcommand the flag spellings, par
 (cli/commands/__init__.py:87-640); dispatch filters the parameters by the target's signature like
 cli/_dispatch.py:96-118 and expands ``--strand`` into both_strands / negative_strand
 (cli/_dispatch.py:25-36).  Out-of-scope subcommands (delfi, breakpoint motifs, filter-file, agg-bw,
-gap-bed) are not registered.  ``EXTRA_COMMANDS``, ``SITE_COMMANDS`` and ``BIAS_COMMANDS`` hold the subcommands this package adds
-(coverage-profile, vplot, gc-bias).
+gap-bed) are not registered.  ``EXTRA_COMMANDS``, ``SITE_COMMANDS``, ``BIAS_COMMANDS`` and ``CORRECTION_COMMANDS`` hold the
+subcommands this package adds (coverage-profile, vplot, gc-bias, gc-corrected-coverage / gc-corrected-profile).
 """
 from __future__ import annotations
 
@@ -205,6 +205,32 @@ BIAS_COMMANDS = {
         _mapq(30), _THREADS, _VERBOSE]),
 }
 
+# subcommands that apply the GC model, in their own table for the same reason
+_GC_MODEL = [
+    _opt("--gc-bias", "gc_bias", metavar="TSV", default=None,
+         help="GC model: a gc-bias table (default: fit one on INPUT first)."),
+    _opt("--gc-regions", "gc_regions", metavar="BED", default=None,
+         help="Regions to fit the GC model over (default: every contig the input and the reference share)."),
+    _opt("--min-length", "min_length", metavar="BP", default=None, type=int,
+         help="Minimum fragment length (default: the model's; 50 when fitting)."),
+    _opt("--max-length", "max_length", metavar="BP", default=None, type=int,
+         help="Maximum fragment length (default: the model's; 500 when fitting)."),
+]
+CORRECTION_COMMANDS = {
+    "gc-corrected-coverage": ("finaletoolkit_b200.frag", "gc_corrected_coverage",
+                              "Plain and GC-corrected fragment-midpoint counts over BED intervals.", [
+        _INPUT, _arg("refseq_file", metavar="REFERENCE"), _arg("interval_file", metavar="REGIONS"), _REF,
+        _out("TSV (or .tsv.gz) of plain and GC-corrected counts per interval."), *_GC_MODEL,
+        _mapq(30), _THREADS, _VERBOSE]),
+    "gc-corrected-profile": ("finaletoolkit_b200.frag", "gc_corrected_profile",
+                             "Plain and GC-corrected fragment-midpoint profiles summed over BED sites.", [
+        _INPUT, _arg("refseq_file", metavar="REFERENCE"), _arg("site_bed", metavar="SITES"), _REF,
+        _out("TSV (or .tsv.gz) of plain and GC-corrected counts by midpoint offset."),
+        _opt("--flank", "flank", metavar="BP", default=1000, show_default=True, type=int,
+             help="Largest midpoint offset from a site centre."),
+        *_GC_MODEL, _mapq(30), _THREADS, _VERBOSE]),
+}
+
 
 def run(module: str, func: str, params: dict):
     """Import the target lazily, translate --strand, keep only the kwargs it accepts, call it."""
@@ -233,7 +259,8 @@ def main_cli():
     """finaletoolkit_b200: the B200-native hot path of FinaleToolkit."""
 
 
-for _name, (_module, _func, _help, _spec) in {**COMMANDS, **EXTRA_COMMANDS, **SITE_COMMANDS, **BIAS_COMMANDS}.items():
+for _name, (_module, _func, _help, _spec) in {**COMMANDS, **EXTRA_COMMANDS, **SITE_COMMANDS, **BIAS_COMMANDS,
+                                              **CORRECTION_COMMANDS}.items():
     main_cli.add_command(_make(_name, _module, _func, _help, _spec))
 
 

@@ -14,7 +14,7 @@ from ._lib import FTK_NONE, FtkLibraryError, check, lib
 
 __all__ = ["ContigFragments", "WpsPlan", "AdjustPlan", "IntervalSet", "PackedContig", "interval_hist", "frag_lengths",
            "end_motif_hist", "delfi_windows", "blacklist_in_windows", "agg_signal", "require_cuda", "none_to_ftk", "policy_code",
-           "vplot_sites", "gc_observed", "gc_expected"]
+           "vplot_sites", "gc_observed", "gc_expected", "gc_weighted_intervals", "gc_weighted_sites"]
 
 _torch = None
 
@@ -405,6 +405,20 @@ def vplot_check(flank, min_length, max_length):
     return shape
 
 
+def _site_windows(c: np.ndarray, site_flip, flank: int, dev):
+    """The windows ``[c - flank, c + flank + 1)`` of site centres ``c`` (int64, non-empty) as an ``IntervalSet``, and
+    the flip flags as a device uint8 column."""
+    lim = 2 ** 31 - 1
+    if int(c.min()) - flank < -lim or int(c.max()) > lim:
+        raise ValueError("site centres must lie within the int32 coordinate range")
+    # centre = window start + flank; a window that ends past 2**31 - 1 has no upper bound (None), since a stop
+    # clipped to 2**31 - 1 would drop a fragment starting there
+    hi = c + flank + 1
+    sites = IntervalSet(c - flank, hi if int(hi.max()) <= lim else [None if v > lim else v for v in hi.tolist()], dev)
+    flip = _to_device(np.asarray(site_flip, dtype=bool).reshape(-1).astype(np.uint8), dev, np.uint8)
+    return sites, flip
+
+
 def vplot_sites(frags: ContigFragments, site_center, site_flip, flank, min_length, max_length, quality_threshold=30,
                 out=None):
     """Fragment-length x midpoint-offset counts summed over the sites of one contig (``ftk_vplot_u64``).
@@ -425,14 +439,7 @@ def vplot_sites(frags: ContigFragments, site_center, site_flip, flank, min_lengt
     if n == 0:
         return out
     flank = int(flank)
-    lim = 2 ** 31 - 1
-    if int(c.min()) - flank < -lim or int(c.max()) > lim:
-        raise ValueError("site centres must lie within the int32 coordinate range")
-    # centre = window start + flank; a window that ends past 2**31 - 1 has no upper bound (None), since a stop
-    # clipped to 2**31 - 1 would drop a fragment starting there
-    hi = c + flank + 1
-    sites = IntervalSet(c - flank, hi if int(hi.max()) <= lim else [None if v > lim else v for v in hi.tolist()], dev)
-    flip = _to_device(np.asarray(site_flip, dtype=bool).reshape(-1).astype(np.uint8), dev, np.uint8)
+    sites, flip = _site_windows(c, site_flip, flank, dev)
     fs, fe, mq = frags.ptrs()
     check(lib().ftk_vplot_u64(
         fs, fe, mq, frags.n, frags.max_len, sites.start.data_ptr(), sites.stop.data_ptr(), flip.data_ptr(), n,
@@ -535,6 +542,91 @@ def gc_expected(ref: PackedContig, reg_start, reg_stop, min_length, max_length, 
         ref.seq.data_ptr(), ref.nmask.data_ptr(), ref.length, d_lo.data_ptr(), d_hi.data_ptr(), lo.size, tile,
         int(min_length), int(max_length), out.data_ptr(), _stream_ptr(ref.device)), "ftk_gc_expected_u64")
     return out
+
+
+def gc_weights_to_device(weights, shape, dev):
+    """The weight table as a contiguous float64 device tensor; ValueError unless it has ``shape`` and every entry is
+    finite and ``>= 0``."""
+    t = torch()
+    w = weights if t.is_tensor(weights) else t.from_numpy(np.asarray(weights, dtype=np.float64))
+    if tuple(w.shape) != tuple(shape):
+        raise ValueError(f"the weight table must have shape {tuple(shape)}, got {tuple(w.shape)}")
+    w = w.to(dev, t.float64).contiguous()
+    if not bool((t.isfinite(w) & (w >= 0)).all()):
+        raise ValueError("the weight table must hold finite, non-negative values")
+    return w
+
+
+def _gc_weighted_out(n, out, dev):
+    t = torch()
+    if out is None:
+        return t.zeros(n, dtype=t.int64, device=dev), t.zeros(n, dtype=t.float64, device=dev)
+    count, corrected = out
+    for x, dt in ((count, t.int64), (corrected, t.float64)):
+        if x.dtype != dt or tuple(x.shape) != (n,) or not x.is_contiguous():
+            raise ValueError(f"out must be contiguous (int64, float64) tensors of shape ({n},)")
+    return count, corrected
+
+
+def gc_weighted_intervals(frags: ContigFragments, ref: PackedContig, ivl_start, ivl_stop, weights, min_length,
+                          max_length, quality_threshold=30, out=None):
+    """Plain and GC-weighted fragment counts of each interval of one contig (``ftk_gc_weighted_intervals_f64``).
+
+    A fragment ``[s, e)`` with ``mapq >= quality_threshold``, ``min_length <= L <= max_length`` and its midpoint
+    ``(s + e) // 2`` in ``[ivl_start[k], ivl_stop[k])`` (None = unbounded) adds 1 to ``count[k]``, and
+    ``weights[L - min_length, g]`` to ``corrected[k]`` when ``0 <= s``, ``e <= ref.length`` and no base of it is N
+    (g = its C/G bases).  ``weights``: float64 of the GC-bias matrices' shape, finite and non-negative.  Returns
+    device tensors ``(count int64[n], corrected float64[n])``; ``out`` (such a pair) is accumulated into.  The
+    corrected sums are bit-identical between runs with the same slice count."""
+    shape = gc_check(min_length, max_length)
+    dev = frags.device
+    n = len(ivl_start)
+    if len(ivl_stop) != n:
+        raise ValueError("ivl_start and ivl_stop must have the same length")
+    w = gc_weights_to_device(weights, shape, dev)
+    count, corrected = _gc_weighted_out(n, out, dev)
+    if n == 0:
+        return count, corrected
+    ivl = IntervalSet(ivl_start, ivl_stop, dev)
+    splits = _splits_for(n, frags.n)
+    scratch = torch().empty(2 * n + 2 * n * splits, dtype=torch().int64, device=dev)
+    fs, fe, mq = frags.ptrs()
+    check(lib().ftk_gc_weighted_intervals_f64(
+        fs, fe, mq, frags.n, frags.max_len, ref.seq.data_ptr(), ref.nmask.data_ptr(), ref.length,
+        ivl.start.data_ptr(), ivl.stop.data_ptr(), n, int(min_length), int(max_length), int(quality_threshold), splits,
+        scratch.data_ptr(), w.data_ptr(), count.data_ptr(), corrected.data_ptr(), _stream_ptr(dev)),
+        "ftk_gc_weighted_intervals_f64")
+    return count, corrected
+
+
+def gc_weighted_sites(frags: ContigFragments, ref: PackedContig, site_center, site_flip, flank, weights, min_length,
+                      max_length, quality_threshold=30, out=None):
+    """Plain and GC-weighted fragment-midpoint profiles around the sites of one contig (``ftk_gc_weighted_sites_f64``).
+
+    Site k is centred on ``site_center[k]`` and mirrored when ``site_flip[k]`` is true; a fragment selected as in
+    ``gc_weighted_intervals`` whose midpoint lies within ``flank`` of the centre adds 1 to ``count[offset + flank]``
+    and its weight to ``corrected[offset + flank]``.  Returns device tensors ``(count int64[2 * flank + 1],
+    corrected float64[2 * flank + 1])`` summed over the sites; ``out`` is accumulated into.  The corrected sums are
+    fp64 atomics, so their last bits may vary between runs."""
+    shape = gc_check(min_length, max_length)
+    flank = int(flank)
+    if not 0 <= flank <= VPLOT_MAX_FLANK:
+        raise ValueError(f"flank must lie in [0, {VPLOT_MAX_FLANK}], got {flank}")
+    dev = frags.device
+    w = gc_weights_to_device(weights, shape, dev)
+    count, corrected = _gc_weighted_out(2 * flank + 1, out, dev)
+    c = np.asarray(site_center, dtype=np.int64).reshape(-1)
+    n = c.size
+    if n == 0:
+        return count, corrected
+    sites, flip = _site_windows(c, site_flip, flank, dev)
+    fs, fe, mq = frags.ptrs()
+    check(lib().ftk_gc_weighted_sites_f64(
+        fs, fe, mq, frags.n, frags.max_len, ref.seq.data_ptr(), ref.nmask.data_ptr(), ref.length,
+        sites.start.data_ptr(), sites.stop.data_ptr(), flip.data_ptr(), n, flank, int(min_length), int(max_length),
+        int(quality_threshold), _splits_for(n, frags.n), sites.scratch.data_ptr(), w.data_ptr(), count.data_ptr(),
+        corrected.data_ptr(), _stream_ptr(dev)), "ftk_gc_weighted_sites_f64")
+    return count, corrected
 
 
 def frag_lengths(frags: ContigFragments, start=None, stop=None, intersect_policy="midpoint",

@@ -21,7 +21,7 @@ from ..io.fragments import as_table
 from ..io.reference import open_reference
 from ._common import check_tsv_output, dist_context, is_writer, per_fetch, write_text
 
-__all__ = ["gc_bias", "GCBias"]
+__all__ = ["gc_bias", "GCBias", "read_gc_bias"]
 
 
 @dataclass
@@ -46,13 +46,56 @@ def gc_ratio(O: np.ndarray, E: np.ndarray) -> np.ndarray:
 
 def gc_text(res: GCBias) -> str:
     """Header ``length\\tgc\\tobserved\\texpected\\tratio``, then one row per ``(L, g)`` with ``g <= L``."""
-    lines = ["length\tgc\tobserved\texpected\tratio"]
+    lines = [_HEADER]
     O, E, R = res.observed.tolist(), res.expected.tolist(), res.ratio.tolist()
     for i in range(len(O)):
         L = res.min_length + i
         o, e, r = O[i], E[i], R[i]
         lines.extend(f"{L}\t{g}\t{o[g]}\t{e[g]}\t{r[g]!r}" for g in range(L + 1))
     return "\n".join(lines) + "\n"
+
+
+_HEADER = "length\tgc\tobserved\texpected\tratio"
+
+
+def read_gc_bias(path) -> GCBias:
+    """The ``GCBias`` a ``gc_bias`` / ``gc-bias`` table (``.tsv`` or ``.tsv.gz``) holds; the inverse of ``gc_text``.
+
+    Ratios are read back as written (``repr`` floats and ``nan`` round-trip exactly).  ValueError for a table that
+    is not one row per ``(L, g)``, ``0 <= g <= L``, for consecutive lengths within ``[1, 1024]``."""
+    import gzip
+    import os
+    path = os.fspath(path)
+    with (gzip.open(path, "rt") if path.endswith(".gz") else open(path)) as fh:
+        lines = fh.read().splitlines()
+    if not lines or lines[0] != _HEADER:
+        raise ValueError(f"{path}: not a GC-bias table (expected the header {_HEADER!r})")
+    rows = []
+    for k, line in enumerate(lines[1:], 2):
+        f = line.split("\t")
+        try:
+            if len(f) != 5:
+                raise ValueError
+            rows.append((int(f[0]), int(f[1]), int(f[2]), int(f[3]), float(f[4])))
+        except ValueError:
+            raise ValueError(f"{path}:{k}: malformed GC-bias row {line!r}") from None
+    if not rows:
+        raise ValueError(f"{path}: the GC-bias table has no rows")
+    lo, hi = rows[0][0], rows[-1][0]
+    if not 1 <= lo <= hi <= 1024 or len(rows) != sum(L + 1 for L in range(lo, hi + 1)):
+        raise ValueError(f"{path}: the GC-bias table does not hold every (length, gc) of lengths {lo}..{hi}")
+    keys = np.array([(r[0], r[1]) for r in rows], np.int64)
+    want = np.array([(L, g) for L in range(lo, hi + 1) for g in range(L + 1)], np.int64)
+    if not np.array_equal(keys, want):
+        raise ValueError(f"{path}: the GC-bias rows are not one per (length, gc) in order")
+    shape = (hi - lo + 1, hi + 1)
+    O, E = np.zeros(shape, np.int64), np.zeros(shape, np.int64)
+    R = np.full(shape, np.nan)
+    i, g = keys[:, 0] - lo, keys[:, 1]
+    O[i, g] = [r[2] for r in rows]
+    E[i, g] = [r[3] for r in rows]
+    R[i, g] = [r[4] for r in rows]
+    return GCBias(O, E, R, lo, hi)
 
 
 def read_regions(interval_file, chrom_len: dict) -> dict:

@@ -462,6 +462,39 @@ int ftk_gc_expected_u64(const uint32_t *seq_words_dev, const uint32_t *nmask_wor
                         const int32_t *tile_lo_dev, const int32_t *tile_hi_dev, int64_t n_tiles, int32_t tile_cap,
                         int32_t min_len, int32_t max_len, uint64_t *out_dev, ftk_stream_t stream);
 
+/* ---------------------------------------------------------------- GC-corrected counts
+ * The GC model applied: weights_dev is a float64 table of the GC-bias matrices' shape, read as
+ * weights[(L - min_len) * (max_len + 1) + g] (typically 1 / ratio, 0 where the ratio is undefined).  A fragment
+ * is selected when mapq >= min_mapq, min_len <= L <= max_len (L = stop - start) and its midpoint
+ * m = (start + stop) / 2 passes the unit's position test.  Every selected fragment adds 1 to a count; it also
+ * adds weights[L - min_len, g] to a corrected sum when start >= 0, stop <= contig_len and none of its bases is N
+ * (the placement rule of ftk_gc_observed_u64; g = its C/G bases).  The reference, lengths and fragments are as
+ * for ftk_gc_observed_u64.  Outputs are ACCUMULATED (the caller zeroes them); each unit's candidate range is split
+ * into `splits` slices, one warp each; n_units == 0 or n_frag == 0 returns 0 without a launch.
+ *   ftk_gc_weighted_intervals_f64: interval k is [ivl_start[k], ivl_stop[k]) (FTK_NONE = unbounded; overlapping and
+ *     unsorted intervals are fine), test ivl_start <= m < ivl_stop; out_count_dev uint64[n_ivl],
+ *     out_corrected_dev fp64[n_ivl].  scratch_dev: int64[2 * n_ivl + 2 * n_ivl * splits] (candidate ranges, then
+ *     one partial count and sum per (interval, slice)).  The partials are reduced in a fixed order, so the result
+ *     is bit-identical run to run for the same `splits`.
+ *   ftk_gc_weighted_sites_f64: the windows of ftk_vplot_u64 ([c - flank, c + flank + 1), flipped when
+ *     site_flip[k] != 0), test |d| <= flank with d = m - c (flipped: c - m); out_count_dev uint64[2 * flank + 1]
+ *     and out_corrected_dev fp64[2 * flank + 1] at d + flank, summed over the sites (fp64 atomics: the order of
+ *     the corrected sums varies between runs).  scratch_dev: int64[2 * n_sites]; flank <= FTK_VPLOT_MAX_FLANK. */
+int ftk_gc_weighted_intervals_f64(const int32_t *frag_start_dev, const int32_t *frag_stop_dev,
+                                  const uint8_t *frag_mapq_dev, int64_t n_frag, int32_t max_frag_len,
+                                  const uint32_t *seq_words_dev, const uint32_t *nmask_words_dev, int64_t contig_len,
+                                  const int32_t *ivl_start_dev, const int32_t *ivl_stop_dev, int64_t n_ivl,
+                                  int32_t min_len, int32_t max_len, int32_t min_mapq, int32_t splits,
+                                  int64_t *scratch_dev, const double *weights_dev, uint64_t *out_count_dev,
+                                  double *out_corrected_dev, ftk_stream_t stream);
+int ftk_gc_weighted_sites_f64(const int32_t *frag_start_dev, const int32_t *frag_stop_dev,
+                              const uint8_t *frag_mapq_dev, int64_t n_frag, int32_t max_frag_len,
+                              const uint32_t *seq_words_dev, const uint32_t *nmask_words_dev, int64_t contig_len,
+                              const int32_t *win_lo_dev, const int32_t *win_hi_dev, const uint8_t *site_flip_dev,
+                              int64_t n_sites, int32_t flank, int32_t min_len, int32_t max_len, int32_t min_mapq,
+                              int32_t splits, int64_t *scratch_dev, const double *weights_dev,
+                              uint64_t *out_count_dev, double *out_corrected_dev, ftk_stream_t stream);
+
 /* ------------------------------------------------- fragment file decode (host)
  * Multi-threaded decode of a BGZF / gzip fragment file into per-contig columns; replaces the
  * per-interval pysam.TabixFile.fetch text stream of io/alignment.py:270-302 (5-column FinaleDB

@@ -1,6 +1,6 @@
 """Kernel timing helper (python tools/quick_kernels.py [motif] [bp] [adjust] [delfi] [hist] [cleavage] [depth] [depth-mid]
 [vplot] [vplot-dense]
-[gc-obs] [gc-exp]):
+[gc-obs] [gc-exp] [gc-cov] [gc-site]):
 CUDA-event time of the secondary kernels at chr1 scale (80 M fragments drawn on the GPU), median of 7 calls after 3
 warm-ups (the call: planning and uploads included).  Every op except adjust also prints an order-sensitive checksum
 of its output (compare two builds with it) and each kernel's own device time (torch.profiler, a separate run)."""
@@ -64,7 +64,7 @@ def op(name, fn, nbytes, result=lambda o: o):
     kernels(fn)
 
 
-if what & {"motif", "bp", "delfi", "gc-obs", "gc-exp"}:
+if what & {"motif", "bp", "delfi", "gc-obs", "gc-exp", "gc-cov", "gc-site"}:
     codes, nm = synth_twobit(CLEN, 0)
     ref = D.PackedContig.from_codes(codes, nm, device=dev)
     ws = np.arange(0, CLEN, 1_000_000, dtype=np.int64); we = np.minimum(ws + 1_000_000, CLEN)
@@ -116,6 +116,34 @@ if "gc-obs" in what:
     print(f"gc-obs: {cand} candidates, {int(o.sum())} counted", flush=True)
     op("gc-obs", lambda: D.gc_observed(fr, ref, [0], [CLEN], 50, 500, 30), 9 * cand)
     print(f"  {cand / timed.ms / 1e6:.2f} G candidates/s over the call", flush=True)
+
+
+def candidates(lo, hi, reach):
+    """Sum over units of the candidate range [lower_bound(lo - reach), lower_bound(hi)) of the start column."""
+    a = torch.searchsorted(st, torch.tensor(lo - reach, dtype=torch.int32, device=dev))
+    b = torch.searchsorted(st, torch.tensor(hi, dtype=torch.int32, device=dev))
+    return int((b - a).sum())
+
+
+# GC-corrected counts: lengths 50..500, q 30, seeded weights (their values do not change the work)
+if what & {"gc-cov", "gc-site"}:
+    W = torch.rand((451, 501), generator=g, device=dev, dtype=torch.float64)
+if "gc-cov" in what:
+    cand = candidates(tiles[:-1], tiles[1:], min(fr.max_len, 500) >> 1)
+    c, w = D.gc_weighted_intervals(fr, ref, tiles[:-1], tiles[1:], W, 50, 500, 30)
+    print(f"gc-cov: {tiles.size - 1} intervals, {cand} candidates, {int(c.sum())} selected", flush=True)
+    op("gc-cov", lambda: D.gc_weighted_intervals(fr, ref, tiles[:-1], tiles[1:], W, 50, 500, 30), 9 * cand,
+       lambda o: torch.cat([o[0], o[1].view(torch.int64)]))
+    print(f"  {cand / timed.ms / 1e6:.2f} G candidates/s over the call", flush=True)
+if "gc-site" in what:
+    # sites every 5 kb (49 850), strands alternating, flank 1000
+    gc_c = np.arange(2500, CLEN, 5000, dtype=np.int64)
+    gc_f = np.arange(gc_c.size) % 2 == 1
+    cand = candidates(gc_c - 1000, gc_c + 1001, min(fr.max_len, 500) >> 1)
+    c, w = D.gc_weighted_sites(fr, ref, gc_c, gc_f, 1000, W, 50, 500, 30)
+    print(f"gc-site: {gc_c.size} sites, {cand} candidates, {int(c.sum())} events", flush=True)
+    op("gc-site", lambda: D.gc_weighted_sites(fr, ref, gc_c, gc_f, 1000, W, 50, 500, 30), 9 * cand, lambda o: o[0])
+    print(f"  {int(c.sum()) / timed.ms / 1e6:.2f} G events/s over the call", flush=True)
 if "gc-exp" in what:
     pairs = sum(max(CLEN - L + 1, 0) for L in range(50, 501))   # (m, L) pairs the kernel walks
     op("gc-exp", lambda: D.gc_expected(ref, [0], [CLEN], 50, 500), 0)
