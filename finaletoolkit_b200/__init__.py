@@ -22,7 +22,8 @@ _EXPORTS = {
     "vplot": ("frag", "vplot"), "gc_bias": ("frag", "gc_bias"), "GCBias": ("frag", "GCBias"),
     "read_gc_bias": ("frag", "read_gc_bias"), "gc_corrected_coverage": ("frag", "gc_corrected_coverage"),
     "gc_corrected_profile": ("frag", "gc_corrected_profile"), "GCCoverageResult": ("frag", "GCCoverageResult"),
-    "GCSiteProfile": ("frag", "GCSiteProfile"),
+    "GCSiteProfile": ("frag", "GCSiteProfile"), "wps_spectrum": ("frag", "wps_spectrum"),
+    "WpsSpectrum": ("frag", "WpsSpectrum"),
     "end_motifs": ("frag", "end_motifs"), "region_end_motifs": ("frag", "region_end_motifs"),
     "interval_end_motifs": ("frag", "interval_end_motifs"),
     "EndMotifFreqs": ("frag", "EndMotifFreqs"), "EndMotifsIntervals": ("frag", "EndMotifsIntervals"),

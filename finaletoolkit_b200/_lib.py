@@ -82,6 +82,8 @@ SYMBOLS = {
                                               c_int32, c_int32, c_int32, _P, _P, _P, _P, _P]),
     "ftk_gc_weighted_sites_f64": (c_int, [_P, _P, _P, c_int64, c_int32, _P, _P, c_int64, _P, _P, _P, c_int64, c_int32,
                                           c_int32, c_int32, c_int32, c_int32, _P, _P, _P, _P, _P]),
+    "ftk_spectrum_i32_f64": (c_int, [_P, _P, c_int64, c_int32, c_int32, _P, _P]),
+    "ftk_spectrum_f64_f64": (c_int, [_P, _P, c_int64, c_int32, c_int32, _P, _P]),
     "ftk_fragfile_open": (c_void_p, [c_char_p, c_int32, _i32p]),
     "ftk_fragfile_open_slice": (c_void_p, [c_char_p, c_int64, c_int32, c_int64, c_int32, c_int32, c_int32, _i32p]),
     "ftk_bamfile_open": (c_void_p, [c_char_p, c_int32, _i32p]),

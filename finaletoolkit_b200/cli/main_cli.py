@@ -5,8 +5,9 @@ Table-driven Click group.  For every in-scope subcommand the flag spellings, par
 (cli/commands/__init__.py:87-640); dispatch filters the parameters by the target's signature like
 cli/_dispatch.py:96-118 and expands ``--strand`` into both_strands / negative_strand
 (cli/_dispatch.py:25-36).  Out-of-scope subcommands (delfi, breakpoint motifs, filter-file, agg-bw,
-gap-bed) are not registered.  ``EXTRA_COMMANDS``, ``SITE_COMMANDS``, ``BIAS_COMMANDS`` and ``CORRECTION_COMMANDS`` hold the
-subcommands this package adds (coverage-profile, vplot, gc-bias, gc-corrected-coverage / gc-corrected-profile).
+gap-bed) are not registered.  ``EXTRA_COMMANDS``, ``SITE_COMMANDS``, ``BIAS_COMMANDS``, ``CORRECTION_COMMANDS`` and
+``SPECTRUM_COMMANDS`` hold the subcommands this package adds (coverage-profile, vplot, gc-bias,
+gc-corrected-coverage / gc-corrected-profile, wps-spectrum).
 """
 from __future__ import annotations
 
@@ -231,6 +232,29 @@ CORRECTION_COMMANDS = {
         *_GC_MODEL, _mapq(30), _THREADS, _VERBOSE]),
 }
 
+# subcommands that transform WPS further, in their own table for the same reason
+SPECTRUM_COMMANDS = {
+    "wps-spectrum": ("finaletoolkit_b200.frag", "wps_spectrum",
+                     "Periodograms of the (adjusted) WPS of BED windows at integer periods (nucleosome repeat).", [
+        _INPUT, _arg("site_bed", metavar="REGIONS"), _REF,
+        _opt("--chrom-sizes", "chrom_sizes", metavar="CHROM_SIZES", help="A .chrom.sizes file."),
+        _out("TSV (or .tsv.gz) of one periodogram per BED row."),
+        _opt("--min-period", "min_period", metavar="BP", default=120, show_default=True, type=int,
+             help="Shortest period (at least 2)."),
+        _opt("--max-period", "max_period", metavar="BP", default=280, show_default=True, type=int,
+             help="Longest period (at most 1024)."),
+        _opt("--adjust/--no-adjust", "adjust", default=True,
+             help="Median-filter + Savitzky-Golay adjust the WPS first. On by default."),
+        _opt("-m", "--median-window-size", "median_window_size", metavar="BP", default=1000, show_default=True,
+             type=int),
+        _opt("--savgol/--no-savgol", "savgol", default=True, help="Apply Savitzky-Golay filtering. On by default."),
+        _opt("--savgol-window-size", "savgol_window_size", metavar="BP", default=21, show_default=True, type=int),
+        _opt("--savgol-poly-deg", "savgol_poly_deg", metavar="DEG", default=2, show_default=True, type=int),
+        _opt("-W", "--window-size", "window_size", metavar="BP", default=120, show_default=True, type=int,
+             help="WPS sliding-window size."),
+        _minlen(120), _maxlen(180), _mapq(30), _THREADS, _VERBOSE]),
+}
+
 
 def run(module: str, func: str, params: dict):
     """Import the target lazily, translate --strand, keep only the kwargs it accepts, call it."""
@@ -260,7 +284,7 @@ def main_cli():
 
 
 for _name, (_module, _func, _help, _spec) in {**COMMANDS, **EXTRA_COMMANDS, **SITE_COMMANDS, **BIAS_COMMANDS,
-                                              **CORRECTION_COMMANDS}.items():
+                                              **CORRECTION_COMMANDS, **SPECTRUM_COMMANDS}.items():
     main_cli.add_command(_make(_name, _module, _func, _help, _spec))
 
 

@@ -14,7 +14,8 @@ from ._lib import FTK_NONE, FtkLibraryError, check, lib
 
 __all__ = ["ContigFragments", "WpsPlan", "AdjustPlan", "IntervalSet", "PackedContig", "interval_hist", "frag_lengths",
            "end_motif_hist", "delfi_windows", "blacklist_in_windows", "agg_signal", "require_cuda", "none_to_ftk", "policy_code",
-           "vplot_sites", "gc_observed", "gc_expected", "gc_weighted_intervals", "gc_weighted_sites"]
+           "vplot_sites", "gc_observed", "gc_expected", "gc_weighted_intervals", "gc_weighted_sites",
+           "spectrum_segments"]
 
 _torch = None
 
@@ -629,6 +630,51 @@ def gc_weighted_sites(frags: ContigFragments, ref: PackedContig, site_center, si
     return count, corrected
 
 
+SPECTRUM_MAX_PERIOD = 1024   # FTK_SPECTRUM_MAX_PERIOD
+
+
+def spectrum_check(min_period, max_period) -> int:
+    """ValueError unless ``2 <= min_period <= max_period <= 1024`` (integers); returns the number of periods."""
+    if min_period is None or max_period is None or isinstance(min_period, bool) or isinstance(max_period, bool) \
+            or int(min_period) != min_period or int(max_period) != max_period:
+        raise ValueError(f"min_period and max_period must be integers, got {min_period!r} and {max_period!r}")
+    if not 2 <= int(min_period) <= int(max_period) <= SPECTRUM_MAX_PERIOD:
+        raise ValueError(f"need 2 <= min_period <= max_period <= {SPECTRUM_MAX_PERIOD}, got {min_period} and "
+                         f"{max_period}")
+    return int(max_period) - int(min_period) + 1
+
+
+def spectrum_segments(x, offsets, min_period=120, max_period=280, out=None):
+    """Periodogram of every segment at the integer periods ``min_period .. max_period`` (``ftk_spectrum_*_f64``).
+
+    ``x``: an int32 or float64 CUDA tensor holding the segments back to back; segment s is
+    ``x[offsets[s]:offsets[s + 1]]`` (host int64 offsets, non-decreasing).  With N values of mean mu,
+    ``I(P) = |sum_n (x[n] - mu) exp(-2 pi i (n mod P) / P)|^2 / N``; an empty segment gives a row of NaN.  Returns the
+    device float64 matrix ``[n_seg, n_periods]`` (``out``, such a matrix, is written).  Bit-identical from run to
+    run; a segment's row does not depend on the other segments."""
+    t = torch()
+    n_p = spectrum_check(min_period, max_period)
+    if not (t.is_tensor(x) and x.is_cuda and x.dtype in (t.int32, t.float64)):
+        raise ValueError("x must be an int32 or float64 CUDA tensor")
+    dev = x.device
+    off = np.asarray(offsets, dtype=np.int64).reshape(-1)
+    if off.size == 0 or off[0] < 0 or (np.diff(off) < 0).any() or off[-1] > x.numel():
+        raise ValueError("offsets must be non-decreasing, start at >= 0 and end within x")
+    shape = (off.size - 1, n_p)
+    if out is None:
+        out = t.empty(shape, dtype=t.float64, device=dev)
+    elif out.dtype != t.float64 or tuple(out.shape) != shape or not out.is_contiguous() or out.device != dev:
+        raise ValueError(f"out must be a contiguous float64 tensor of shape {shape} on {dev}")
+    if shape[0] == 0:
+        return out
+    xd = x.contiguous() if x.numel() else t.zeros(1, dtype=x.dtype, device=dev)
+    d_off = _to_device(off, dev, np.int64)
+    name = "ftk_spectrum_i32_f64" if xd.dtype == t.int32 else "ftk_spectrum_f64_f64"
+    check(getattr(lib(), name)(xd.data_ptr(), d_off.data_ptr(), shape[0], int(min_period), int(max_period),
+                               out.data_ptr(), _stream_ptr(dev)), name)
+    return out
+
+
 def frag_lengths(frags: ContigFragments, start=None, stop=None, intersect_policy="midpoint",
                  min_length=0, max_length=1000000000, quality_threshold=30):
     """int32 lengths of the stream of one region, in stream order (device tensor)."""
@@ -894,9 +940,7 @@ class AdjustPlan:
                              "(frag/_adjust_wps.py:43 slices w//2 from both ends)")
         n_out = seg_lengths - w
         if skip_short:
-            # segments the reference's driver would skip (frag/_adjust_wps.py:125-129 raises per interval,
-            # :145-153 skips it) stay in the sample layout but produce no output
-            n_out = np.where((n_out >= (savgol_window_size if savgol else 0)) & (n_out > 0), n_out, 0)
+            n_out = self.output_lengths(seg_lengths, w, savgol, savgol_window_size)
         else:
             if (seg_lengths < w).any():
                 bad = int(seg_lengths[seg_lengths < w][0])
@@ -926,6 +970,14 @@ class AdjustPlan:
             if s_cap <= 65535 - 64 and _rank_smem(a_cap, s_cap) <= _RANK_SMEM_MAX:
                 self.rank = (tuple(_to_device(a, dev, np.int32) for a in (tile_seg, tile_t0, tile_n)),
                              len(tile_seg), a_cap, s_cap)
+
+    @staticmethod
+    def output_lengths(seg_lengths, median_window_size=1000, savgol=True, savgol_window_size=21):
+        """Outputs per segment with ``skip_short``: ``n - median_window_size``, or 0 for a segment too short for the
+        filters (the reference's driver skips it: frag/_adjust_wps.py:125-129 raises per interval, :145-153 skips
+        it); such segments stay in the sample layout."""
+        n_out = np.asarray(seg_lengths, dtype=np.int64) - int(median_window_size)
+        return np.where((n_out >= (int(savgol_window_size) if savgol else 0)) & (n_out > 0), n_out, 0)
 
     def run_rank(self, xd, shift_ptr=0, out=None):
         """Launch the fused median + Savitzky-Golay kernel; returns ``(out, tile_flag)`` (no sync:

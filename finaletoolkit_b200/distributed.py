@@ -18,7 +18,7 @@ from .sharding import DistContext, genome_length_dict, lpt_pack, reduce_length_d
 
 __all__ = ["owned_contigs", "genome_total_coverage", "genome_length_distribution", "genome_end_motif_counts",
            "genome_delfi_windows", "genome_bin_counts", "table_shard", "ContigWps", "GenomeShard", "multi_wps_genome", "adjust_wps_genome", "tile_genome",
-           "gather_to_writer"]
+           "wps_spectrum_genome", "gather_to_writer"]
 
 
 def owned_contigs(table, ctx: DistContext | None = None):
@@ -551,6 +551,27 @@ def adjust_wps_genome(results: dict, **adjust):
         if aplan.n_total:
             res.adjusted, _ = adjust_segments(res.wps, None, plan=aplan, **adjust)
     return results
+
+
+def wps_spectrum_genome(results: dict, min_period=120, max_period=280) -> dict:
+    """Periodograms (``device.spectrum_segments``) of every interval of ``multi_wps_genome`` results, from the
+    adjusted series when the results hold them (``adjust=`` or ``adjust_wps_genome``), otherwise from the raw WPS -
+    all in HBM.  Returns {contig: float64[n_intervals, n_periods] device tensor}; an interval with an empty series
+    (too short for the filters) gives a row of NaN."""
+    from .device import spectrum_check, spectrum_segments, torch
+    spectrum_check(min_period, max_period)
+    out = {}
+    for c, res in results.items():
+        if res.adj_offsets is None:
+            x, off = res.wps, res.offsets
+        else:
+            if res.adjusted is None and res.adj_offsets[-1] > 0:
+                raise ValueError(f"the results of {c} hold no adjusted series (keep_adjusted=False)")
+            x = res.adjusted if res.adjusted is not None else torch().zeros(0, dtype=torch().float64,
+                                                                              device=res.wps.device)
+            off = res.adj_offsets
+        out[c] = spectrum_segments(x, off, min_period, max_period)
+    return out
 
 
 def gather_to_writer(obj, ctx: DistContext | None = None):

@@ -495,6 +495,21 @@ int ftk_gc_weighted_sites_f64(const int32_t *frag_start_dev, const int32_t *frag
                               int32_t splits, int64_t *scratch_dev, const double *weights_dev,
                               uint64_t *out_count_dev, double *out_corrected_dev, ftk_stream_t stream);
 
+/* ---------------------------------------------------------------- periodicity spectra
+ * Segment s is x_dev[offsets_dev[s] .. offsets_dev[s + 1]) (int64 offsets, segments back to back; N values,
+ * mean mu).  For every integer period P in [min_period, max_period]:
+ *   X(P) = sum_{n<N} (x[n] - mu) * exp(-2 pi i (n mod P) / P),  out_dev[s * n_periods + P - min_period] = |X(P)|^2 / N
+ * (n_periods = max_period - min_period + 1; fp64).  The per-residue folds sum_{n = r mod P} x[n] are exact int64
+ * sums for int32 input and fp64 sums for fp64 input.  An empty segment gives a row of NaN.  No atomics: the output
+ * is bit-identical from run to run, and a segment's row does not depend on the other segments of the call.
+ * 2 <= min_period <= max_period <= FTK_SPECTRUM_MAX_PERIOD; n_seg == 0 returns 0 without a launch (replaces the
+ * bigWig export + host FFT of Snyder et al. 2016's gene-body WPS periodograms). */
+#define FTK_SPECTRUM_MAX_PERIOD 1024
+int ftk_spectrum_i32_f64(const int32_t *x_dev, const int64_t *offsets_dev, int64_t n_seg, int32_t min_period,
+                         int32_t max_period, double *out_dev, ftk_stream_t stream);
+int ftk_spectrum_f64_f64(const double *x_dev, const int64_t *offsets_dev, int64_t n_seg, int32_t min_period,
+                         int32_t max_period, double *out_dev, ftk_stream_t stream);
+
 /* ------------------------------------------------- fragment file decode (host)
  * Multi-threaded decode of a BGZF / gzip fragment file into per-contig columns; replaces the
  * per-interval pysam.TabixFile.fetch text stream of io/alignment.py:270-302 (5-column FinaleDB

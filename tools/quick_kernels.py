@@ -1,6 +1,6 @@
 """Kernel timing helper (python tools/quick_kernels.py [motif] [bp] [adjust] [delfi] [hist] [cleavage] [depth] [depth-mid]
 [vplot] [vplot-dense]
-[gc-obs] [gc-exp] [gc-cov] [gc-site]):
+[gc-obs] [gc-exp] [gc-cov] [gc-site] [spectrum]):
 CUDA-event time of the secondary kernels at chr1 scale (80 M fragments drawn on the GPU), median of 7 calls after 3
 warm-ups (the call: planning and uploads included).  Every op except adjust also prints an order-sensitive checksum
 of its output (compare two builds with it) and each kernel's own device time (torch.profiler, a separate run)."""
@@ -157,3 +157,14 @@ if "adjust" in what:
     print("  checksum", float(out.sum()), "flags", int(ap.run_rank(wps, 0, out)[1].sum()))
     ap0 = D.AdjustPlan(np.diff(plan.offsets), 1000, False, 21, 2, dev, skip_short=True)
     timed("adjust_wps median only", lambda: ap0.run_rank(wps, 0, out), 4 * plan.n_positions + 8 * ap.n_total)
+if "spectrum" in what:
+    # 20 000 windows x 10 kb (the gene-body workload), periods 120..280; the values do not change the work
+    n_win, win, lo_p, hi_p = 20_000, 10_000, 120, 280
+    xi = torch.randint(-300, 300, (n_win * win,), generator=g, device=dev, dtype=torch.int32)
+    off = np.arange(0, n_win * win + 1, win, dtype=np.int64)
+    adds = n_win * win * (hi_p - lo_p + 1)            # fold additions: one per (position, period)
+    for name, xs in (("spectrum-i32", xi), ("spectrum-f64", xi.to(torch.float64))):
+        op(name, lambda: D.spectrum_segments(xs, off, lo_p, hi_p), xs.numel() * xs.element_size())
+        print(f"  {adds / timed.ms / 1e9:.1f} T fold additions/s; shared-memory loads "
+              f"{adds * xs.element_size() / timed.ms / 1e9:.1f} TB/s", flush=True)
+    del xi
