@@ -926,13 +926,17 @@ extern "C" int ftk_adjust_wps_f64(const float *x, const int64_t *seg_off, const 
     const long long *so = reinterpret_cast<const long long *>(seg_off);
     const long long *oo = reinterpret_cast<const long long *>(seg_out_off);
     const long long *ro = reinterpret_cast<const long long *>(seg_run_off);
+    int dev = 0;
+    rc = ftk::current_device(&dev);
+    if (rc != FTK_OK) return rc;
+    // the dynamic shared-memory limit belongs to (kernel, device): raise it on every device this thread launches on
 #define FTK_ADJ_LAUNCH(M, S)                                                                                   \
     do {                                                                                                       \
-        static thread_local bool attr_set = false;                                                             \
-        if (!attr_set) {                                                                                       \
+        static thread_local bool smem_opted_in[ftk::kMaxDevices] = {};                                         \
+        if (!smem_opted_in[dev]) {                                                                             \
             FTK_CUDA_TRY(cudaFuncSetAttribute(adjust_hist_kernel<M, S>,                                         \
                                               cudaFuncAttributeMaxDynamicSharedMemorySize, smem));             \
-            attr_set = true;                                                                                   \
+            smem_opted_in[dev] = true;                                                                         \
         }                                                                                                      \
         adjust_hist_kernel<M, S><<<grid, kAdjThreads, smem, stream>>>(x, so, oo, ro, seg_shift, n_seg, n_runs, \
                                                                       P, adj_out, fallback);                   \

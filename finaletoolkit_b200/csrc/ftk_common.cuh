@@ -24,6 +24,15 @@ int cuda_fail(cudaError_t e, const char *what);
         if (_e != cudaSuccess) return ::ftk::cuda_fail(_e, name); \
     } while (0)
 
+// Per-device tables (SM counts, shared-memory opt-ins) hold this many devices.
+constexpr int kMaxDevices = 64;
+
+// The calling thread's current CUDA device: the one a launch runs on.
+inline int current_device(int *dev) {
+    FTK_CUDA_TRY(cudaGetDevice(dev));
+    return (*dev < 0 || *dev >= kMaxDevices) ? FTK_E_RANGE : FTK_OK;
+}
+
 // Streaming (read-once) global loads: keep them out of L1.
 __device__ __forceinline__ int ld_stream(const int32_t *p) {
     int v;

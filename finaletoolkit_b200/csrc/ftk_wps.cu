@@ -581,14 +581,14 @@ extern "C" int ftk_wps_tile_ranges(const int32_t *frag_start, int64_t n_frag,
                               wps_left_reach(window_size, max_len), scratch, static_cast<cudaStream_t>(stream_));
 }
 
-static int device_sm_count(int *sm) {
-    static thread_local int sm_count[64] = {0};
-    int dev = 0;
-    FTK_CUDA_TRY(cudaGetDevice(&dev));
-    if (dev < 0 || dev >= 64) return FTK_E_RANGE;
-    if (!sm_count[dev])
-        FTK_CUDA_TRY(cudaDeviceGetAttribute(&sm_count[dev], cudaDevAttrMultiProcessorCount, dev));
-    *sm = sm_count[dev];
+// SM count of the current device, which is returned in *dev
+static int device_sm_count(int *sm, int *dev) {
+    static thread_local int sm_count[ftk::kMaxDevices] = {0};
+    int rc = ftk::current_device(dev);
+    if (rc != FTK_OK) return rc;
+    if (!sm_count[*dev])
+        FTK_CUDA_TRY(cudaDeviceGetAttribute(&sm_count[*dev], cudaDevAttrMultiProcessorCount, *dev));
+    *sm = sm_count[*dev];
     return FTK_OK;
 }
 
@@ -609,15 +609,16 @@ static int launch_stream(const WpsLaunch &a, OutT *out) {
     static_assert(sizeof(Smem) <= 227 * 1024, "a CTA may own at most 227 KB of shared memory on sm_100a");
     static_assert(ctas_per_sm * (sizeof(Smem) + 1024) <= 228 * 1024,
                   "the resident CTAs, with the 1 KB reserved for each, must fit the SM's 228 KB");
-    int sm = 0;
-    int rc = device_sm_count(&sm);
+    int sm = 0, dev = 0;
+    int rc = device_sm_count(&sm, &dev);
     if (rc != FTK_OK) return rc;
-    static thread_local bool attr_set = false;
+    // the dynamic shared-memory limit belongs to (kernel, device): raise it on every device this thread launches on
+    static thread_local bool smem_opted_in[kMaxDevices] = {};
     const int smem = (int)sizeof(Smem);
-    if (!attr_set) {
+    if (!smem_opted_in[dev]) {
         FTK_CUDA_TRY(cudaFuncSetAttribute(wps_stream_kernel<ODD, OutT, GROUPS, FUSE>,
                                           cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-        attr_set = true;
+        smem_opted_in[dev] = true;
     }
     // persistent CTAs; a plain-WPS CTA is launched only when there are two tiles for its two groups
     int64_t grid = (int64_t)sm * ctas_per_sm;

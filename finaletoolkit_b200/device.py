@@ -29,15 +29,17 @@ def torch():
 
 
 def require_cuda(device=None):
-    """Return a CUDA ``torch.device`` or raise: there is no CPU compute path."""
+    """Return a CUDA ``torch.device`` with its index (the current device when ``device`` names none) or raise:
+    there is no CPU compute path."""
     t = torch()
     if not t.cuda.is_available():
         raise FtkLibraryError(
             "finaletoolkit_b200 needs a CUDA device (sm_100a); no CPU fallback exists")
     lib()  # fail loudly if the extension is missing
-    if device is None:
+    dev = t.device("cuda") if device is None else t.device(device)
+    if dev.type == "cuda" and dev.index is None:
         return t.device("cuda", t.cuda.current_device())
-    return t.device(device)
+    return dev
 
 
 def none_to_ftk(v) -> int:
@@ -46,6 +48,23 @@ def none_to_ftk(v) -> int:
 
 def _stream_ptr(device) -> int:
     return int(torch().cuda.current_stream(device).cuda_stream)
+
+
+def _launch(dev, name: str, *args) -> None:
+    """``libftk_b200.<name>(*args, stream)`` on device ``dev`` and its current stream, result checked.
+
+    The library launches on the calling thread's current CUDA device, so the call runs with ``dev`` made current:
+    tensors on a device other than the current one are worked on where they live.  Nothing changes when ``dev`` is
+    already current (e.g. inside a CUDA graph capture)."""
+    with torch().cuda.device(dev):
+        check(getattr(lib(), name)(*args, _stream_ptr(dev)), name)
+
+
+def _same_device(dev, *objs) -> None:
+    """ValueError unless every object (tensor, ``ContigFragments``, ``PackedContig``, plan) lives on ``dev``."""
+    for o in objs:
+        if o.device != dev:
+            raise ValueError(f"inputs on {o.device} and {dev}: every input of a call must be on one device")
 
 
 def _np_ptr(a, ctype):
@@ -212,10 +231,9 @@ class WpsPlan:
     def ranges(self, frags: ContigFragments, window_size=120):
         """Only the per-tile fragment-range prepass (lets a caller time the main kernel alone)."""
         if self.n_tiles:
-            check(lib().ftk_wps_tile_ranges(frags.start.data_ptr(), frags.n, self.tile_p0.data_ptr(),
-                                            self.tile_len.data_ptr(), self.n_tiles, int(window_size),
-                                            self.max_length, self.scratch.data_ptr(), _stream_ptr(self.device)),
-                  "ftk_wps_tile_ranges")
+            _launch(self.device, "ftk_wps_tile_ranges", frags.start.data_ptr(), frags.n, self.tile_p0.data_ptr(),
+                    self.tile_len.data_ptr(), self.n_tiles, int(window_size), self.max_length,
+                    self.scratch.data_ptr())
 
     def run(self, frags: ContigFragments, window_size=120, min_length=120, max_length=180,
             quality_threshold=30, out=None, ranges_ready=False):
@@ -223,6 +241,7 @@ class WpsPlan:
         t = torch()
         if int(max_length) != self.max_length:
             raise ValueError("plan was built for a different max_length")
+        _same_device(self.device, frags)
         if out is None:
             out = t.empty(self.n_positions, dtype=t.int32, device=self.device)
         elif out.dtype != t.int32 or out.numel() < self.n_positions or not out.is_contiguous():
@@ -230,13 +249,12 @@ class WpsPlan:
         if self.n_tiles == 0:
             return out
         fs, fe, mq = frags.ptrs()
-        check(lib().ftk_wps_tiles_i32(
+        _launch(self.device, "ftk_wps_tiles_i32",
             fs, fe, mq, frags.n,
             self.tile_p0.data_ptr(), self.tile_len.data_ptr(), self.tile_mid_lo.data_ptr(),
             self.tile_mid_hi.data_ptr(), self.tile_out_off.data_ptr(), self.n_tiles,
             int(window_size), none_to_ftk(min_length), int(max_length), int(quality_threshold),
-            int(bool(ranges_ready)), self.scratch.data_ptr(), out.data_ptr(), _stream_ptr(self.device)),
-            "ftk_wps_tiles_i32")
+            int(bool(ranges_ready)), self.scratch.data_ptr(), out.data_ptr())
         return out
 
     def ranges_fused(self, frags: ContigFragments, window_size=120, cov_max_length=None, zero_counts=None,
@@ -244,12 +262,11 @@ class WpsPlan:
         """Only the fragment-range prepass of ``run_fused`` (lets a caller time the main kernel alone).
         ``zero_counts`` / ``zero_hist``: int64 accumulators the prepass clears on the way (no extra launch)."""
         if self.n_tiles:
-            check(lib().ftk_wps_cov_tile_ranges(
+            _launch(self.device, "ftk_wps_cov_tile_ranges",
                 frags.start.data_ptr(), frags.n, self.tile_p0.data_ptr(), self.tile_len.data_ptr(), self.n_tiles,
                 int(window_size), self.max_length, none_to_ftk(cov_max_length), frags.max_len, self.scratch.data_ptr(),
                 0 if zero_counts is None else zero_counts.data_ptr(), 0 if zero_counts is None else zero_counts.numel(),
-                0 if zero_hist is None else zero_hist.data_ptr(), 0 if zero_hist is None else zero_hist.numel(),
-                _stream_ptr(self.device)), "ftk_wps_cov_tile_ranges")
+                0 if zero_hist is None else zero_hist.data_ptr(), 0 if zero_hist is None else zero_hist.numel())
         else:
             for z in (zero_counts, zero_hist):
                 if z is not None:
@@ -267,6 +284,7 @@ class WpsPlan:
         t = torch()
         if int(max_length) != self.max_length:
             raise ValueError("plan was built for a different max_length")
+        _same_device(self.device, frags)
         if out is None:
             out = t.empty(self.n_positions, dtype=t.int32, device=self.device)
         kind = {t.int32: 0, t.int16: 1, t.int8: 2}.get(out.dtype)
@@ -284,15 +302,14 @@ class WpsPlan:
         if self.n_tiles == 0:
             return out, counts[: self.n_intervals], hist
         fs, fe, mq = frags.ptrs()
-        check(lib().ftk_wps_cov_tiles(
+        _launch(self.device, "ftk_wps_cov_tiles",
             fs, fe, mq, frags.n, frags.max_len,
             self.tile_p0.data_ptr(), self.tile_len.data_ptr(), self.tile_mid_lo.data_ptr(),
             self.tile_mid_hi.data_ptr(), self.tile_out_off.data_ptr(), self.tile_ivl.data_ptr(), self.n_tiles,
             int(window_size), none_to_ftk(min_length), int(max_length), int(quality_threshold),
             none_to_ftk(cov_min_length), none_to_ftk(cov_max_length), int(cov_quality_threshold), int(n_bins),
             int(bool(ranges_ready)), self.scratch.data_ptr(), kind, out.data_ptr(), 0 if overflow is None else overflow.data_ptr(),
-            counts.data_ptr(), 0 if hist is None else hist.data_ptr(), _stream_ptr(self.device)),
-            "ftk_wps_cov_tiles")
+            counts.data_ptr(), 0 if hist is None else hist.data_ptr())
         return out, counts[: self.n_intervals], hist
 
 
@@ -377,12 +394,12 @@ def interval_hist(frags: ContigFragments, ivl_start=None, ivl_stop=None, interse
     if n_ivl == 0:
         return counts[:rows], hist, first
     fs, fe, mq = frags.ptrs()
-    check(lib().ftk_interval_hist_u64(
+    _launch(dev, "ftk_interval_hist_u64",
         fs, fe, mq, frags.n, frags.max_len, ivl_set.start.data_ptr(), ivl_set.stop.data_ptr(), n_ivl,
         policy_code(intersect_policy), none_to_ftk(min_length), none_to_ftk(max_length),
         int(quality_threshold), int(n_bins), pool_mode, _splits_for(n_ivl, frags.n),
         ivl_set.scratch.data_ptr(), counts.data_ptr(), 0 if hist is None else hist.data_ptr(),
-        0 if first is None else first.data_ptr(), _stream_ptr(dev)), "ftk_interval_hist_u64")
+        0 if first is None else first.data_ptr())
     return counts[:rows], hist, first
 
 
@@ -442,10 +459,10 @@ def vplot_sites(frags: ContigFragments, site_center, site_flip, flank, min_lengt
     flank = int(flank)
     sites, flip = _site_windows(c, site_flip, flank, dev)
     fs, fe, mq = frags.ptrs()
-    check(lib().ftk_vplot_u64(
+    _launch(dev, "ftk_vplot_u64",
         fs, fe, mq, frags.n, frags.max_len, sites.start.data_ptr(), sites.stop.data_ptr(), flip.data_ptr(), n,
         flank, int(min_length), int(max_length), int(quality_threshold), _splits_for(n, frags.n),
-        sites.scratch.data_ptr(), out.data_ptr(), _stream_ptr(dev)), "ftk_vplot_u64")
+        sites.scratch.data_ptr(), out.data_ptr())
     return out
 
 
@@ -492,6 +509,7 @@ def gc_observed(frags: ContigFragments, ref: PackedContig, reg_start, reg_stop, 
     Returns the device int64 matrix of shape ``(max_length - min_length + 1, max_length + 1)``; ``out`` (such a
     matrix) is accumulated into."""
     shape = gc_check(min_length, max_length)
+    _same_device(frags.device, ref)
     out = _gc_out(shape, out, frags.device)
     s, e = _gc_regions(reg_start, reg_stop)
     n = s.size
@@ -499,11 +517,10 @@ def gc_observed(frags: ContigFragments, ref: PackedContig, reg_start, reg_stop, 
         return out
     regs = IntervalSet(s, e, frags.device)
     fs, fe, mq = frags.ptrs()
-    check(lib().ftk_gc_observed_u64(
+    _launch(frags.device, "ftk_gc_observed_u64",
         fs, fe, mq, frags.n, frags.max_len, ref.seq.data_ptr(), ref.nmask.data_ptr(), ref.length,
         regs.start.data_ptr(), regs.stop.data_ptr(), n, int(min_length), int(max_length), int(quality_threshold),
-        _splits_for(n, frags.n), regs.scratch.data_ptr(), out.data_ptr(), _stream_ptr(frags.device)),
-        "ftk_gc_observed_u64")
+        _splits_for(n, frags.n), regs.scratch.data_ptr(), out.data_ptr())
     return out
 
 
@@ -539,9 +556,9 @@ def gc_expected(ref: PackedContig, reg_start, reg_stop, min_length, max_length, 
     if lo.size == 0:
         return out
     d_lo, d_hi = _to_device(lo, ref.device, np.int32), _to_device(hi, ref.device, np.int32)
-    check(lib().ftk_gc_expected_u64(
+    _launch(ref.device, "ftk_gc_expected_u64",
         ref.seq.data_ptr(), ref.nmask.data_ptr(), ref.length, d_lo.data_ptr(), d_hi.data_ptr(), lo.size, tile,
-        int(min_length), int(max_length), out.data_ptr(), _stream_ptr(ref.device)), "ftk_gc_expected_u64")
+        int(min_length), int(max_length), out.data_ptr())
     return out
 
 
@@ -581,6 +598,7 @@ def gc_weighted_intervals(frags: ContigFragments, ref: PackedContig, ivl_start, 
     corrected sums are bit-identical between runs with the same slice count."""
     shape = gc_check(min_length, max_length)
     dev = frags.device
+    _same_device(dev, ref)
     n = len(ivl_start)
     if len(ivl_stop) != n:
         raise ValueError("ivl_start and ivl_stop must have the same length")
@@ -592,11 +610,10 @@ def gc_weighted_intervals(frags: ContigFragments, ref: PackedContig, ivl_start, 
     splits = _splits_for(n, frags.n)
     scratch = torch().empty(2 * n + 2 * n * splits, dtype=torch().int64, device=dev)
     fs, fe, mq = frags.ptrs()
-    check(lib().ftk_gc_weighted_intervals_f64(
+    _launch(dev, "ftk_gc_weighted_intervals_f64",
         fs, fe, mq, frags.n, frags.max_len, ref.seq.data_ptr(), ref.nmask.data_ptr(), ref.length,
         ivl.start.data_ptr(), ivl.stop.data_ptr(), n, int(min_length), int(max_length), int(quality_threshold), splits,
-        scratch.data_ptr(), w.data_ptr(), count.data_ptr(), corrected.data_ptr(), _stream_ptr(dev)),
-        "ftk_gc_weighted_intervals_f64")
+        scratch.data_ptr(), w.data_ptr(), count.data_ptr(), corrected.data_ptr())
     return count, corrected
 
 
@@ -614,6 +631,7 @@ def gc_weighted_sites(frags: ContigFragments, ref: PackedContig, site_center, si
     if not 0 <= flank <= VPLOT_MAX_FLANK:
         raise ValueError(f"flank must lie in [0, {VPLOT_MAX_FLANK}], got {flank}")
     dev = frags.device
+    _same_device(dev, ref)
     w = gc_weights_to_device(weights, shape, dev)
     count, corrected = _gc_weighted_out(2 * flank + 1, out, dev)
     c = np.asarray(site_center, dtype=np.int64).reshape(-1)
@@ -622,11 +640,11 @@ def gc_weighted_sites(frags: ContigFragments, ref: PackedContig, site_center, si
         return count, corrected
     sites, flip = _site_windows(c, site_flip, flank, dev)
     fs, fe, mq = frags.ptrs()
-    check(lib().ftk_gc_weighted_sites_f64(
+    _launch(dev, "ftk_gc_weighted_sites_f64",
         fs, fe, mq, frags.n, frags.max_len, ref.seq.data_ptr(), ref.nmask.data_ptr(), ref.length,
         sites.start.data_ptr(), sites.stop.data_ptr(), flip.data_ptr(), n, flank, int(min_length), int(max_length),
         int(quality_threshold), _splits_for(n, frags.n), sites.scratch.data_ptr(), w.data_ptr(), count.data_ptr(),
-        corrected.data_ptr(), _stream_ptr(dev)), "ftk_gc_weighted_sites_f64")
+        corrected.data_ptr())
     return count, corrected
 
 
@@ -670,8 +688,7 @@ def spectrum_segments(x, offsets, min_period=120, max_period=280, out=None):
     xd = x.contiguous() if x.numel() else t.zeros(1, dtype=x.dtype, device=dev)
     d_off = _to_device(off, dev, np.int64)
     name = "ftk_spectrum_i32_f64" if xd.dtype == t.int32 else "ftk_spectrum_f64_f64"
-    check(getattr(lib(), name)(xd.data_ptr(), d_off.data_ptr(), shape[0], int(min_period), int(max_period),
-                               out.data_ptr(), _stream_ptr(dev)), name)
+    _launch(dev, name, xd.data_ptr(), d_off.data_ptr(), shape[0], int(min_period), int(max_period), out.data_ptr())
     return out
 
 
@@ -685,11 +702,11 @@ def frag_lengths(frags: ContigFragments, start=None, stop=None, intersect_policy
     out = t.empty(max(frags.n, 1), dtype=t.int32, device=dev)
     n_out = t.zeros(1, dtype=t.int64, device=dev)
     fs, fe, mq = frags.ptrs()
-    check(lib().ftk_frag_lengths_i32(
+    _launch(dev, "ftk_frag_lengths_i32",
         fs, fe, mq, frags.n, frags.max_len, none_to_ftk(start), none_to_ftk(stop),
         policy_code(intersect_policy), none_to_ftk(min_length), none_to_ftk(max_length),
         int(quality_threshold), scratch.data_ptr(), scratch.numel(), out.data_ptr(),
-        n_out.data_ptr(), _stream_ptr(dev)), "ftk_frag_lengths_i32")
+        n_out.data_ptr())
     return out[: int(n_out.item())]
 
 
@@ -717,6 +734,7 @@ def end_motif_hist(frags: ContigFragments, ref: PackedContig, ivl_start, ivl_sto
     instead of 5' end motifs; that variant has no error path."""
     t = torch()
     dev = frags.device
+    _same_device(dev, ref)
     n_ivl = len(ivl_start)
     rows = 1 if pooled else n_ivl
     if counts is None:
@@ -731,17 +749,16 @@ def end_motif_hist(frags: ContigFragments, ref: PackedContig, ivl_start, ivl_sto
     # paid once per slice: 16 K fragments amortise it (and the zero + flush of a 4^k-bin histogram)
     splits = _splits_for(n_ivl, frags.n, unit_frags=max(16384, 16 * 4 ** min(int(k), 6)))
     if breakpoint:
-        check(lib().ftk_breakpoint_motif_hist_u64(
+        _launch(dev, "ftk_breakpoint_motif_hist_u64",
             fs, fe, mq, sd, frags.n, frags.max_len, ref.seq.data_ptr(), ref.nmask.data_ptr(), ref.length,
             ivl.start.data_ptr(), ivl.stop.data_ptr(), n_ivl, int(k), int(strand_mode), int(quality_threshold),
-            int(bool(pooled)), splits, ivl.scratch.data_ptr(), counts.data_ptr(),
-            _stream_ptr(dev)), "ftk_breakpoint_motif_hist_u64")
+            int(bool(pooled)), splits, ivl.scratch.data_ptr(), counts.data_ptr())
         return counts[:rows]
-    check(lib().ftk_end_motif_hist_u64(
+    _launch(dev, "ftk_end_motif_hist_u64",
         fs, fe, mq, sd, frags.n, frags.max_len, ref.seq.data_ptr(), ref.nmask.data_ptr(), ref.length,
         ivl.start.data_ptr(), ivl.stop.data_ptr(), n_ivl, int(k), int(strand_mode), int(quality_threshold),
         int(bool(pooled)), splits, ivl.scratch.data_ptr(), counts.data_ptr(),
-        err.data_ptr(), _stream_ptr(dev)), "ftk_end_motif_hist_u64")
+        err.data_ptr())
     if int(err.item()):
         raise RuntimeError(
             "Error querying sequence: reverse k-mer window out of contig bounds. Please verify "
@@ -779,6 +796,7 @@ def delfi_windows(frags: ContigFragments, ref: PackedContig | None, win_start, w
     (start, stop), [telomere (start, stop), ...]) or None (frag/_delfi.py:404-511)."""
     t = torch()
     dev = frags.device
+    _same_device(dev, *([] if ref is None else [ref]))
     n_win = len(win_start)
     counts = t.zeros((max(n_win, 1), 4), dtype=t.int64, device=dev)
     if n_win == 0:
@@ -798,28 +816,28 @@ def delfi_windows(frags: ContigFragments, ref: PackedContig | None, win_start, w
         lim = 2 ** 31 - 1
         g5 = np.array([c0, c1, len(telomeres), max((a for a, _ in telomeres), default=0),
                        min((b for _, b in telomeres), default=0)], dtype=np.int64).clip(-lim, lim).astype(np.int32)
-    check(lib().ftk_delfi_windows_u64(
+    _launch(dev, "ftk_delfi_windows_u64",
         fs, fe, mq, frags.n, frags.max_len, 0 if ref is None else ref.seq.data_ptr(),
         0 if ref is None else ref.nmask.data_ptr(), 0 if ref is None else ref.length,
         win.start.data_ptr(), win.stop.data_ptr(), n_win, *bl, None if g5 is None else _np_ptr(g5, c_int32),
-        int(quality_threshold), _splits_for(n_win, frags.n), win.scratch.data_ptr(), counts.data_ptr(),
-        _stream_ptr(dev)), "ftk_delfi_windows_u64")
+        int(quality_threshold), _splits_for(n_win, frags.n), win.scratch.data_ptr(), counts.data_ptr())
     return counts
 
 
 def agg_signal(rows, strand, trim_lo: int, out_len: int, device=None):
     """Strand-aware fp64 sum of equal-length signal rows (utils/_agg_bw.py:84-123) -> float64[out_len] (device).
 
-    ``rows``: float32 [n_seg, row_len] (numpy or CUDA tensor); ``strand``: int8 per row (+1, -1, 0 = skip)."""
+    ``rows``: float32 [n_seg, row_len] (numpy or CUDA tensor); ``strand``: int8 per row (+1, -1, 0 = skip).
+    ``device`` defaults to the device of a CUDA ``rows``, else the current device."""
     t = torch()
-    dev = require_cuda(device)
+    dev = require_cuda(rows.device if device is None and t.is_tensor(rows) and rows.is_cuda else device)
     x = rows if t.is_tensor(rows) else _to_device(np.ascontiguousarray(rows, np.float32), dev, np.float32)
     x = x.to(dev, t.float32).contiguous()
     sd = _to_device(np.ascontiguousarray(strand, np.int8), dev, np.int8)
     n_seg, row_len = (int(x.shape[0]), int(x.shape[1])) if x.dim() == 2 else (0, 0)
     out = t.zeros(int(out_len), dtype=t.float64, device=dev)
-    check(lib().ftk_agg_signal_f64(x.data_ptr(), n_seg, row_len, int(trim_lo), int(out_len), sd.data_ptr(),
-                                   out.data_ptr(), _stream_ptr(dev)), "ftk_agg_signal_f64")
+    _launch(dev, "ftk_agg_signal_f64", x.data_ptr(), n_seg, row_len, int(trim_lo), int(out_len), sd.data_ptr(),
+            out.data_ptr())
     return out
 
 
@@ -988,12 +1006,12 @@ class AdjustPlan:
             out = t.empty(max(self.n_total, 1), dtype=t.float64, device=self.device)
         flag = t.empty(n_tiles, dtype=t.uint8, device=self.device)
         tb = self.tables
-        check(lib().ftk_adjust_rank_f64(
+        _launch(self.device, "ftk_adjust_rank_f64",
             xd.data_ptr(), 1 if xd.dtype == t.int32 else 0, self.d_seg.data_ptr(), self.d_out.data_ptr(), shift_ptr,
             self.n_seg, d_ts.data_ptr(), d_t0.data_ptr(), d_tn.data_ptr(), n_tiles, self.w, self.sg_w,
             tb[0].data_ptr() if tb else 0, tb[1].data_ptr() if tb else 0, tb[2].data_ptr() if tb else 0,
             *(self.sg_rational if not shift_ptr else (0, 0, 0)),
-            a_cap, s_cap, out.data_ptr(), flag.data_ptr(), _stream_ptr(self.device)), "ftk_adjust_rank_f64")
+            a_cap, s_cap, out.data_ptr(), flag.data_ptr())
         return out, flag
 
 
@@ -1012,18 +1030,21 @@ def adjust_segments(x, seg_lengths, median_window_size=1000, use_mean=False, sav
     one pass, 12 B of HBM traffic per position); tiles it flags (non-integer samples, huge values) and the
     mean path go through the sliding-histogram / generic kernels + the separate Savitzky-Golay kernel.
     ``impl="hist"`` forces that older path (``run_len`` only applies to it).  ``plan``: a prebuilt
-    ``AdjustPlan`` for this layout and these parameters (skips all host-side planning and uploads).
+    ``AdjustPlan`` for this layout and these parameters (skips all host-side planning and uploads), on the device
+    of ``x`` when ``x`` is a CUDA tensor (ValueError otherwise).
     ``defer_check=True`` (median path with a rank plan only): no host synchronisation - returns
     ``(out, out_off, tile_flag)`` and the caller looks at ``tile_flag.any()`` later (and calls again
     with ``impl="hist"`` if it is set).
     """
     t = torch()
-    dev = require_cuda(x.device if t.is_tensor(x) and x.is_cuda else None)
+    on_device = t.is_tensor(x) and x.is_cuda
+    dev = require_cuda(x.device if on_device else None if plan is None else plan.device)
     if plan is None:
         plan = AdjustPlan(seg_lengths, median_window_size, savgol, savgol_window_size, savgol_poly_deg, dev)
+    _same_device(dev, plan)
     w, n_seg, n_out, n_total = plan.w, plan.n_seg, plan.n_out, plan.n_total
     out_off = plan.out_off
-    if t.is_tensor(x) and x.is_cuda and x.dtype == t.int32:
+    if on_device and x.dtype == t.int32:
         xd = x.contiguous()
     else:
         xd = x if t.is_tensor(x) else _to_device(np.asarray(x), dev, np.float32)
@@ -1032,14 +1053,12 @@ def adjust_segments(x, seg_lengths, median_window_size=1000, use_mean=False, sav
     if n_total == 0:
         return out[:0], out_off
     d_seg, d_out = plan.d_seg, plan.d_out
-    L = lib()
-    sp = _stream_ptr(dev)
     shift_ptr = 0
     if subtract_edges:
         xf = xd if xd.dtype == t.float32 else xd.to(t.float32)
         shift = t.empty(n_seg, dtype=t.float64, device=dev)
-        check(L.ftk_adjust_edge_shift_f64(xf.data_ptr(), d_seg.data_ptr(), n_seg, int(edge_size),
-                                          shift.data_ptr(), sp), "ftk_adjust_edge_shift_f64")
+        _launch(dev, "ftk_adjust_edge_shift_f64", xf.data_ptr(), d_seg.data_ptr(), n_seg, int(edge_size),
+                shift.data_ptr())
         shift_ptr = shift.data_ptr()
     sg_w, tables = plan.sg_w, plan.tables
 
@@ -1072,20 +1091,17 @@ def adjust_segments(x, seg_lengths, median_window_size=1000, use_mean=False, sav
     d_run = _to_device(run_off, dev, np.int64)
     adj = t.empty(max(n_total, 1), dtype=t.float64, device=dev) if savgol else out
     fb = t.empty(n_runs, dtype=t.uint8, device=dev)
-    check(L.ftk_adjust_wps_f64(xd.data_ptr(), d_seg.data_ptr(), d_out.data_ptr(), d_run.data_ptr(), shift_ptr,
-                               n_seg, n_runs, int(w), int(bool(use_mean)), int(run_len), adj.data_ptr(),
-                               fb.data_ptr(), sp), "ftk_adjust_wps_f64")
+    _launch(dev, "ftk_adjust_wps_f64", xd.data_ptr(), d_seg.data_ptr(), d_out.data_ptr(), d_run.data_ptr(), shift_ptr,
+            n_seg, n_runs, int(w), int(bool(use_mean)), int(run_len), adj.data_ptr(), fb.data_ptr())
     flagged = t.nonzero(fb).flatten().to(t.int64)   # plumbing: compact the flagged run ids
     if flagged.numel():
         scratch = t.empty(flagged.numel() * w, dtype=t.float32, device=dev)
-        check(L.ftk_adjust_wps_generic_f64(xd.data_ptr(), d_seg.data_ptr(), d_out.data_ptr(), d_run.data_ptr(),
-                                           shift_ptr, n_seg, flagged.data_ptr(), flagged.numel(), int(w),
-                                           int(bool(use_mean)), int(run_len), adj.data_ptr(),
-                                           scratch.data_ptr(), sp), "ftk_adjust_wps_generic_f64")
+        _launch(dev, "ftk_adjust_wps_generic_f64", xd.data_ptr(), d_seg.data_ptr(), d_out.data_ptr(),
+                d_run.data_ptr(), shift_ptr, n_seg, flagged.data_ptr(), flagged.numel(), int(w), int(bool(use_mean)),
+                int(run_len), adj.data_ptr(), scratch.data_ptr())
     if savgol:
-        check(L.ftk_savgol_f64(adj.data_ptr(), d_out.data_ptr(), n_seg, n_total, sg_w,
-                               tables[0].data_ptr(), tables[1].data_ptr(), tables[2].data_ptr(), out.data_ptr(), sp),
-              "ftk_savgol_f64")
+        _launch(dev, "ftk_savgol_f64", adj.data_ptr(), d_out.data_ptr(), n_seg, n_total, sg_w, tables[0].data_ptr(),
+                tables[1].data_ptr(), tables[2].data_ptr(), out.data_ptr())
     if defer_check:
         return out[:n_total], out_off, None
     return out[:n_total], out_off
@@ -1103,11 +1119,11 @@ def cleavage_intervals(frags: ContigFragments, ivl_start, ivl_stop, chrom_size, 
     if plan.n_tiles:
         fs, fe, mq = frags.ptrs()
         sd = 0 if frags.strand is None else frags.strand.data_ptr()
-        check(lib().ftk_cleavage_tiles_f64(
+        _launch(frags.device, "ftk_cleavage_tiles_f64",
             fs, fe, mq, sd, frags.n, frags.max_len, plan.tile_p0.data_ptr(), plan.tile_len.data_ptr(),
             plan.tile_mid_lo.data_ptr(), plan.tile_mid_hi.data_ptr(), plan.tile_out_off.data_ptr(), plan.n_tiles,
             none_to_ftk(min_length), none_to_ftk(max_length), int(quality_threshold),
-            plan.scratch.data_ptr(), out.data_ptr(), _stream_ptr(frags.device)), "ftk_cleavage_tiles_f64")
+            plan.scratch.data_ptr(), out.data_ptr())
     return out[: plan.n_positions], plan.offsets
 
 
@@ -1124,9 +1140,9 @@ def depth_intervals(frags: ContigFragments, ivl_start, ivl_stop, chrom_size, min
     out = t.empty(max(plan.n_positions, 1), dtype=t.int32, device=frags.device)
     if plan.n_tiles:
         fs, fe, mq = frags.ptrs()
-        check(lib().ftk_depth_tiles_i32(
+        _launch(frags.device, "ftk_depth_tiles_i32",
             fs, fe, mq, frags.n, frags.max_len, plan.tile_p0.data_ptr(), plan.tile_len.data_ptr(),
             plan.tile_mid_lo.data_ptr(), plan.tile_mid_hi.data_ptr(), plan.tile_out_off.data_ptr(), plan.n_tiles,
             none_to_ftk(min_length), none_to_ftk(max_length), int(quality_threshold), int(bool(midpoint)),
-            plan.scratch.data_ptr(), out.data_ptr(), _stream_ptr(frags.device)), "ftk_depth_tiles_i32")
+            plan.scratch.data_ptr(), out.data_ptr())
     return out[: plan.n_positions], plan.offsets

@@ -13,7 +13,7 @@ from ctypes import POINTER, c_int32, c_uint8, c_uint32
 import numpy as np
 
 from ._lib import check, lib
-from .device import ContigFragments, _stream_ptr, require_cuda, torch
+from .device import ContigFragments, _launch, require_cuda, torch
 
 __all__ = ["PackedFragments", "PACK_BLOCK"]
 
@@ -94,11 +94,11 @@ class PackedFragments:
     def unpack_into(self, d_words, d_anchors, d_raw, n, d_start, d_stop, d_mapq, d_strand, device):
         """Launch the unpack kernel on the current stream: device words/anchors (of the slice's first
         block) -> columns of ``n`` fragments."""
-        check(lib().ftk_unpack_fragments(
-            d_words.data_ptr(), d_anchors.data_ptr(), d_raw[0].data_ptr(), d_raw[1].data_ptr(), d_raw[2].data_ptr(),
-            d_raw[3].data_ptr() if self.has_strand else 0, self.n_raw, int(n), d_start.data_ptr(), d_stop.data_ptr(),
-            0 if d_mapq is None else d_mapq.data_ptr(), 0 if d_strand is None else d_strand.data_ptr(),
-            self.record_bytes, _stream_ptr(device)), "ftk_unpack_fragments")
+        _launch(device, "ftk_unpack_fragments",
+                d_words.data_ptr(), d_anchors.data_ptr(), d_raw[0].data_ptr(), d_raw[1].data_ptr(), d_raw[2].data_ptr(),
+                d_raw[3].data_ptr() if self.has_strand else 0, self.n_raw, int(n), d_start.data_ptr(), d_stop.data_ptr(),
+                0 if d_mapq is None else d_mapq.data_ptr(), 0 if d_strand is None else d_strand.data_ptr(),
+                self.record_bytes)
 
     def to_device(self, device=None, contig=None) -> ContigFragments:
         """H2D of the packed columns + on-device unpack -> resident ``ContigFragments``."""

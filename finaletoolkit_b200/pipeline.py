@@ -20,8 +20,7 @@ from __future__ import annotations
 
 import numpy as np
 
-from ._lib import check, lib
-from .device import WpsPlan, _stream_ptr, none_to_ftk, require_cuda, torch
+from .device import WpsPlan, _launch, none_to_ftk, require_cuda, torch
 from .packed import PACK_BLOCK, PackedFragments
 
 __all__ = ["StreamedContig"]
@@ -153,18 +152,19 @@ class StreamedContig:
     def run(self):
         """One end-to-end pass; returns after every result is in the pinned host buffers."""
         t = torch()
-        if self.use_graph and self._warm:
-            if self._graph is None:
-                g = t.cuda.CUDAGraph()
-                cap = t.cuda.Stream(self.device)
-                cap.wait_stream(t.cuda.current_stream(self.device))
-                with t.cuda.graph(g, stream=cap):
-                    self._enqueue()
-                self._graph = g
-            self._graph.replay()
-        else:
-            self._enqueue()
-            self._warm = True
+        with t.cuda.device(self.device):     # the graph is captured and replayed on the buffers' device
+            if self.use_graph and self._warm:
+                if self._graph is None:
+                    g = t.cuda.CUDAGraph()
+                    cap = t.cuda.Stream(self.device)
+                    cap.wait_stream(t.cuda.current_stream(self.device))
+                    with t.cuda.graph(g, stream=cap):
+                        self._enqueue()
+                    self._graph = g
+                self._graph.replay()
+            else:
+                self._enqueue()
+                self._warm = True
         t.cuda.current_stream(self.device).synchronize()
         if int(self.h_flag[0]):
             raise OverflowError(f"WPS does not fit {self.wps_dtype} on this input; rerun with "
@@ -177,9 +177,8 @@ class StreamedContig:
         t = torch()
         W, lo, hi, q = self.params
         c_lo, c_hi, c_q = self.cov_params
-        L = lib()
         kind = 1 if self.wps_dtype == "int16" else 2
-        wps_tiles = L.ftk_wps_tiles_i16 if self.wps_dtype == "int16" else L.ftk_wps_tiles_i8
+        wps_tiles = "ftk_wps_tiles_i16" if self.wps_dtype == "int16" else "ftk_wps_tiles_i8"
         cur = t.cuda.current_stream(self.device)
         for s_ in (self.s_in, self.s_comp, self.s_out):
             s_.wait_stream(cur)
@@ -208,22 +207,20 @@ class StreamedContig:
                     if self.packed is not None and not self.packed.has_mapq:
                         mq = 0
                     if self.fused:
-                        check(L.ftk_wps_cov_tiles(
-                            fs, fe, mq, nf, self.max_frag_len,
+                        _launch(
+                            self.device, "ftk_wps_cov_tiles", fs, fe, mq, nf, self.max_frag_len,
                             plan.tile_p0.data_ptr(), plan.tile_len.data_ptr(), plan.tile_mid_lo.data_ptr(),
                             plan.tile_mid_hi.data_ptr(), plan.tile_out_off.data_ptr(), plan.tile_ivl.data_ptr(),
                             plan.n_tiles, W, none_to_ftk(lo), hi, q, none_to_ftk(c_lo), none_to_ftk(c_hi), c_q,
                             self.n_bins, 0, plan.scratch.data_ptr(), kind, self.d_out[b].data_ptr(),
                             self.d_flag.data_ptr(), self.d_cov[c["i0"]:].data_ptr(),
-                            self.d_hist.data_ptr() if self.n_bins else 0, _stream_ptr(self.device)),
-                            "ftk_wps_cov_tiles")
+                            self.d_hist.data_ptr() if self.n_bins else 0)
                     else:
-                        check(wps_tiles(
-                            fs, fe, mq, nf, plan.tile_p0.data_ptr(), plan.tile_len.data_ptr(),
+                        _launch(
+                            self.device, wps_tiles, fs, fe, mq, nf, plan.tile_p0.data_ptr(), plan.tile_len.data_ptr(),
                             plan.tile_mid_lo.data_ptr(), plan.tile_mid_hi.data_ptr(), plan.tile_out_off.data_ptr(),
                             plan.n_tiles, W, none_to_ftk(lo), hi, q, 0, plan.scratch.data_ptr(),
-                            self.d_out[b].data_ptr(), self.d_flag.data_ptr(), _stream_ptr(self.device)),
-                            "ftk_wps_tiles_" + self.wps_dtype[3:])
+                            self.d_out[b].data_ptr(), self.d_flag.data_ptr())
                     launches += 2
                 self.ev_comp[b].record(self.s_comp)
             with t.cuda.stream(self.s_out):
