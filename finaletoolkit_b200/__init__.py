@@ -19,7 +19,8 @@ _EXPORTS = {
     "wps": ("frag", "wps"), "multi_wps": ("frag", "multi_wps"), "adjust_wps": ("frag", "adjust_wps"),
     "cleavage_profile": ("frag", "cleavage_profile"), "multi_cleavage_profile": ("frag", "multi_cleavage_profile"),
     "coverage_profile": ("frag", "coverage_profile"), "multi_coverage_profile": ("frag", "multi_coverage_profile"),
-    "vplot": ("frag", "vplot"), "gc_bias": ("frag", "gc_bias"), "GCBias": ("frag", "GCBias"),
+    "vplot": ("frag", "vplot"), "ocf": ("frag", "ocf"), "OcfResult": ("frag", "OcfResult"),
+    "gc_bias": ("frag", "gc_bias"), "GCBias": ("frag", "GCBias"),
     "read_gc_bias": ("frag", "read_gc_bias"), "gc_corrected_coverage": ("frag", "gc_corrected_coverage"),
     "gc_corrected_profile": ("frag", "gc_corrected_profile"), "GCCoverageResult": ("frag", "GCCoverageResult"),
     "GCSiteProfile": ("frag", "GCSiteProfile"), "wps_spectrum": ("frag", "wps_spectrum"),

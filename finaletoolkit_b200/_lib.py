@@ -75,6 +75,8 @@ SYMBOLS = {
                                     c_int32, c_int32, c_int32, c_int32, _P, _P, _P]),
     "ftk_vplot_u64": (c_int, [_P, _P, _P, c_int64, c_int32, _P, _P, _P, c_int64, c_int32, c_int32, c_int32,
                               c_int32, c_int32, _P, _P, _P]),
+    "ftk_ocf_u64": (c_int, [_P, _P, _P, c_int64, c_int32, _P, _P, _P, _P, c_int64, c_int32, c_int32, c_int32,
+                            c_int32, c_int32, c_int32, _P, c_int32, c_int64, _P, _P, _P]),
     "ftk_gc_observed_u64": (c_int, [_P, _P, _P, c_int64, c_int32, _P, _P, c_int64, _P, _P, c_int64, c_int32, c_int32,
                                     c_int32, c_int32, _P, _P, _P]),
     "ftk_gc_expected_u64": (c_int, [_P, _P, c_int64, _P, _P, c_int64, c_int32, c_int32, c_int32, _P, _P]),

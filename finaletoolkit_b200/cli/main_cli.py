@@ -6,8 +6,8 @@ Table-driven Click group.  For every in-scope subcommand the flag spellings, par
 cli/_dispatch.py:96-118 and expands ``--strand`` into both_strands / negative_strand
 (cli/_dispatch.py:25-36).  Out-of-scope subcommands (delfi, breakpoint motifs, filter-file, agg-bw,
 gap-bed) are not registered.  ``EXTRA_COMMANDS``, ``SITE_COMMANDS``, ``BIAS_COMMANDS``, ``CORRECTION_COMMANDS`` and
-``SPECTRUM_COMMANDS`` hold the subcommands this package adds (coverage-profile, vplot, gc-bias,
-gc-corrected-coverage / gc-corrected-profile, wps-spectrum).
+``SPECTRUM_COMMANDS`` and ``ORIENTATION_COMMANDS`` hold the subcommands this package adds (coverage-profile, vplot,
+gc-bias, gc-corrected-coverage / gc-corrected-profile, wps-spectrum, ocf).
 """
 from __future__ import annotations
 
@@ -255,6 +255,23 @@ SPECTRUM_COMMANDS = {
         _minlen(120), _maxlen(180), _mapq(30), _THREADS, _VERBOSE]),
 }
 
+# fragment-end orientation subcommands, in their own table for the same reason
+ORIENTATION_COMMANDS = {
+    "ocf": ("finaletoolkit_b200.frag", "ocf",
+            "Orientation-aware fragment end profiles (OCF) summed over the sites of each BED file.", [
+        _INPUT, _arg("site_beds", metavar="SITES", nargs=-1, required=True), _REF,
+        _out("TSV (or .tsv.gz) of the OCF value of each site set."),
+        _opt("--profiles", "profile_file", metavar="PATH", default=None,
+             help="TSV (or .tsv.gz) of the upstream and downstream end counts of each site set."),
+        _opt("--flank", "flank", metavar="BP", default=1000, show_default=True, type=int,
+             help="Largest end offset from a site centre (at most 8192)."),
+        _opt("--peak-offset", "peak_offset", metavar="BP", default=60, show_default=True, type=int,
+             help="Centre of the OCF peak windows."),
+        _opt("--peak-width", "peak_width", metavar="BP", default=20, show_default=True, type=int,
+             help="Width of the OCF peak windows."),
+        _minlen(None), _maxlen(None), _mapq(30), _THREADS, _VERBOSE]),
+}
+
 
 def run(module: str, func: str, params: dict):
     """Import the target lazily, translate --strand, keep only the kwargs it accepts, call it."""
@@ -284,7 +301,7 @@ def main_cli():
 
 
 for _name, (_module, _func, _help, _spec) in {**COMMANDS, **EXTRA_COMMANDS, **SITE_COMMANDS, **BIAS_COMMANDS,
-                                              **CORRECTION_COMMANDS, **SPECTRUM_COMMANDS}.items():
+                                              **CORRECTION_COMMANDS, **SPECTRUM_COMMANDS, **ORIENTATION_COMMANDS}.items():
     main_cli.add_command(_make(_name, _module, _func, _help, _spec))
 
 

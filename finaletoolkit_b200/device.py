@@ -14,7 +14,7 @@ from ._lib import FTK_NONE, FtkLibraryError, check, lib
 
 __all__ = ["ContigFragments", "WpsPlan", "AdjustPlan", "IntervalSet", "PackedContig", "interval_hist", "frag_lengths",
            "end_motif_hist", "delfi_windows", "blacklist_in_windows", "agg_signal", "require_cuda", "none_to_ftk", "policy_code",
-           "vplot_sites", "gc_observed", "gc_expected", "gc_weighted_intervals", "gc_weighted_sites",
+           "vplot_sites", "ocf_sites", "gc_observed", "gc_expected", "gc_weighted_intervals", "gc_weighted_sites",
            "spectrum_segments"]
 
 _torch = None
@@ -463,6 +463,112 @@ def vplot_sites(frags: ContigFragments, site_center, site_flip, flank, min_lengt
         fs, fe, mq, frags.n, frags.max_len, sites.start.data_ptr(), sites.stop.data_ptr(), flip.data_ptr(), n,
         flank, int(min_length), int(max_length), int(quality_threshold), _splits_for(n, frags.n),
         sites.scratch.data_ptr(), out.data_ptr())
+    return out
+
+
+OCF_MAX_FLANK = 8192          # FTK_OCF_MAX_FLANK
+OCF_MAX_CELLS = 1 << 27       # FTK_OCF_MAX_CELLS
+# A CTA of the OCF kernel adds its 32-bit shared counters to the output before the candidate fragments it has taken
+# since its last flush could pass this (one candidate adds at most 1 to a counter).  Tests set it small.
+OCF_FLUSH_CANDIDATES = 2 ** 32 - 1
+
+
+def _ocf_shape(flank, n_sets):
+    if isinstance(flank, bool) or int(flank) != flank or not 0 <= int(flank) <= OCF_MAX_FLANK:
+        raise ValueError(f"flank must be an integer in [0, {OCF_MAX_FLANK}], got {flank!r}")
+    if isinstance(n_sets, bool) or int(n_sets) != n_sets or int(n_sets) < 1:
+        raise ValueError(f"need at least one site set, got {n_sets!r}")
+    shape = (int(n_sets), 2, 2 * int(flank) + 1)
+    if shape[0] * shape[1] * shape[2] > OCF_MAX_CELLS:
+        raise ValueError(f"{shape[0]} site sets x 2 x {shape[2]} offsets exceed {OCF_MAX_CELLS} cells")
+    return shape
+
+
+def ocf_check(flank, peak_offset, peak_width, n_sets):
+    """ValueError unless ``0 <= flank <= 8192``, ``n_sets >= 1`` and the peak windows ``P+ = [o - w // 2,
+    o - w // 2 + w)`` and ``P- = -P+`` (``o = peak_offset``, ``w = peak_width``, integers) satisfy ``w >= 1``,
+    ``o - w // 2 >= 1`` and ``o - w // 2 + w - 1 <= flank``; returns the shape ``(n_sets, 2, 2 * flank + 1)`` of
+    the end-count matrix."""
+    shape = _ocf_shape(flank, n_sets)
+    for name, v in (("peak_offset", peak_offset), ("peak_width", peak_width)):
+        if isinstance(v, bool) or not isinstance(v, (int, np.integer)):
+            raise ValueError(f"{name} must be an integer, got {v!r}")
+    o, w, f = int(peak_offset), int(peak_width), int(flank)
+    if w < 1 or o - w // 2 < 1 or o - w // 2 + w - 1 > f:
+        raise ValueError(f"the peak window [{o - w // 2}, {o - w // 2 + w - 1}] (peak_offset {o}, peak_width {w}) "
+                         f"must have a width >= 1 and lie within [1, flank = {f}]")
+    return shape
+
+
+def ocf_length_check(min_length, max_length) -> None:
+    """ValueError unless each bound is None (unbounded) or an integer in [0, 2**31 - 1] and min <= max."""
+    for name, v in (("min_length", min_length), ("max_length", max_length)):
+        if v is not None and (isinstance(v, bool) or int(v) != v or not 0 <= int(v) <= 2 ** 31 - 1):
+            raise ValueError(f"{name} must be None or an integer in [0, 2**31 - 1], got {v!r}")
+    if min_length is not None and max_length is not None and int(max_length) < int(min_length):
+        raise ValueError(f"need min_length <= max_length, got {min_length} and {max_length}")
+
+
+def _ocf_cta_bounds(site_set: np.ndarray, n_sets: int, splits: int) -> np.ndarray:
+    """Unit boundaries of the OCF kernel's CTAs over sites sorted by set (unit = site * splits + slice): each set's
+    units are split into about ``_TARGET_CTAS`` * (its share of the units) CTAs of at least 8 units (one per warp)
+    where it has that many; no CTA crosses a set."""
+    per_set = np.bincount(site_set, minlength=n_sets).astype(np.int64) * splits
+    total = int(per_set.sum())
+    bounds, first = [0], 0
+    for u in per_set.tolist():
+        if u == 0:
+            continue
+        n_cta = max(1, min(-(-u // 8), -(-u * _TARGET_CTAS // total)))
+        bounds += [first + u * j // n_cta for j in range(1, n_cta + 1)]
+        first += u
+    return np.asarray(bounds, dtype=np.int32)
+
+
+def ocf_sites(frags: ContigFragments, site_center, site_flip, site_set, n_sets, flank, min_length=None,
+              max_length=None, quality_threshold=30, out=None):
+    """Upstream- and downstream-end offset counts around the sites of one contig, summed per site set
+    (``ftk_ocf_u64``).
+
+    Site k is centred on ``site_center[k]``, mirrored when ``site_flip[k]`` is true and belongs to set
+    ``site_set[k]`` (``0 <= site_set[k] < n_sets``).  A fragment ``[s, e)`` passes when mapq >=
+    ``quality_threshold`` and ``max(1, min_length) <= e - s <= max_length`` (None = unbounded).  Its upstream end
+    offset is ``s - c`` and its downstream one ``e - 1 - c`` (mirrored: ``c - (e - 1)`` and ``c - s``); each end
+    within ``flank`` of the centre adds 1 at ``[set, 0, x + flank]`` (upstream) or ``[set, 1, x + flank]``
+    (downstream).  Returns the device int64 tensor of shape ``(n_sets, 2, 2 * flank + 1)``; ``out`` (such a tensor)
+    is accumulated into."""
+    t = torch()
+    shape = _ocf_shape(flank, n_sets)
+    ocf_length_check(min_length, max_length)
+    dev = frags.device
+    if out is None:
+        out = t.zeros(shape, dtype=t.int64, device=dev)
+    elif out.dtype != t.int64 or tuple(out.shape) != shape or not out.is_contiguous():
+        raise ValueError(f"out must be a contiguous int64 tensor of shape {shape}")
+    c = np.asarray(site_center, dtype=np.int64).reshape(-1)
+    n = c.size
+    s = np.asarray(site_set, dtype=np.int64).reshape(-1)
+    f = np.asarray(site_flip, dtype=bool).reshape(-1)
+    if s.size != n or f.size != n:
+        raise ValueError(f"site_center, site_flip and site_set must have the same length, got {n}, {f.size}, {s.size}")
+    if n == 0:
+        return out
+    if int(s.min()) < 0 or int(s.max()) >= shape[0]:
+        raise ValueError(f"site sets must lie in [0, {shape[0]})")
+    flank = int(flank)
+    # a CTA counts one set; 16-bit keys take numpy's linear-time radix sort
+    order = np.argsort(s.astype(np.uint16) if shape[0] <= 1 << 16 else s, kind="stable")
+    c, f, s = c[order], f[order], s[order]
+    sites, flip = _site_windows(c, f, flank, dev)
+    splits = _splits_for(n, frags.n)
+    bounds = _ocf_cta_bounds(s, shape[0], splits)
+    tab = _to_device(np.concatenate([s.astype(np.int32), bounds]), dev, np.int32)
+    fs, fe, mq = frags.ptrs()
+    _launch(dev, "ftk_ocf_u64",
+        fs, fe, mq, frags.n, frags.max_len, sites.start.data_ptr(), sites.stop.data_ptr(), flip.data_ptr(),
+        tab.data_ptr(), n, shape[0], flank, none_to_ftk(min_length), none_to_ftk(max_length), int(quality_threshold),
+        splits, tab[n:].data_ptr(), bounds.size - 1, int(OCF_FLUSH_CANDIDATES), sites.scratch.data_ptr(),
+        out.data_ptr())
     return out
 
 

@@ -430,6 +430,34 @@ int ftk_vplot_u64(const int32_t *frag_start_dev, const int32_t *frag_stop_dev, c
                   const uint8_t *site_flip_dev, int64_t n_sites, int32_t flank, int32_t min_len, int32_t max_len,
                   int32_t min_mapq, int32_t splits, int64_t *scratch_dev, uint64_t *out_dev, ftk_stream_t stream);
 
+/* ---------------------------------------------------------------- OCF end profiles
+ * Orientation-aware fragment end profiles (Sun et al. 2019): upstream- and downstream-end offset counts
+ * around sites, summed over the sites of each of n_sets site sets.  Site k has the window of ftk_vplot_u64
+ * ([win_lo[k], win_hi[k]) = [c - flank, c + flank + 1), c = win_lo[k] + flank), is flipped when
+ * site_flip[k] != 0 and belongs to set site_set[k] (0 <= site_set[k] < n_sets).  A fragment [s, e) passes when
+ * mapq >= min_mapq, L = e - s >= 1 and min_len <= L <= max_len (FTK_NONE = unbounded).  Its upstream end
+ * offset is x_U = s - c and its downstream one x_D = (e - 1) - c (flipped: x_U = c - (e - 1), x_D = c - s).
+ * For every site of set k and every passing fragment, each end independently:
+ *   out[(2 k + 0) * (2 * flank + 1) + x_U + flank] += 1  when |x_U| <= flank
+ *   out[(2 k + 1) * (2 * flank + 1) + x_D + flank] += 1  when |x_D| <= flank
+ * out_dev: uint64[n_sets][2][2 * flank + 1], ACCUMULATED (the caller zeroes it).
+ * Work split: each site's candidate range is split into `splits` slices, unit u = site * splits + slice is one
+ * warp, and CTA b (of n_cta) takes the units [cta_bounds_dev[b], cta_bounds_dev[b + 1]) (int32[n_cta + 1]),
+ * which must all belong to one set: sort the sites by set.  A CTA counts in shared memory and adds its counts
+ * to out_dev before the candidate fragments it has taken since the last such flush pass flush_every
+ * (1 <= flush_every <= 2^32 - 1; 2^32 - 1 flushes only when a 32-bit counter could overflow).
+ * scratch_dev: int64[2 * n_sites].  max_frag_len = max(stop - start) over the contig.  0 <= flank <=
+ * FTK_OCF_MAX_FLANK, at most FTK_OCF_MAX_CELLS cells, n_sites * splits <= INT32_MAX; n_sites == 0 or
+ * n_frag == 0 returns 0 without a launch. */
+#define FTK_OCF_MAX_FLANK 8192
+#define FTK_OCF_MAX_CELLS (1 << 27)
+int ftk_ocf_u64(const int32_t *frag_start_dev, const int32_t *frag_stop_dev, const uint8_t *frag_mapq_dev,
+                int64_t n_frag, int32_t max_frag_len, const int32_t *win_lo_dev, const int32_t *win_hi_dev,
+                const uint8_t *site_flip_dev, const int32_t *site_set_dev, int64_t n_sites, int32_t n_sets,
+                int32_t flank, int32_t min_len, int32_t max_len, int32_t min_mapq, int32_t splits,
+                const int32_t *cta_bounds_dev, int32_t n_cta, int64_t flush_every, int64_t *scratch_dev,
+                uint64_t *out_dev, ftk_stream_t stream);
+
 /* ---------------------------------------------------------------- GC bias
  * Fragment-level GC model (Benjamini & Speed 2012): fragment counts by (length, G+C bases), observed over the
  * sample's fragments and expected over every placement a fragment of that length could take.

@@ -1,5 +1,5 @@
 """Kernel timing helper (python tools/quick_kernels.py [motif] [bp] [adjust] [delfi] [hist] [cleavage] [depth] [depth-mid]
-[vplot] [vplot-dense]
+[vplot] [vplot-dense] [ocf] [ocf-dense]
 [gc-obs] [gc-exp] [gc-cov] [gc-site] [spectrum]):
 CUDA-event time of the secondary kernels at chr1 scale (80 M fragments drawn on the GPU), median of 7 calls after 3
 warm-ups (the call: planning and uploads included).  Every op except adjust also prints an order-sensitive checksum
@@ -107,6 +107,20 @@ for name, step in (("vplot", 5000), ("vplot-dense", 500)):
         print(f"{name}: {vc.size} sites, {cand} candidates, {events} events", flush=True)
         op(name, lambda: D.vplot_sites(fr, vc, vf, 1000, 0, 600, 30), 9 * cand)
         print(f"  {events / timed.ms / 1e6:.2f} G events/s over the call", flush=True)
+for name, step in (("ocf", 5000), ("ocf-dense", 500)):
+    if name in what:
+        # the sites of vplot / vplot-dense dealt round-robin into 8 sets, flank 1000, every length, q 30
+        oc = np.arange(step // 2, CLEN, step, dtype=np.int64)
+        of = np.arange(oc.size) % 2 == 1
+        osets = np.arange(oc.size) % 8
+        reach = fr.max_len
+        a = torch.searchsorted(st, torch.tensor(oc - 1000 - reach, dtype=torch.int32, device=dev))
+        b = torch.searchsorted(st, torch.tensor(oc + 1001, dtype=torch.int32, device=dev))
+        cand = int((b - a).sum())
+        o = D.ocf_sites(fr, oc, of, osets, 8, 1000, None, None, 30)
+        print(f"{name}: {oc.size} sites, {cand} candidates, {int(o.sum())} events", flush=True)
+        op(name, lambda: D.ocf_sites(fr, oc, of, osets, 8, 1000, None, None, 30), 9 * cand)
+        print(f"  {int(o.sum()) / timed.ms / 1e6:.2f} G events/s over the call", flush=True)
 # GC bias: one whole-contig region, lengths 50..500, q 30
 if "gc-obs" in what:
     o = D.gc_observed(fr, ref, [0], [CLEN], 50, 500, 30)
