@@ -220,6 +220,8 @@ adjust_hist_kernel(const float *__restrict__ x, const long long *__restrict__ se
 // ------------------------------------------------------------ generic path
 // Any float input: the window is kept sorted in a per-thread scratch array (binary
 // search + shift on every step, O(w) per output).  Only flagged runs come here.
+// NaN has no place in a sorted order: the window keeps its non-NaN samples sorted
+// (len of them) and counts the NaNs; a window holding a NaN has median NaN, as numpy's.
 __global__ void __launch_bounds__(64)
 adjust_generic_kernel(const float *__restrict__ x, const long long *__restrict__ seg_off,
                       const long long *__restrict__ seg_out_off, const long long *__restrict__ seg_run_off,
@@ -239,18 +241,28 @@ adjust_generic_kernel(const float *__restrict__ x, const long long *__restrict__
     const long long ca = (run - seg_run_off[s]) * P.run;
     const long long cb = (ca + P.run < n_out) ? ca + P.run : n_out;
     const int w = P.w;
-    for (int t = 0; t < w; ++t) {  // insertion sort of the first window
-        const float v = xs[ca + t];
-        int k = t;
+    int len = 0, n_nan = 0;        // sorted non-NaN samples in win[0, len), NaNs in the window
+    auto insert = [&](float v) {
+        if (v != v) { ++n_nan; return; }
+        int k = len++;
         while (k > 0 && win[k - 1] > v) { win[k] = win[k - 1]; --k; }
         win[k] = v;
-    }
+    };
+    auto find = [&](float v) {     // position of one copy of v
+        int lo = 0, hi = len;
+        while (lo < hi) { const int mid = (lo + hi) >> 1; if (win[mid] < v) lo = mid + 1; else hi = mid; }
+        return lo;
+    };
+    if (!P.use_mean)
+        for (int t = 0; t < w; ++t) insert(xs[ca + t]);   // insertion sort of the first window
     for (long long c = ca; c < cb; ++c) {
         double stat;
         if (P.use_mean) {
             double sum = 0.0;  // fp64 left-to-right sum of the shifted window (numpy: pairwise; <= 1e-13 rel apart)
             for (int t = 0; t < w; ++t) sum += (double)xs[c + t] - shift;
             stat = sum / (double)w;
+        } else if (n_nan) {
+            stat = nan("");
         } else {
             const double lo = (double)win[(w - 1) >> 1] - shift, hi = (double)win[w >> 1] - shift;
             stat = (lo + hi) / 2.0;
@@ -258,12 +270,19 @@ adjust_generic_kernel(const float *__restrict__ x, const long long *__restrict__
         out[c] = ((double)xs[c + (w >> 1)] - shift) - stat;
         if (c + 1 < cb && !P.use_mean) {
             const float vo = xs[c], vi = xs[c + w];
-            int lo = 0, hi = w;  // position of one copy of vo
-            while (lo < hi) { const int mid = (lo + hi) >> 1; if (win[mid] < vo) lo = mid + 1; else hi = mid; }
-            int k = lo;
-            if (vi >= vo) { while (k + 1 < w && win[k + 1] < vi) { win[k] = win[k + 1]; ++k; } }
-            else { while (k > 0 && win[k - 1] > vi) { win[k] = win[k - 1]; --k; } }
-            win[k] = vi;
+            if (vo != vo || vi != vi) {   // a NaN enters or leaves: drop vo, then insert vi
+                if (vo != vo) --n_nan;
+                else {
+                    for (int k = find(vo); k + 1 < len; ++k) win[k] = win[k + 1];
+                    --len;
+                }
+                insert(vi);
+            } else {                      // replace vo by vi in one pass
+                int k = find(vo);
+                if (vi >= vo) { while (k + 1 < len && win[k + 1] < vi) { win[k] = win[k + 1]; ++k; } }
+                else { while (k > 0 && win[k - 1] > vi) { win[k] = win[k - 1]; --k; } }
+                win[k] = vi;
+            }
         }
     }
 }
@@ -873,19 +892,22 @@ adjust_rank_kernel(const InT *__restrict__ x, const long long *__restrict__ seg_
     }
 }
 
-// subtract_edges (frag/_adjust_wps.py:119-123): shift[s] = mean(mean(x[:e]), mean(x[-e:]))
+// subtract_edges (frag/_adjust_wps.py:119-123): shift[s] = mean(mean(x[:e]), mean(x[-e:])) with Python's slice
+// bounds: e >= n takes all of x twice, e == 0 an empty head (x[-0:] is all of x), e < 0 drops |e| samples from the
+// other end.  The mean of an empty slice is 0 / 0 = NaN, and so is the shift then.
 __global__ void adjust_edge_shift_kernel(const float *__restrict__ x, const long long *__restrict__ seg_off,
                                          int n_seg, int edge, double *__restrict__ shift) {
     const int s = blockIdx.x * blockDim.x + threadIdx.x;
     if (s >= n_seg) return;
     const long long n = seg_off[s + 1] - seg_off[s];
     const float *xs = x + seg_off[s];
-    const long long e = edge < n ? edge : n;
-    if (e <= 0) { shift[s] = 0.0; return; }
+    const long long e = edge;
+    const long long a_end = e >= 0 ? (e < n ? e : n) : (n + e > 0 ? n + e : 0);                 // x[:e]
+    const long long b_beg = e > 0 ? (n - e > 0 ? n - e : 0) : e == 0 ? 0 : (-e < n ? -e : n);  // x[-e:]
     double a = 0.0, b = 0.0;  // exact for integer-valued samples (|sum| < 2^53)
-    for (long long t = 0; t < e; ++t) a += (double)xs[t];
-    for (long long t = n - e; t < n; ++t) b += (double)xs[t];
-    shift[s] = ((a / (double)e) + (b / (double)e)) / 2.0;
+    for (long long t = 0; t < a_end; ++t) a += (double)xs[t];
+    for (long long t = b_beg; t < n; ++t) b += (double)xs[t];
+    shift[s] = ((a / (double)a_end) + (b / (double)(n - b_beg))) / 2.0;
 }
 
 }  // namespace ftk
@@ -895,7 +917,7 @@ using namespace ftk;
 extern "C" int ftk_adjust_edge_shift_f64(const float *x, const int64_t *seg_off, int32_t n_seg,
                                          int32_t edge_size, double *shift, ftk_stream_t stream_) {
     if (n_seg == 0) return FTK_OK;
-    if (!x || !seg_off || !shift || n_seg < 0 || edge_size < 0) return FTK_E_INVALID;
+    if (!x || !seg_off || !shift || n_seg < 0) return FTK_E_INVALID;
     adjust_edge_shift_kernel<<<(n_seg + 127) / 128, 128, 0, static_cast<cudaStream_t>(stream_)>>>(
         x, reinterpret_cast<const long long *>(seg_off), n_seg, edge_size, shift);
     FTK_CHECK_LAUNCH("adjust_edge_shift_kernel");

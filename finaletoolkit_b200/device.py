@@ -960,20 +960,33 @@ def savgol_tables(window: int, degree: int):
 def _savgol_tables_cached(window: int, degree: int):
     """The tables of ``savgol_tables``.
 
-    Same least-squares construction as scipy.signal.savgol_filter (reference call site
-    frag/_adjust_wps.py:135-138; scipy/signal/_savitzky_golay.py): interior = the centre
-    row of the hat matrix of a degree-``degree`` polynomial fit over ``window`` points;
-    the first/last ``window//2`` outputs evaluate the fit of the first/last ``window``
-    samples at their own positions.
+    The filter of scipy.signal.savgol_filter (reference call site frag/_adjust_wps.py:135-138;
+    scipy/signal/_savitzky_golay.py): interior = the centre row of the hat matrix of a
+    degree-``degree`` least-squares polynomial fit over ``window`` points; the first/last
+    ``window//2`` outputs evaluate the fit of the first/last ``window`` samples at their own
+    positions.
+
+    The hat matrix is ``Q Q^T`` with ``Q`` an orthonormal basis of the polynomials of degree
+    <= ``degree`` on the window positions, built by the Arnoldi (Stieltjes) process: column
+    k+1 = position * column k, orthogonalised twice against every earlier column.  A
+    Vandermonde matrix and its pseudo-inverse lose digits with the degree (wrong filters
+    from degree ~10 on a 93-point window); this stays within a few ulp of the exact rational
+    hat matrix at every degree.
     """
     if window % 2 != 1 or window < 1:
         raise ValueError("window_length must be odd.")
     if degree >= window:
         raise ValueError("polyorder must be less than window_length.")
     half = window // 2
-    pos = np.arange(-half, half + 1, dtype=np.float64)
-    A = np.vander(pos, degree + 1, increasing=True)
-    hat = A @ np.linalg.pinv(A)              # hat[i, j]: weight of sample j in the fit at i
+    pos = np.arange(-half, half + 1, dtype=np.float64) / max(half, 1)
+    Q = np.empty((window, degree + 1))
+    Q[:, 0] = 1.0 / np.sqrt(window)
+    for k in range(degree):
+        v = pos * Q[:, k]
+        for _ in range(2):
+            v -= Q[:, : k + 1] @ (Q[:, : k + 1].T @ v)
+        Q[:, k + 1] = v / np.linalg.norm(v)
+    hat = Q @ Q.T                            # hat[i, j]: weight of sample j in the fit at i
     coef = np.ascontiguousarray(hat[half])   # symmetric: correlation == convolution
     edge_first = np.ascontiguousarray(hat[:half])
     edge_last = np.ascontiguousarray(hat[half + 1:])

@@ -327,7 +327,8 @@ int ftk_agg_signal_f64(const float *signal_dev, int64_t n_seg, int64_t row_len, 
  * (sg_w/2 x sg_w) edge-fit matrices.  w even, 2 <= w <= 32767; sg_w odd <= 127.
  * seg_shift_dev: per-segment constant to subtract (NULL = 0), e.g. from
  * ftk_adjust_edge_shift_f64 = mean(mean(x[:edge]), mean(x[-edge:]))
- * (subtract_edges, frag/_adjust_wps.py:119-123). */
+ * (subtract_edges, frag/_adjust_wps.py:119-123), with Python's slice semantics for any edge: 0 or a
+ * negative edge that empties a slice gives NaN. */
 int ftk_adjust_edge_shift_f64(const float *x_dev, const int64_t *seg_off_dev, int32_t n_seg,
                               int32_t edge_size, double *shift_dev, ftk_stream_t stream);
 

@@ -227,6 +227,34 @@ def test_savgol_tables_match_scipy():
         savgol_tables(20, 2)
 
 
+def test_savgol_tables_match_exact_hat_matrix():
+    """Every table entry within 16 ulp (``TABLE_ULPS``) of max |H| of the exact rational hat matrix (tests/savgol_oracle.py), over
+    every odd window 1..127 with degrees 0..min(m - 1, 20), and the extremes (127, 126) and (3, 2).  An entry of
+    ``Q Q^T`` is a (degree + 1)-term sum of products of basis entries that are each a few ulp off; the worst on this
+    grid is 8.5 ulp, at (113, 9).  The Vandermonde / pseudo-inverse construction it replaced was ~1e-4 off at (127, 8)
+    and a different filter at (93, 10).  Where scipy's own coefficients drift from the exact filter (more than 1e-9
+    relative) the tables must be the closer of the two."""
+    from scipy.signal import savgol_coeffs
+    from finaletoolkit_b200.device import savgol_tables
+    from savgol_oracle import TABLE_ULPS, hat_float
+    eps = np.finfo(np.float64).eps
+    n_scipy_off = 0
+    grid = [(m, d) for m in range(1, 128, 2) for d in range(min(m - 1, 20) + 1)]
+    for m, d in grid + [(127, 126), (3, 2)]:
+        c, ef, el = savgol_tables(m, d)
+        h = m // 2
+        assert c.shape == (m,) and ef.shape == (h, m) and el.shape == (h, m)
+        E = hat_float(m, d)                                    # the exact H, correctly rounded entry by entry
+        scale = np.abs(E).max()
+        err = np.abs(np.vstack([ef, c[None], el]) - E).max()
+        assert err <= TABLE_ULPS * eps * scale, (m, d, err / (eps * scale))
+        err_sp = np.abs(savgol_coeffs(m, d) - E[h]).max()
+        if err_sp > 1e-9 * scale:
+            n_scipy_off += 1
+            assert np.abs(c - E[h]).max() < err_sp, (m, d)
+    assert n_scipy_off >= 10                                   # the grid does reach the degrees where scipy drifts
+
+
 def test_lpt_packing():
     from finaletoolkit_b200.sharding import lpt_pack
     from finaletoolkit_b200.synth import B37_CONTIGS
