@@ -73,6 +73,8 @@ SYMBOLS = {
                                        c_int32, c_int32, c_int32, _P, _P, _P]),
     "ftk_depth_tiles_i32": (c_int, [_P, _P, _P, c_int64, c_int32, _P, _P, _P, _P, _P, c_int64,
                                     c_int32, c_int32, c_int32, c_int32, _P, _P, _P]),
+    "ftk_gc_depth_tiles_f64": (c_int, [_P, _P, _P, c_int64, c_int32, _P, _P, c_int64, _P, _P, _P, _P, _P, c_int64,
+                                       c_int32, c_int32, c_int32, c_int32, _P, c_int64, _P, _P, _P, _P]),
     "ftk_vplot_u64": (c_int, [_P, _P, _P, c_int64, c_int32, _P, _P, _P, c_int64, c_int32, c_int32, c_int32,
                               c_int32, c_int32, _P, _P, _P]),
     "ftk_ocf_u64": (c_int, [_P, _P, _P, c_int64, c_int32, _P, _P, _P, _P, c_int64, c_int32, c_int32, c_int32,

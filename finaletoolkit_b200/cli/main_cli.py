@@ -5,9 +5,10 @@ Table-driven Click group.  For every in-scope subcommand the flag spellings, par
 (cli/commands/__init__.py:87-640); dispatch filters the parameters by the target's signature like
 cli/_dispatch.py:96-118 and expands ``--strand`` into both_strands / negative_strand
 (cli/_dispatch.py:25-36).  Out-of-scope subcommands (delfi, breakpoint motifs, filter-file, agg-bw,
-gap-bed) are not registered.  ``EXTRA_COMMANDS``, ``SITE_COMMANDS``, ``BIAS_COMMANDS``, ``CORRECTION_COMMANDS`` and
-``SPECTRUM_COMMANDS`` and ``ORIENTATION_COMMANDS`` hold the subcommands this package adds (coverage-profile, vplot,
-gc-bias, gc-corrected-coverage / gc-corrected-profile, wps-spectrum, ocf).
+gap-bed) are not registered.  ``EXTRA_COMMANDS``, ``SITE_COMMANDS``, ``BIAS_COMMANDS``, ``CORRECTION_COMMANDS``,
+``GC_TRACK_COMMANDS``, ``SPECTRUM_COMMANDS`` and ``ORIENTATION_COMMANDS`` hold the subcommands this package adds
+(coverage-profile, vplot, gc-bias, gc-corrected-coverage / gc-corrected-profile, gc-corrected-coverage-profile,
+wps-spectrum, ocf).
 """
 from __future__ import annotations
 
@@ -232,6 +233,26 @@ CORRECTION_COMMANDS = {
         *_GC_MODEL, _mapq(30), _THREADS, _VERBOSE]),
 }
 
+# GC-corrected per-base tracks, in their own table for the same reason
+GC_TRACK_COMMANDS = {
+    "gc-corrected-coverage-profile": ("finaletoolkit_b200.frag", "multi_gc_corrected_coverage_profile",
+                                      "Per-base GC-corrected fragment depth (or fragment-midpoint sum) over BED "
+                                      "intervals.", [
+        _INPUT, _arg("refseq_file", metavar="REFERENCE"), _arg("interval_file", metavar="REGIONS"),
+        _arg("chrom_sizes", metavar="CHROM_SIZES"), _REF,
+        _out("bigWig or gzipped bedGraph of per-base GC-corrected depth."), *_GC_MODEL, _mapq(30),
+        _opt("--pad-left", "left", metavar="BP", default=0, show_default=True, type=int,
+             help="Base pairs to subtract from each start coordinate."),
+        _opt("--pad-right", "right", metavar="BP", default=0, show_default=True, type=int,
+             help="Base pairs to add to each stop coordinate."),
+        _opt("--midpoint", "midpoint", is_flag=True, help="Sum at fragment midpoints instead of spanned bases."),
+        _opt("--scale-factor", "scale_factor", metavar="X", default=1.0, show_default=True, type=float,
+             help="Scale factor for depth values."),
+        _opt("-n", "--normalize", "normalize", is_flag=True,
+             help="Divide the scale factor by the number of passing fragments in the file."),
+        _THREADS, _VERBOSE]),
+}
+
 # subcommands that transform WPS further, in their own table for the same reason
 SPECTRUM_COMMANDS = {
     "wps-spectrum": ("finaletoolkit_b200.frag", "wps_spectrum",
@@ -301,7 +322,8 @@ def main_cli():
 
 
 for _name, (_module, _func, _help, _spec) in {**COMMANDS, **EXTRA_COMMANDS, **SITE_COMMANDS, **BIAS_COMMANDS,
-                                              **CORRECTION_COMMANDS, **SPECTRUM_COMMANDS, **ORIENTATION_COMMANDS}.items():
+                                              **CORRECTION_COMMANDS, **GC_TRACK_COMMANDS, **SPECTRUM_COMMANDS,
+                                              **ORIENTATION_COMMANDS}.items():
     main_cli.add_command(_make(_name, _module, _func, _help, _spec))
 
 

@@ -7,11 +7,9 @@
 // out[(L - min_len) * (max_len + 1) + g] += 1 in both kernels (DESIGN.md 4.10).
 // weighted: the model applied; selected fragments counted per interval or by offset from a site centre, with their
 // weights[(L - min_len) * (max_len + 1) + g] summed where g is defined (DESIGN.md 4.11).
-//
-// Packed layout (synth.pack_twobit): base i in bits 2(i%16) of seq word i/16 (A0 C1 G2 T3), its N flag in bit
-// i%32 of nmask word i/32.  A 64-bit seq word k and nmask word k cover the same 32 bases, so every read here is
-// one aligned 64-bit seq load + one 32-bit nmask load per 32 bases; G/C <=> bit0 ^ bit1 of a base's code.
+// The packed layout and the per-fragment walk (gc_walk) are in ftk_gc_walk.cuh.
 #include "ftk_common.cuh"
+#include "ftk_gc_walk.cuh"
 
 namespace ftk {
 
@@ -21,37 +19,6 @@ constexpr int kGcLanes = 32;   // lengths per expected CTA: lane l owns length L
 
 __device__ __forceinline__ void red_global_add_u64(unsigned long long *p, unsigned long long v) {
     asm volatile("red.global.add.u64 [%0], %1;" :: "l"(p), "l"(v) : "memory");
-}
-
-__device__ __forceinline__ uint64_t gc_bits64(uint64_t x) {   // bit 2j set <=> base j of the word is C or G
-    return (x ^ (x >> 1)) & 0x5555555555555555ull;
-}
-
-// G/C bases g of [fs, fe) and whether any of its bases is N (0 <= fs < fe <= contig_len).  Walks the 32-base
-// words of the span: the N flags OR-ed from the end-masked nmask words, G/C by popc of the end-masked 64-bit G/C
-// bit pairs (a caller drops a fragment with an N before G/C of an N base could matter, so the G/C bits need no
-// N mask).
-struct GcWalk {
-    int g;
-    bool has_n;
-};
-
-__device__ __forceinline__ GcWalk gc_walk(const uint64_t *__restrict__ seq64, const uint32_t *__restrict__ nmask,
-                                          int fs, int fe) {
-    const int k0 = fs >> 5, k1 = (fe - 1) >> 5;
-    int g = 0;
-    uint32_t n = 0;
-    for (int k = k0; k <= k1; ++k) {
-        uint32_t sel = ~0u;
-        if (k == k0) sel &= ~0u << (fs & 31);
-        if (k == k1) sel &= ~0u >> (31 - ((fe - 1) & 31));
-        uint64_t sel2 = ~0ull;                               // sel spread to the base pairs of the seq word
-        if (k == k0) sel2 &= ~0ull << (2 * (fs & 31));
-        if (k == k1) sel2 &= ~0ull >> (62 - 2 * ((fe - 1) & 31));
-        n |= __ldg(nmask + k) & sel;
-        g += __popcll(gc_bits64(__ldg(seq64 + k)) & sel2);
-    }
-    return GcWalk{g, n != 0};
 }
 
 // ------------------------------------------------------------------------------------------------ observed

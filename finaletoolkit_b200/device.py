@@ -15,7 +15,7 @@ from ._lib import FTK_NONE, FtkLibraryError, check, lib
 __all__ = ["ContigFragments", "WpsPlan", "AdjustPlan", "IntervalSet", "PackedContig", "interval_hist", "frag_lengths",
            "end_motif_hist", "delfi_windows", "blacklist_in_windows", "agg_signal", "require_cuda", "none_to_ftk", "policy_code",
            "vplot_sites", "ocf_sites", "gc_observed", "gc_expected", "gc_weighted_intervals", "gc_weighted_sites",
-           "spectrum_segments"]
+           "gc_depth_intervals", "spectrum_segments"]
 
 _torch = None
 
@@ -1264,4 +1264,58 @@ def depth_intervals(frags: ContigFragments, ivl_start, ivl_stop, chrom_size, min
             plan.tile_mid_lo.data_ptr(), plan.tile_mid_hi.data_ptr(), plan.tile_out_off.data_ptr(), plan.n_tiles,
             none_to_ftk(min_length), none_to_ftk(max_length), int(quality_threshold), int(bool(midpoint)),
             plan.scratch.data_ptr(), out.data_ptr())
+    return out[: plan.n_positions], plan.offsets
+
+
+GC_DEPTH_MAX_WEIGHT = 2 ** 62   # FTK_GC_DEPTH_MAX_WEIGHT: quantised weights stay below it
+
+
+def gc_quantise_weights(weights, shape) -> np.ndarray:
+    """The weight table in units of 2^-32: ``rint(W * 2^32)`` as int64 (fp64 on the host; the scaling is exact and
+    ``rint`` rounds half to even).  ValueError unless ``weights`` has ``shape`` and every entry is finite and ``>= 0``,
+    or when a quantised weight reaches 2^62."""
+    t = torch()
+    w = weights.detach().cpu().numpy() if t.is_tensor(weights) else np.asarray(weights)
+    if tuple(w.shape) != tuple(shape):
+        raise ValueError(f"the weight table must have shape {tuple(shape)}, got {tuple(w.shape)}")
+    w = w.astype(np.float64)
+    if not bool((np.isfinite(w) & (w >= 0)).all()):
+        raise ValueError("the weight table must hold finite, non-negative values")
+    q = np.rint(w * 2.0 ** 32)
+    if q.size and float(q.max()) >= GC_DEPTH_MAX_WEIGHT:
+        raise ValueError(f"a GC weight of {float(w.max())!r} is too large for the depth tracks (below 2^30 needed)")
+    return q.astype(np.int64)
+
+
+def gc_depth_intervals(frags: ContigFragments, ref: PackedContig, ivl_start, ivl_stop, chrom_size, weights,
+                       min_length, max_length, quality_threshold=30, midpoint=False):
+    """GC-weighted per-base fragment depth (float64) of every interval back to back + host offsets
+    (``ftk_gc_depth_tiles_f64``).
+
+    A fragment ``[s, e)`` with ``mapq >= quality_threshold`` and ``min_length <= L <= max_length`` weighs
+    ``Q[L - min_length, g] * 2^-32`` with ``Q = gc_quantise_weights(weights)`` when ``0 <= s``, ``e <= ref.length`` and
+    no base of it is N (g = its C/G bases), else 0.  Span depth sums the weights of the fragments with
+    ``s <= p < e``, ``midpoint=True`` those with ``(s + e) // 2 == p``.  The sums are int64, so the result is exact
+    (``fp64(S) * 2^-32``), 0.0 where no weighted fragment counts and bit-identical between runs and batchings.
+    ``ivl_start/ivl_stop`` are already padded/clamped bounds; one launch for all of them.  OverflowError when a tile's
+    sums could pass 2^63 (a pile-up of huge weights); nothing is returned then."""
+    t = torch()
+    shape = gc_check(min_length, max_length)
+    dev = frags.device
+    _same_device(dev, ref)
+    q = gc_quantise_weights(weights, shape)
+    plan = WpsPlan(ivl_start, ivl_stop, int(chrom_size), 0, dev)   # the tile table of depth_intervals
+    out = t.empty(max(plan.n_positions, 1), dtype=t.float64, device=dev)
+    if plan.n_tiles:
+        qd = _to_device(q, dev, np.int64)
+        flag = t.zeros(1, dtype=t.int32, device=dev)
+        fs, fe, mq = frags.ptrs()
+        _launch(dev, "ftk_gc_depth_tiles_f64",
+            fs, fe, mq, frags.n, frags.max_len, ref.seq.data_ptr(), ref.nmask.data_ptr(), ref.length,
+            plan.tile_p0.data_ptr(), plan.tile_len.data_ptr(), plan.tile_mid_lo.data_ptr(), plan.tile_mid_hi.data_ptr(),
+            plan.tile_out_off.data_ptr(), plan.n_tiles, int(min_length), int(max_length), int(quality_threshold),
+            int(bool(midpoint)), qd.data_ptr(), int(q.max()), plan.scratch.data_ptr(), flag.data_ptr(), out.data_ptr())
+        if int(flag.item()):
+            raise OverflowError(f"GC-weighted depth of contig {frags.contig!r}: a pile-up of large GC weights could "
+                                "overflow the int64 sums of a tile")
     return out[: plan.n_positions], plan.offsets

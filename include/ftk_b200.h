@@ -524,6 +524,31 @@ int ftk_gc_weighted_sites_f64(const int32_t *frag_start_dev, const int32_t *frag
                               int32_t splits, int64_t *scratch_dev, const double *weights_dev,
                               uint64_t *out_count_dev, double *out_corrected_dev, ftk_stream_t stream);
 
+/* ---------------------------------------------------------------- GC-corrected depth tracks
+ * The per-base depth of ftk_depth_tiles_i32 (same tile table, scratch and midpoint switch) with the GC model
+ * applied.  weights_dev: int64 of the GC-bias matrices' shape, the weights quantised to units of 2^-32
+ * (Q = rint(W * 2^32)), read as weights[(L - min_len) * (max_len + 1) + g]; max_weight = max(Q), 0 <= max_weight <
+ * FTK_GC_DEPTH_MAX_WEIGHT.  A fragment passes when mapq >= min_mapq and min_len <= L <= max_len (1 <= min_len <=
+ * max_len <= FTK_GC_MAX_LENGTH, no FTK_NONE); its weight is Q[L - min_len, g] when start >= 0, stop <= contig_len and
+ * no base of it is N (g = its C/G bases, the placement rule of ftk_gc_observed_u64), else 0.
+ * midpoint == 0: S(p) = sum of the weights of passing fragments with start <= p < stop
+ * midpoint != 0: S(p) = sum of the weights of passing fragments with (start + stop) / 2 == p
+ * out[tile_out_off + (p - p0)] = (double)S(p) * 2^-32 (fp64; S is summed in int64, so the result is exact below 2^53
+ * units and bit-identical between runs and batchings).  Every partial sum of a tile is bounded by its candidate
+ * fragments times max_weight; a tile where that bound exceeds INT64_MAX ORs 1 into *overflow_dev (int32, zeroed by
+ * the caller) and writes none of its positions.  seq_words_dev / nmask_words_dev: the packed contig of
+ * ftk_gc_observed_u64; out_dev 8-byte aligned.  n_tiles == 0 returns 0 without a launch. */
+#define FTK_GC_DEPTH_MAX_WEIGHT (INT64_C(1) << 62)
+int ftk_gc_depth_tiles_f64(const int32_t *frag_start_dev, const int32_t *frag_stop_dev,
+                           const uint8_t *frag_mapq_dev, int64_t n_frag, int32_t max_frag_len,
+                           const uint32_t *seq_words_dev, const uint32_t *nmask_words_dev, int64_t contig_len,
+                           const int32_t *tile_p0_dev, const int32_t *tile_len_dev,
+                           const int32_t *tile_ivl_lo_dev, const int32_t *tile_ivl_hi_dev,
+                           const int64_t *tile_out_off_dev, int64_t n_tiles,
+                           int32_t min_len, int32_t max_len, int32_t min_mapq, int32_t midpoint,
+                           const int64_t *weights_dev, int64_t max_weight, int64_t *scratch_dev,
+                           int32_t *overflow_dev, double *out_dev, ftk_stream_t stream);
+
 /* ---------------------------------------------------------------- periodicity spectra
  * Segment s is x_dev[offsets_dev[s] .. offsets_dev[s + 1]) (int64 offsets, segments back to back; N values,
  * mean mu).  For every integer period P in [min_period, max_period]:

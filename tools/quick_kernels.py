@@ -1,6 +1,6 @@
 """Kernel timing helper (python tools/quick_kernels.py [motif] [bp] [adjust] [delfi] [hist] [cleavage] [depth] [depth-mid]
 [vplot] [vplot-dense] [ocf] [ocf-dense]
-[gc-obs] [gc-exp] [gc-cov] [gc-site] [spectrum]):
+[gc-obs] [gc-exp] [gc-cov] [gc-site] [gc-depth] [gc-depth-mid] [spectrum]):
 CUDA-event time of the secondary kernels at chr1 scale (80 M fragments drawn on the GPU), median of 7 calls after 3
 warm-ups (the call: planning and uploads included).  Every op except adjust also prints an order-sensitive checksum
 of its output (compare two builds with it) and each kernel's own device time (torch.profiler, a separate run)."""
@@ -44,9 +44,12 @@ def kernels(fn, reps=5):
         for _ in range(reps):
             fn()
         torch.cuda.synchronize()
+    times = {}
     for ev in prof.key_averages():
         if "ftk::" in ev.key:
-            print(f"  kernel {ev.key.split('(')[0]}: {ev.device_time_total / reps / 1e3:.3f} ms", flush=True)
+            times[ev.key.split('(')[0]] = ms = ev.device_time_total / reps / 1e3
+            print(f"  kernel {ev.key.split('(')[0]}: {ms:.3f} ms", flush=True)
+    return times
 
 
 def checksum(o):
@@ -61,10 +64,10 @@ def checksum(o):
 def op(name, fn, nbytes, result=lambda o: o):
     o = timed(name, fn, nbytes)
     print("  checksum", checksum(result(o)), flush=True)
-    kernels(fn)
+    return kernels(fn)
 
 
-if what & {"motif", "bp", "delfi", "gc-obs", "gc-exp", "gc-cov", "gc-site"}:
+if what & {"motif", "bp", "delfi", "gc-obs", "gc-exp", "gc-cov", "gc-site", "gc-depth", "gc-depth-mid"}:
     codes, nm = synth_twobit(CLEN, 0)
     ref = D.PackedContig.from_codes(codes, nm, device=dev)
     ws = np.arange(0, CLEN, 1_000_000, dtype=np.int64); we = np.minimum(ws + 1_000_000, CLEN)
@@ -140,7 +143,7 @@ def candidates(lo, hi, reach):
 
 
 # GC-corrected counts: lengths 50..500, q 30, seeded weights (their values do not change the work)
-if what & {"gc-cov", "gc-site"}:
+if what & {"gc-cov", "gc-site", "gc-depth", "gc-depth-mid"}:
     W = torch.rand((451, 501), generator=g, device=dev, dtype=torch.float64)
 if "gc-cov" in what:
     cand = candidates(tiles[:-1], tiles[1:], min(fr.max_len, 500) >> 1)
@@ -158,6 +161,18 @@ if "gc-site" in what:
     print(f"gc-site: {gc_c.size} sites, {cand} candidates, {int(c.sum())} events", flush=True)
     op("gc-site", lambda: D.gc_weighted_sites(fr, ref, gc_c, gc_f, 1000, W, 50, 500, 30), 9 * cand, lambda o: o[0])
     print(f"  {int(c.sum()) / timed.ms / 1e6:.2f} G events/s over the call", flush=True)
+for name in ("gc-depth", "gc-depth-mid"):
+    if name in what:
+        # GC-corrected depth tracks over the 5-kb tiling: a tile's candidates start up to 500 bp before it
+        cand = candidates(tiles[:-1], tiles[1:], min(fr.max_len, 500))
+        print(f"{name}: {tiles.size - 1} intervals, {cand} candidates", flush=True)
+        kt = op(name, lambda: D.gc_depth_intervals(fr, ref, tiles[:-1], tiles[1:], CLEN, W, 50, 500, 30,
+                                                   name == "gc-depth-mid"), 9 * cand + 8 * CLEN, lambda o: o[0])
+        k = [v for key, v in kt.items() if "gc_depth_tile_kernel" in key]
+        if k:
+            print(f"  over the kernel: {cand / k[0] / 1e6:.2f} G candidates/s; 9 B x candidates "
+                  f"{9 * cand / k[0] / 1e6:.0f} GB/s = {9 * cand / k[0] / 1e6 / 6541.1:.1%} of measured HBM peak",
+                  flush=True)
 if "gc-exp" in what:
     pairs = sum(max(CLEN - L + 1, 0) for L in range(50, 501))   # (m, L) pairs the kernel walks
     op("gc-exp", lambda: D.gc_expected(ref, [0], [CLEN], 50, 500), 0)
